@@ -54,6 +54,7 @@ GATHER_CHECK = 4096
 # evaluations x 22 + 196512 internal-level evaluations x 47
 ALG_SLOTS_PER_SAMPLE = 393216 * 22 + 196512 * 47
 ALG_SLOTS_EVAL = {1: 17, 3: 21}  # 2d + 1 + 14 (SURVEY.md 8d, C3 / C5)
+DUMP_LIMIT = 64 << 20  # bytes written by --dump-outputs, .npy headers included
 
 
 def synth_points(j):
@@ -76,6 +77,25 @@ def mixture(rng, d, N, sigma=0.6):
 def silverman(pts):
     d, N = pts.shape
     return pts.std(axis=1, ddof=1) * (4.0 / ((d + 2.0) * N)) ** (1.0 / (d + 4.0))
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """--dump-outputs: writes every float32 / float64 array of `arrays` (name -> array, one row per sample) as
+    out_dir/<name>.npy, so that two builds can be compared output for output.  If the rows do not fit in `limit`
+    bytes, the same fixed, seeded sample of rows is taken from every array and its row indices go to rows.npy."""
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise ValueError("--dump-outputs writes float32 / float64 only: %s is %s" % (name, a.dtype))
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.itemsize * (a.size // max(n, 1)) for a in arrays.values())
+    header = 128  # .npy header of a 1- or 2-D array
+    if n * row_bytes + len(arrays) * header > limit:
+        k = (limit - (len(arrays) + 1) * header) // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(SEED).choice(n, size=k, replace=False))
+        arrays = dict({name: a[rows] for name, a in arrays.items()}, rows=rows.astype(np.float64))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def host_cores():
@@ -165,8 +185,10 @@ def run_reference(args, rank, world):
         O.gibbs(trees, min(n, cores), NITER, U, G, nthreads=cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        O.gibbs(trees, n, NITER, U, G, nthreads=cores)
+        pts, ind = O.gibbs(trees, n, NITER, U, G, nthreads=cores)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"points": pts.T, "indices": ind.T.astype(np.float32)})
     val = n / dt
     sample = "%d of %d samples per step (C4 shape, injected numpy streams), %d OpenMP threads over chains" % (
         n, SAMPLES_PER_GPU, cores)
@@ -406,7 +428,11 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the C5 / C3 secondary records")
     ap.add_argument("--c5-n", type=int, default=1_000_000)
     ap.add_argument("--c3-n", type=int, default=100_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the points and labels of the last timed step to "
+                    "DIR/points.npy (float64) and DIR/indices.npy (float32), one row per sample")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -506,6 +532,10 @@ def main():
 
     total_ms, clocks = timed(step, args.steps, args.warmup, sample_clocks=True)
     value = Np_total * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:  # the legs below overwrite d_pts / d_idx
+        out_pts, out_idx = (g_pts, g_idx) if world > 1 else (d_pts, d_idx)
+        dump_outputs(args.dump_outputs, {"points": out_pts.cpu().numpy(),
+                                         "indices": out_idx.to(torch.float32).cpu().numpy()})
     gather_ok = gather_check(Np_total, g_pts, g_idx) if world > 1 else None
 
     # ---- strong scaling: BASELINE configs[3], 1M samples in total ---------------------------------------------

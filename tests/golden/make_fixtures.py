@@ -1,7 +1,7 @@
 """Regenerates tests/golden/reference_fixtures.json from the reference's own test data.
 
-Run in the build container only (/root/reference does not exist on the GPU box):
-    python tests/golden/make_fixtures.py
+Run with a checkout of KernelDensityEstimate.jl (the tests only read the JSON it writes):
+    python tests/golden/make_fixtures.py <path to KernelDensityEstimate.jl>
 
 The reference's fixtures (test/testdata/*Result.txt) are MATLAB print-outs of complete
 BallTreeDensity structs with 0-based indices; test/runtests.jl:8-18 parses them and
@@ -11,8 +11,9 @@ them, together with the tolerance each reference test uses.
 """
 import json
 import os
+import sys
 
-REF = "/root/reference/test/testdata"
+REF = os.path.join(sys.argv[1], "test", "testdata")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_fixtures.json")
 
 

@@ -56,6 +56,9 @@ SIGNATURES = {
     "kdeb200_set_pruning": (C.c_int, [C.c_int]),
     "kdeb200_set_gibbs_precision": (C.c_int, [C.c_int]),
     "kdeb200_gibbs_f32_slow_draws": (C.c_int, [C.POINTER(C.c_ulonglong)]),
+    "kdeb200_gibbs_exact_redone": (C.c_int, [C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]),
+    "kdeb200_gibbs_exact_bound_probe": (C.c_int, [C.POINTER(tree_t), C.c_int, C.c_int, C.c_int, C.c_int, f64p, f64p, C.c_int,
+                                                  f64p, C.c_int64]),
     "kdeb200_pruned_stats": (C.c_int, [f64p, i64p]),
     "kdeb200_pipe_peak": (C.c_int, [C.c_int, C.c_int, f64p, f64p]),
     "kdeb200_dfma_probe": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, f64p]),

@@ -29,7 +29,7 @@ __all__ = [
     "KDEError", "BallTree", "BallTreeDensity", "kde", "kde_bang", "getPoints", "getBW", "getWeights", "marginal",
     "sample", "rand", "resample", "evaluateDualTree", "evalAvgLogL", "entropy", "kld", "minkld", "nLOO_LL", "golden",
     "ksize", "neighborMinMax", "lcv_bandwidths", "updateBandwidth", "prodAppxMSGibbsS", "Ndim", "Npts", "init", "init_multi", "multi_count", "gibbs_sizes",
-    "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
+    "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
     "getKDEMax", "getKDEMean", "getKDEfit", "intersIntgAppxIS", "eval_marginals", "to_string", "from_string",
 ]
 
@@ -83,6 +83,30 @@ def gibbs_f32_slow_draws():
     n = C.c_ulonglong(0)
     check(lib().kdeb200_gibbs_f32_slow_draws(C.byref(n)))
     return int(n.value)
+
+
+def gibbs_exact_redone():
+    """(lane-draws, warp-draws) of the FP64 sampler whose leaf-level label the certified FP32 bound could not decide and
+    that were redone in FP64, since the last call"""
+    n, w = C.c_ulonglong(0), C.c_ulonglong(0)
+    check(lib().kdeb200_gibbs_exact_redone(C.byref(n), C.byref(w)))
+    return int(n.value), int(w.value)
+
+
+def _gibbs_exact_bound_probe(trees, Niter, density, level, mu, cadd):
+    """tests: per query conditional (rows of mu, cadd) the header and per-node table of kdeb200_gibbs_exact_bound_probe,
+    as (headers [nq, 8], nodes [nq, n, 8])"""
+    mu = np.ascontiguousarray(mu, dtype=np.float64)
+    cadd = np.ascontiguousarray(cadd, dtype=np.float64)
+    nq = mu.shape[0]
+    n = max(Npts(t) for t in trees)
+    out = np.zeros(nq * (8 + 8 * n))
+    check(lib().kdeb200_gibbs_exact_bound_probe(_handles(trees), len(trees), int(Niter), int(density), int(level),
+                                                fptr(mu), fptr(cadd), nq, fptr(out), out.size))
+    n = int(out[5])
+    per = 8 + 8 * n
+    out = out[:nq * per].reshape(nq, per)
+    return out[:, :8], out[:, 8:].reshape(nq, n, 8)
 
 
 def pruned_stats():

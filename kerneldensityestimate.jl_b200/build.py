@@ -6,8 +6,9 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libkdeb200.so")
-SOURCES = ["context.cu", "tree.cu", "eval.cu", "eval_pruned.cu", "eval_f32.cu", "extras.cu", "lcv.cu", "gibbs.cu", "gibbs_f32.cu", "peaks.cu", "capi.cu"] + [
-    "gibbs_d%d.cu" % d for d in range(1, 9)] + ["gibbs_f32_d%d.cu" % d for d in range(1, 9)]
+SOURCES = ["context.cu", "tree.cu", "eval.cu", "eval_pruned.cu", "eval_f32.cu", "extras.cu", "lcv.cu", "gibbs.cu", "gibbs_f32.cu", "gibbs_exact.cu", "peaks.cu", "capi.cu"] + [
+    "gibbs_d%d.cu" % d for d in range(1, 9)] + ["gibbs_f32_d%d.cu" % d for d in range(1, 9)] + [
+    "gibbs_exact_d%d.cu" % d for d in range(1, 9)]
 GIBBS_TUNED = ["gibbs.cu", "gibbs_d3.cu"]  # what the tuning variants rebuild (GB_ONLY_D3)
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
@@ -24,6 +25,7 @@ KERNEL_SOURCES = {
     "eval_f32": ["eval_f32.cu", "common.cuh"],
     "lcv": ["lcv.cu", "eval_shared.cuh", "common.cuh"],
     "gibbs_f32": ["gibbs_f32_kernel.cuh", "gibbs_f32.cu", "gibbs_kernel.cuh", "common.cuh"],
+    "gibbs_exact": ["gibbs_exact_kernel.cuh", "gibbs_exact.cu", "gibbs_f32_kernel.cuh", "gibbs_kernel.cuh", "common.cuh"],
 }
 
 

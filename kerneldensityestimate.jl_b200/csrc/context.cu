@@ -44,12 +44,14 @@ ScopedDevice::~ScopedDevice() {
 static std::mutex g_mu;
 
 void gibbs_drop_schedules(int slot);  // gibbs.cu
+void gibbs_exact_drop_schedules(int slot);  // gibbs_exact.cu
 
 static void drop_context(Context &c) {
   if (!c.ready) return;
   cudaSetDevice(c.device);
   cudaDeviceSynchronize();
   gibbs_drop_schedules(c.slot);
+  gibbs_exact_drop_schedules(c.slot);
   cudaStreamSynchronize(c.stream);
   cudaFree(c.d_exptab);
   cudaEventDestroy(c.ev0);

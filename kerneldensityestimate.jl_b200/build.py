@@ -1,5 +1,6 @@
 """Builds libkdeb200.so in-tree with nvcc for sm_100a (no JIT cache: the .so travels with the repo)."""
 import os
+import re
 import subprocess
 import sys
 
@@ -9,68 +10,82 @@ OUT = os.path.join(HERE, "libkdeb200.so")
 SOURCES = ["context.cu", "tree.cu", "eval.cu", "eval_pruned.cu", "eval_f32.cu", "extras.cu", "lcv.cu", "gibbs.cu", "gibbs_f32.cu", "gibbs_exact.cu", "peaks.cu", "capi.cu"] + [
     "gibbs_d%d.cu" % d for d in range(1, 9)] + ["gibbs_f32_d%d.cu" % d for d in range(1, 9)] + [
     "gibbs_exact_d%d.cu" % d for d in range(1, 9)]
-GIBBS_TUNED = ["gibbs.cu", "gibbs_d3.cu"]  # what the tuning variants rebuild (GB_ONLY_D3)
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
          "-ccbin", "/usr/bin/g++", "-Xptxas", "-v"]
 
 
-# the sources that determine each hot kernel's instruction stream (tools/ncu_issued.py keys its ncu counters by this
-# hash; bench.py refuses to quote issued-instruction numbers measured on other sources)
-# (device code and the host code that shapes a launch; tree.cuh -- the host-side handle struct -- is deliberately not in)
-KERNEL_SOURCES = {
-    "gibbs": ["gibbs_kernel.cuh", "gibbs.cu", "common.cuh"],
-    "eval": ["eval.cu", "eval_shared.cuh", "common.cuh"],
-    "eval_pruned": ["eval_pruned.cu", "eval_shared.cuh", "common.cuh"],
-    "eval_f32": ["eval_f32.cu", "common.cuh"],
-    "lcv": ["lcv.cu", "eval_shared.cuh", "common.cuh"],
-    "gibbs_f32": ["gibbs_f32_kernel.cuh", "gibbs_f32.cu", "gibbs_kernel.cuh", "common.cuh"],
-    "gibbs_exact": ["gibbs_exact_kernel.cuh", "gibbs_exact.cu", "gibbs_f32_kernel.cuh", "gibbs_kernel.cuh", "common.cuh"],
+# What each Nsight Compute record in profiles/ncu_issued.json (tools/ncu_issued.py) describes, per kind: the object of
+# the library build that holds the profiled kernels, their mangled names, and the launch sources -- the host code that
+# decides the profiled launch's shape (grid, schedule, chunk and tile sizes).  The key hashes the kernels' SASS and
+# resource usage as compiled, plus the launch sources' text, so edits that change neither (comments, other kernels,
+# other host code) leave the records valid.  bench.py refuses to quote a record whose key no longer matches.
+KERNEL_KEYS = {
+    "gibbs": ("gibbs_d3", ["_ZN7kdeb20012gibbs_kernelILi3ELb0ELi8EEEvNS_11GibbsParamsE"],
+              ["gibbs_plan.cuh", "gibbs_kernel.cuh"]),
+    "gibbs_f32": ("gibbs_f32_d3", ["_ZN7kdeb20016gibbs_f32_kernelILi3ELi8EEEvNS_11GibbsParamsE"],
+                  ["gibbs_plan.cuh", "gibbs_f32_kernel.cuh"]),
+    "eval": ("eval", ["_ZN7kdeb20011eval_kernelILi3ELi2ELb0EEEvNS_10EvalParamsE",
+                      "_ZN7kdeb20011eval_kernelILi1ELi6ELb1EEEvNS_10EvalParamsE"], ["eval.cu"]),
+    "eval_pruned": ("eval_pruned", ["_ZN7kdeb20018eval_pruned_kernelILi3ELb0EEEvNS_12PrunedParamsE",
+                                    "_ZN7kdeb20014loo_sym_kernelILi1ELi8EEEvNS_9SymParamsE"], ["eval_pruned.cu"]),
 }
+
+
+def _cuobjdump(*args):
+    exe = os.path.join(os.path.dirname(NVCC), "cuobjdump")
+    if not os.path.exists(exe):
+        raise RuntimeError("kernel_source_hash needs cuobjdump next to nvcc (%s)" % exe)
+    return subprocess.run([exe] + list(args), check=True, capture_output=True, text=True).stdout
 
 
 def kernel_source_hash(kind):
     import hashlib
+    obj, funcs, launch_sources = KERNEL_KEYS[kind]
+    build()
+    o = os.path.join(HERE, "build", obj + ".o")
+    usage = _cuobjdump("-res-usage", o).splitlines()
     h = hashlib.sha256()
-    for f in KERNEL_SOURCES[kind]:
+    for fn in funcs:
+        sass = _cuobjdump("-sass", "-fun", fn, o)
+        at = sass.find("Function : " + fn)  # the header before it names the source file's path
+        use = [usage[i + 1] for i, line in enumerate(usage[:-1]) if line.strip() == "Function %s:" % fn]
+        if at < 0 or len(use) != 1:
+            raise RuntimeError("kernel_source_hash(%r): %s not found in %s" % (kind, fn, o))
+        h.update(fn.encode() + b"\0" + sass[at:].encode() + b"\0" + use[0].strip().encode() + b"\0")
+    for f in launch_sources:
         with open(os.path.join(CSRC, f), "rb") as fh:
             h.update(f.encode() + b"\0" + fh.read())
-    h.update(" ".join(FLAGS).encode())
     return h.hexdigest()[:16]
 
 
 def _stale():
     if not os.path.exists(OUT):
         return True
+    if not all(os.path.exists(os.path.join(HERE, "build", s.replace(".cu", ".o"))) for s in SOURCES):
+        return True  # kernel_source_hash and build_variant read the objects
     t = os.path.getmtime(OUT)
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", "kdeb200.h")]
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_variant(tag, defines, tuned=None):
-    """Experimental builds (tuning sweeps): libkdeb200_<tag>.so with extra -D flags on the sources in `tuned`
-    (default: the Gibbs kernel); selected at run time with KDEB200_SO=<path>."""
-    global GIBBS_TUNED
-    saved = GIBBS_TUNED
-    if tuned is not None:
-        GIBBS_TUNED = list(tuned)
-    try:
-        return _build_variant(tag, defines)
-    finally:
-        GIBBS_TUNED = saved
-
-
-def _build_variant(tag, defines):
+def build_variant(tag, defines):
+    """Experimental builds (tuning sweeps): libkdeb200_<tag>.so with extra -D flags, selected at run time with
+    KDEB200_SO=<path>.  Every Gibbs source is rebuilt with the flags: the host code plans each route's chunks and tiles
+    with the same constants (GB_TILE_N, GB_MAXCK_N, unroll depths) its kernel is compiled with.  With GB_ONLY_D3 or
+    GF_ONLY_D3 the host code launches d = 3 only, and the other instantiations are left out."""
     out = os.path.join(HERE, "libkdeb200_%s.so" % tag)
     bdir = os.path.join(HERE, "build", tag)
     os.makedirs(bdir, exist_ok=True)
+    only_d3 = any("ONLY_D3" in d for d in defines)
     procs, objs = [], []
     build()
     for s in SOURCES:
-        if s not in GIBBS_TUNED:  # everything else comes from the main build
-            if not (s.startswith("gibbs_d") and any("GB_ONLY_D3" in d for d in defines)) and not (
-                    s.startswith("gibbs_f32_d") and s != "gibbs_f32_d3.cu" and any("GF_ONLY_D3" in d for d in defines)):
-                objs.append(os.path.join(HERE, "build", s.replace(".cu", ".o")))
+        if not s.startswith("gibbs"):  # everything else comes from the main build
+            objs.append(os.path.join(HERE, "build", s.replace(".cu", ".o")))
+            continue
+        inst = re.search(r"_d(\d)\.cu$", s)  # one instantiation per dimension
+        if only_d3 and inst and inst.group(1) != "3":
             continue
         o = os.path.join(bdir, s.replace(".cu", ".o"))
         objs.append(o)

@@ -8,7 +8,7 @@
 #include <thread>
 #include <vector>
 
-#include "tree.cuh"
+#include "gibbs.cuh"
 
 namespace kdeb200 {
 int tree_build_host(int d, int64_t N, const double *points, const double *weights, const double *bw_var,
@@ -41,23 +41,6 @@ int eval_device_f32(kdeb200_tree_t bd, const double *d_pos, int64_t M, int loo, 
                     int *launches);
 int loo_partial_device(kdeb200_tree_t bd, const double *bw_var, int64_t j0, int64_t j1, double *d_sum, int *d_flag,
                        cudaStream_t st, int *launches);
-int gibbs_sizes(const kdeb200_tree_t *trees, int ndens, int Niter, int *nlevels, int64_t *perU, int64_t *perN,
-                int64_t *evals);
-int gibbs_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, int add_entropy,
-                 const uint8_t *dimmask, const double *d_randU, int64_t nU, const double *d_randN, int64_t nN,
-                 uint64_t seed, int64_t s0, int64_t s1, double *d_points, int64_t *d_indices,
-                 int64_t *d_level_labels, cudaStream_t st, int *launches);
-int gibbs_exact_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, int add_entropy,
-                       const uint8_t *dimmask, const double *d_randU, int64_t nU, const double *d_randN, int64_t nN,
-                       uint64_t seed, int64_t s0, int64_t s1, double *d_points, int64_t *d_indices,
-                       int64_t *d_level_labels, cudaStream_t st, int *launches);
-int gibbs_exact_redone(unsigned long long *lanes, unsigned long long *warps);
-int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, int level, const double *mu,
-                      const double *cadd, int nq, double *out, int64_t out_len);
-int philox_streams_device(uint64_t seed, int64_t Np, int64_t perU, int64_t perN, double *d_U, double *d_G,
-                          cudaStream_t st);
-int gibbs_set_precision(int p);
-int gibbs32_slow_draws(unsigned long long *out);
 int pipe_peak(int which, int iters, double *lane_ops_per_s, double *ms_out);
 int dfma_probe(int ilp, int blocks_per_sm, int threads, int iters, double *lane_ops_per_s);
 
@@ -173,10 +156,10 @@ static int gibbs_host_block(const kdeb200_tree_t *trees, int ndens, int64_t Np, 
   int rc;
   if (randU) {
     // device slices are re-based: sample s reads U[(s-a)*perU + c - 1 + 1] => pass pointer + 1
-    rc = gibbs_exact_device(loc, ndens, n, Niter, add_entropy, dimmask, dU.as<double>() + 1, n * perU - 1, dN.as<double>(),
+    rc = gibbs_device(loc, ndens, n, Niter, add_entropy, dimmask, dU.as<double>() + 1, n * perU - 1, dN.as<double>(),
                       n * perN, seed, 0, n, dP.as<double>(), dI.as<int64_t>(), d_rec, c.stream, &launches);
   } else {
-    rc = gibbs_exact_device(loc, ndens, Np, Niter, add_entropy, dimmask, nullptr, 0, nullptr, 0, seed, a, b, dP.as<double>(),
+    rc = gibbs_device(loc, ndens, Np, Niter, add_entropy, dimmask, nullptr, 0, nullptr, 0, seed, a, b, dP.as<double>(),
                       dI.as<int64_t>(), d_rec, c.stream, &launches);
   }
   if (rc) return rc;
@@ -321,7 +304,7 @@ int kdeb200_gibbs_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int
   if (int rc = ensure_init()) return rc;
   if (!trees || !d_points || !d_indices) KDE_FAIL(2, "gibbs_device: NULL argument");
   int launches = 0;
-  int rc = gibbs_exact_device(trees, ndens, Np, Niter, add_entropy, dimmask, d_randU, nU, d_randN, nN, seed, s0, s1,
+  int rc = gibbs_device(trees, ndens, Np, Niter, add_entropy, dimmask, d_randU, nU, d_randN, nN, seed, s0, s1,
                         d_points, d_indices, d_level_labels, (cudaStream_t)stream, &launches);
   ctx().last_launches = launches;
   return rc;
@@ -526,7 +509,7 @@ int kdeb200_product_kde(const kdeb200_tree_t *trees, int ndens, int64_t Np, int 
   KDE_CUDA(dO.alloc(sizeof(double) * 5 * d));
   Timer tm(c);
   int launches = 0;
-  if (int rc = gibbs_exact_device(trees, ndens, Np, Niter, add_entropy, dimmask, nullptr, 0, nullptr, 0, seed, 0, Np,
+  if (int rc = gibbs_device(trees, ndens, Np, Niter, add_entropy, dimmask, nullptr, 0, nullptr, 0, seed, 0, Np,
                             dP.as<double>(), dI.as<int64_t>(), nullptr, c.stream, &launches))
     return rc;
   const bool fused = Np <= 512;  // the samples never leave the device between the two kernels

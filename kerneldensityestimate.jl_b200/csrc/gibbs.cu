@@ -1,5 +1,6 @@
-// gibbs.cu -- host side of K1: schedule construction, launch, Philox stream materialisation.
-// The kernel lives in gibbs_kernel.cuh and is instantiated once per dimension in gibbs_d<N>.cu.
+// gibbs.cu -- host side of the Gibbs sampler: argument checks, routing (K1w, K1f, K1x, K1), the schedule cache of the
+// thread-per-chain kernels, the launches of K1 and K1w, Philox stream materialisation.  K1's kernels live in
+// gibbs_kernel.cuh and are instantiated once per dimension in gibbs_d<N>.cu; the schedule is planned in gibbs_plan.cuh.
 #include <atomic>
 #include <cmath>
 #include <cstdlib>
@@ -8,32 +9,16 @@
 #include <mutex>
 #include <vector>
 
-#include "gibbs_kernel.cuh"
+#include "gibbs.cuh"
+#include "gibbs_plan.cuh"
 
 namespace kdeb200 {
 
-// gibbs_f32.cu
-int gibbs_precision();
-void gibbs32_drop_schedules(int slot);
-int gibbs32_launch(const kdeb200_tree_t *trees, int ndens, int L, int Niter, bool masked, GibbsParams &P, cudaStream_t st);
-
-extern template cudaError_t launch_gibbs_d<1>(const GibbsParams &, bool, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_d<2>(const GibbsParams &, bool, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_d<3>(const GibbsParams &, bool, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_d<4>(const GibbsParams &, bool, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_d<5>(const GibbsParams &, bool, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_d<6>(const GibbsParams &, bool, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_d<7>(const GibbsParams &, bool, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_d<8>(const GibbsParams &, bool, int, size_t, cudaStream_t, int);
-
-extern template cudaError_t launch_gibbs_warp_d<1>(const GibbsParams &, bool, int, cudaStream_t);
-extern template cudaError_t launch_gibbs_warp_d<2>(const GibbsParams &, bool, int, cudaStream_t);
-extern template cudaError_t launch_gibbs_warp_d<3>(const GibbsParams &, bool, int, cudaStream_t);
-extern template cudaError_t launch_gibbs_warp_d<4>(const GibbsParams &, bool, int, cudaStream_t);
-extern template cudaError_t launch_gibbs_warp_d<5>(const GibbsParams &, bool, int, cudaStream_t);
-extern template cudaError_t launch_gibbs_warp_d<6>(const GibbsParams &, bool, int, cudaStream_t);
-extern template cudaError_t launch_gibbs_warp_d<7>(const GibbsParams &, bool, int, cudaStream_t);
-extern template cudaError_t launch_gibbs_warp_d<8>(const GibbsParams &, bool, int, cudaStream_t);
+#define GB_EXTERN(D)                                                                                      \
+  extern template cudaError_t launch_gibbs_d<D>(const GibbsParams &, bool, int, size_t, cudaStream_t, int); \
+  extern template cudaError_t launch_gibbs_warp_d<D>(const GibbsParams &, bool, int, cudaStream_t);
+GB_EXTERN(1) GB_EXTERN(2) GB_EXTERN(3) GB_EXTERN(4) GB_EXTERN(5) GB_EXTERN(6) GB_EXTERN(7) GB_EXTERN(8)
+#undef GB_EXTERN
 
 __global__ void philox_streams_kernel(uint64_t seed, int64_t Np, int64_t perU, int64_t perN, double *U, double *G) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -52,69 +37,6 @@ int gibbs_nlevels(const kdeb200_tree_t *trees, int ndens) {
   for (int j = 0; j < ndens; ++j)
     if (maxNp < trees[j]->N) maxNp = trees[j]->N;
   return (int)std::floor((std::log((double)maxNp) / std::log(2.0)) + 1.0);  // src/MSGibbs01.jl:568
-}
-
-struct Schedule {
-  std::vector<Draw> draws;
-  std::vector<TileDesc> tiles;
-  int64_t evals = 0;
-};
-
-static void build_schedule(const kdeb200_tree_t *trees, int M, int L, int T, bool masked, bool literal, Schedule &S) {
-  for (int l = 1; l <= L; ++l) {
-    for (int pass = 0; pass <= T; ++pass) {
-      for (int j = 0; j < M; ++j) {
-        const kdeb200_tree_s *t = trees[j];
-        const Level &lv = t->levels[l < t->depth ? l : t->depth];
-        Draw dr;
-        std::memset(&dr, 0, sizeof(dr));
-        dr.j = (short)j;
-        dr.kind = pass == 0 ? 0 : 1;
-        dr.level = (short)l;
-        dr.new_level = (pass == 0 && j == 0) ? 1 : 0;
-        dr.n = (int)lv.n;
-        dr.wts = t->d_buf + lv.offW;
-        dr.levperm = t->d_levperm + lv.offP;
-        if (lv.cls == 0) {
-          dr.variant = VAR_A;
-          dr.rec = t->d_buf + lv.offA;
-          dr.stride = t->SA;
-          dr.rec_state = dr.rec;
-          dr.state_stride = t->SA;
-          dr.state_has_bw = 0;
-        } else {
-          dr.variant = (pass == 0 && !masked && !literal) ? VAR_B : VAR_C;  // B records hold -0.5/b, not b
-          dr.rec = t->d_buf + (dr.variant == VAR_B ? lv.offB : lv.offC);
-          dr.stride = t->SC;
-          dr.rec_state = t->d_buf + lv.offC;
-          dr.state_stride = t->SC;
-          dr.state_has_bw = 1;
-        }
-        int G = 1;
-        while ((int64_t)G * GB_MAXCK < lv.n) G *= 2;
-        const int dg = gb_dg(t->d, dr.variant);
-        if (G < dg && lv.n >= 2 * dg) G = dg;  // pass 1 checkpoints per whole double group
-        dr.G = G;
-        dr.nchunks = (int)((lv.n + G - 1) / G);
-        int tn = 1;
-        while (tn * 2 * dr.stride * 8 <= GB_TILE_BYTES) tn *= 2;
-        dr.tnodes = tn;
-        dr.ntiles = (int)((lv.n + tn - 1) / tn);
-        dr.tile0 = (int)S.tiles.size();
-        for (int q = 0; q < dr.ntiles; ++q) {
-          const int64_t a = (int64_t)q * tn;
-          const int64_t cnt = (lv.n - a < tn) ? (lv.n - a) : tn;
-          TileDesc td;
-          td.src = dr.rec + a * dr.stride;
-          td.bytes = (uint32_t)(cnt * dr.stride * sizeof(double));
-          td.pad = 0;
-          S.tiles.push_back(td);
-        }
-        S.evals += lv.n;
-        S.draws.push_back(dr);
-      }
-    }
-  }
 }
 
 int gibbs_sizes(const kdeb200_tree_t *trees, int ndens, int Niter, int *nlevels, int64_t *perU, int64_t *perN,
@@ -141,52 +63,89 @@ int gibbs_sizes(const kdeb200_tree_t *trees, int ndens, int Niter, int *nlevels,
 }
 
 // ---- schedule cache -----------------------------------------------------------------------------------------
-// The static schedule (draws + tile list) depends only on the tree set, Niter and the mask class.  It used to be rebuilt,
-// allocated (3 x cudaMallocAsync), uploaded and SYNCHRONISED on every call -- irrelevant at 1M samples, but it was the
-// difference between a 0.34 ms kernel and a 0.39 ms call at the small configurations, and it made kdeb200_gibbs_device
-// block.  Entries are keyed by (context slot, tree handles, Niter, masked) and invalidated wholesale whenever any tree
-// is destroyed (a global epoch); each context keeps the 8 most recent.  Batch counters come from a ring of 256 slots
-// per entry, zeroed once at creation and reset by the LAST CTA of each launch.
+// The static schedule (draws + tile list, and K1f's / K1x's FP32 records) depends only on the tree set, Niter and the
+// route's key (SchedEntry).  It used to be rebuilt, allocated, uploaded and SYNCHRONISED on every call -- irrelevant at
+// 1M samples, but it was the difference between a 0.34 ms kernel and a 0.39 ms call at the small configurations, and it
+// made kdeb200_gibbs_device block.  Entries are invalidated wholesale whenever any tree is destroyed (a global epoch);
+// each context keeps the most recent ones of each route (K1 8, K1f 4, K1x 4).  Batch counters come from a ring of 256
+// slots per entry, zeroed once at creation and reset by the LAST CTA of each launch.
 std::atomic<uint64_t> g_tree_epoch{1};
 void gibbs_invalidate_schedules() { g_tree_epoch.fetch_add(1); }
 
 namespace {
-struct SchedEntry {
-  uint64_t epoch = 0;
-  int slot = 0, M = 0, T = 0;
-  bool masked = false, literal = false;
-  kdeb200_tree_t trees[KDEB200_MAX_DENS] = {nullptr};
-  char *d_base = nullptr;  // draws | tiles | counters, one allocation on the context's device
-  Draw *d_draws = nullptr;
-  TileDesc *d_tiles = nullptr;
-  int *d_counters = nullptr;
-  int ndraws = 0, ntiles = 0;
-  unsigned next_counter = 0;
-};
 constexpr int SCHED_COUNTERS = 256;
-constexpr size_t SCHED_KEEP = 8;
+constexpr size_t SCHED_KEEP[NROUTES] = {8, 4, 4};
 std::mutex g_sched_mu;
-std::list<SchedEntry> g_sched[KDEB200_MAX_GPUS];
+std::list<SchedEntry> g_sched[NROUTES][KDEB200_MAX_GPUS];
+unsigned long long *g_counters[KDEB200_MAX_GPUS] = {nullptr};
+constexpr int NCOUNTERS = 3;
 
 void sched_free(SchedEntry &e, cudaStream_t st) {
   if (e.d_base) cudaFreeAsync(e.d_base, st);
-  e.d_base = nullptr;
+  if (e.d_extra) cudaFreeAsync(e.d_extra, st);
+  e.d_base = e.d_extra = nullptr;
+}
+
+bool same_key(const SchedEntry &a, const SchedEntry &b) {
+  if (a.M != b.M || a.T != b.T || a.masked != b.masked || a.literal != b.literal ||
+      std::memcmp(a.mask, b.mask, sizeof(a.mask)) != 0)
+    return false;
+  for (int j = 0; j < a.M; ++j)
+    if (a.trees[j] != b.trees[j]) return false;
+  return true;
+}
+
+size_t up256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// plan, allocate, run the route's part, upload; the upload runs on the library stream of this context and is complete
+// before the entry is published, so the caller's stream only ever sees finished buffers
+int sched_build(Route r, const kdeb200_tree_t *trees, int L, SchedEntry &e) {
+  Context &c = ctx();
+  Plan S;
+  plan_schedule(trees, e.M, L, e.T, !e.masked && !e.literal, r != ROUTE_K1, r == ROUTE_K1F, S);
+  const size_t b_draws = up256(sizeof(Draw) * S.draws.size()), b_tiles = up256(sizeof(TileDesc) * S.tiles.size()),
+               b_cnt = up256(sizeof(int) * SCHED_COUNTERS),
+               b_rec = S.blocks.empty() ? 0 : up256(sizeof(float) * (S.nfloats + 8));
+  KDE_CUDA(cudaMallocAsync(&e.d_base, b_draws + b_tiles + b_cnt + b_rec, c.stream));
+  e.d_draws = reinterpret_cast<Draw *>(e.d_base);
+  e.d_tiles = reinterpret_cast<TileDesc *>(e.d_base + b_draws);
+  e.d_counters = reinterpret_cast<int *>(e.d_base + b_draws + b_tiles);
+  e.d_rec = b_rec ? reinterpret_cast<float *>(e.d_base + b_draws + b_tiles + b_cnt) : nullptr;
+  if (r == ROUTE_K1F)
+    if (int rc = gibbs32_build(trees, S, e)) return rc;
+  if (r == ROUTE_K1X)
+    if (int rc = gibbs_exact_build(trees, S, e)) return rc;
+  std::vector<TileDesc> tds(S.tiles.size());
+  for (size_t i = 0; i < S.tiles.size(); ++i) {
+    tds[i].src = S.tiles[i].src ? S.tiles[i].src : reinterpret_cast<const double *>(e.d_rec + S.tiles[i].off);
+    tds[i].bytes = S.tiles[i].bytes;
+    tds[i].pad = 0;
+  }
+  e.ndraws = (int)S.draws.size();
+  e.ntiles = (int)tds.size();
+  cudaError_t err = cudaMemcpyAsync(e.d_draws, S.draws.data(), sizeof(Draw) * S.draws.size(), cudaMemcpyHostToDevice, c.stream);
+  if (err == cudaSuccess) err = cudaMemcpyAsync(e.d_tiles, tds.data(), sizeof(TileDesc) * tds.size(), cudaMemcpyHostToDevice, c.stream);
+  if (err == cudaSuccess) err = cudaMemsetAsync(e.d_counters, 0, b_cnt, c.stream);
+  if (err == cudaSuccess) err = cudaStreamSynchronize(c.stream);  // the host vectors are pageable memory
+  if (err != cudaSuccess) KDE_FAIL(100 + (int)err, "gibbs: uploading the schedule: %s", cudaGetErrorString(err));
+  return 0;
 }
 }  // namespace
 
-// drops every cached schedule of a context (its device memory is about to go away)
 void gibbs_drop_schedules(int slot) {
-  gibbs32_drop_schedules(slot);
   std::lock_guard<std::mutex> lk(g_sched_mu);
-  for (auto &e : g_sched[slot]) sched_free(e, ctx_at(slot).stream);
-  g_sched[slot].clear();
+  for (auto &lst : g_sched) {
+    for (auto &e : lst[slot]) sched_free(e, ctx_at(slot).stream);
+    lst[slot].clear();
+  }
+  if (g_counters[slot]) cudaFreeAsync(g_counters[slot], ctx_at(slot).stream);
+  g_counters[slot] = nullptr;
 }
 
-static int sched_get(const kdeb200_tree_t *trees, int M, int L, int T, bool masked, bool literal, cudaStream_t st,
-                     SchedEntry *out, int **counter) {
+int sched_get(Route r, const kdeb200_tree_t *trees, int L, const SchedEntry &key, SchedEntry *out, int **counter) {
   Context &c = ctx();
   std::lock_guard<std::mutex> lk(g_sched_mu);
-  auto &lst = g_sched[c.slot];
+  auto &lst = g_sched[r][c.slot];
   const uint64_t epoch = g_tree_epoch.load();
   for (auto it = lst.begin(); it != lst.end();) {  // entries from before the last tree_destroy may point at freed records
     if (it->epoch != epoch) {
@@ -196,57 +155,76 @@ static int sched_get(const kdeb200_tree_t *trees, int M, int L, int T, bool mask
       ++it;
     }
   }
-  for (auto it = lst.begin(); it != lst.end(); ++it) {
-    if (it->M != M || it->T != T || it->masked != masked || it->literal != literal) continue;
-    bool same = true;
-    for (int j = 0; j < M; ++j) same = same && it->trees[j] == trees[j];
-    if (!same) continue;
+  auto it = lst.begin();
+  while (it != lst.end() && !same_key(*it, key)) ++it;
+  if (it != lst.end()) {
     lst.splice(lst.begin(), lst, it);  // most recently used first
-    *counter = it->d_counters + (it->next_counter++ % SCHED_COUNTERS);
-    *out = *it;
-    return 0;
+  } else {
+    SchedEntry e = key;
+    e.epoch = epoch;
+    if (int rc = sched_build(r, trees, L, e)) {
+      sched_free(e, c.stream);
+      return rc;
+    }
+    lst.push_front(e);
+    while (lst.size() > SCHED_KEEP[r]) {
+      // an evicted entry may still be read by a kernel in flight on a caller stream: release it only after the device
+      // has drained (rare: more distinct tree sets alternating than the route keeps)
+      cudaDeviceSynchronize();
+      sched_free(lst.back(), c.stream);
+      lst.pop_back();
+    }
   }
-  Schedule S;
-  build_schedule(trees, M, L, T, masked, literal, S);
-  SchedEntry e;
-  e.epoch = epoch;
-  e.slot = c.slot;
-  e.M = M;
-  e.T = T;
-  e.masked = masked;
-  e.literal = literal;
-  for (int j = 0; j < M; ++j) e.trees[j] = trees[j];
-  e.ndraws = (int)S.draws.size();
-  e.ntiles = (int)S.tiles.size();
-  auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-  const size_t b_draws = up(sizeof(Draw) * S.draws.size()), b_tiles = up(sizeof(TileDesc) * S.tiles.size()),
-               b_cnt = up(sizeof(int) * SCHED_COUNTERS);
-  // the upload runs on the library stream of this context and is complete before the entry is published; the caller's
-  // stream only ever sees finished buffers
-  KDE_CUDA(cudaMallocAsync(&e.d_base, b_draws + b_tiles + b_cnt, c.stream));
-  e.d_draws = reinterpret_cast<Draw *>(e.d_base);
-  e.d_tiles = reinterpret_cast<TileDesc *>(e.d_base + b_draws);
-  e.d_counters = reinterpret_cast<int *>(e.d_base + b_draws + b_tiles);
-  cudaError_t err = cudaMemcpyAsync(e.d_draws, S.draws.data(), sizeof(Draw) * S.draws.size(), cudaMemcpyHostToDevice, c.stream);
-  if (err == cudaSuccess) err = cudaMemcpyAsync(e.d_tiles, S.tiles.data(), sizeof(TileDesc) * S.tiles.size(), cudaMemcpyHostToDevice, c.stream);
-  if (err == cudaSuccess) err = cudaMemsetAsync(e.d_counters, 0, b_cnt, c.stream);
-  if (err == cudaSuccess) err = cudaStreamSynchronize(c.stream);  // S's vectors are pageable host memory
-  if (err != cudaSuccess) {
-    cudaFreeAsync(e.d_base, c.stream);
-    KDE_FAIL(100 + (int)err, "gibbs: uploading the schedule: %s", cudaGetErrorString(err));
-  }
-  (void)st;
-  lst.push_front(e);
-  while (lst.size() > SCHED_KEEP) {
-    // an evicted entry may still be read by a kernel in flight on a caller stream: release it only after the device
-    // has drained (rare: more than 8 distinct tree sets alternating)
-    cudaDeviceSynchronize();
-    sched_free(lst.back(), c.stream);
-    lst.pop_back();
-  }
-  *counter = lst.front().d_counters + (lst.front().next_counter++ % SCHED_COUNTERS);
+  if (counter) *counter = lst.front().d_counters + (lst.front().next_counter++ % SCHED_COUNTERS);
   *out = lst.front();
   return 0;
+}
+
+int gibbs_counters(unsigned long long **out) {
+  Context &c = ctx();
+  std::lock_guard<std::mutex> lk(g_sched_mu);
+  if (!g_counters[c.slot]) {
+    KDE_CUDA(cudaMallocAsync(&g_counters[c.slot], NCOUNTERS * sizeof(unsigned long long), c.stream));
+    KDE_CUDA(cudaMemsetAsync(g_counters[c.slot], 0, NCOUNTERS * sizeof(unsigned long long), c.stream));
+    KDE_CUDA(cudaStreamSynchronize(c.stream));  // the caller's stream must see a finished buffer
+  }
+  *out = g_counters[c.slot];
+  return 0;
+}
+
+// counters [first, first + n) of the calling context's device, reset to zero (synchronises the device)
+static int take_counters(int first, int n, unsigned long long *h) {
+  unsigned long long *d = nullptr;
+  if (int rc = gibbs_counters(&d)) return rc;
+  KDE_CUDA(cudaDeviceSynchronize());
+  KDE_CUDA(cudaMemcpy(h, d + first, n * sizeof(*h), cudaMemcpyDeviceToHost));
+  KDE_CUDA(cudaMemset(d + first, 0, n * sizeof(*h)));
+  return 0;
+}
+
+// K1f draws redone in FP64 since the last call
+int gibbs32_slow_draws(unsigned long long *out) { return take_counters(0, 1, out); }
+
+// K1x lane-draws and warp-draws redone in FP64 since the last call
+int gibbs_exact_redone(unsigned long long *lanes, unsigned long long *warps) {
+  unsigned long long h[2] = {0, 0};
+  if (int rc = take_counters(1, 2, h)) return rc;
+  if (lanes) *lanes = h[0];
+  if (warps) *warps = h[1];
+  return 0;
+}
+
+// K1x takes the thread-per-chain FP64 calls that it has been measured to win: every dimension of every density (no
+// partial-dimension mask, no lone density), no literal arithmetic, d = 3 (the only dimension measured so far; C4: 904
+// -> 776 ms per 1M samples, DESIGN.md K1x), and leaf bandwidths whose FP32 scale s_k = sqrt(0.5 log2 e / c_k) stays a
+// normal float.  KDEB200_GIBBS_EXACT=0 forces K1.
+static bool exact_eligible(const kdeb200_tree_t *trees, int ndens, bool masked, bool literal) {
+  const char *ev = getenv("KDEB200_GIBBS_EXACT");
+  if ((ev && atoi(ev) == 0) || ndens < 2 || masked || literal || trees[0]->d != 3) return false;
+  for (int j = 0; j < ndens; ++j)
+    for (int k = 0; k < trees[0]->d; ++k)
+      if (!(trees[j]->hvar[k] >= 1e-20 && trees[j]->hvar[k] <= 1e20)) return false;
+  return true;
 }
 
 int gibbs_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, int add_entropy,
@@ -289,10 +267,40 @@ int gibbs_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, 
         if (i != j && P.mask[i][k]) o = 1;
       P.other[j][k] = o;
     }
+  if (literal) masked = true;  // the literal evaluation reads the activity flags in every mode
+
+  // Few chains: one warp per chain (K1w).  The thread-per-chain kernel needs ~128 x 4 x SMs chains to fill the chip and
+  // costs the same 0.3 - 3 ms whether it runs 100 chains or 10 000; measured crossover (tools/gibbs_kernel_crossover.py,
+  // profiles/r02_gibbs_crossover.json): ~4 000 chains for 2 - 6 densities of 100 - 1000 components, so the warp
+  // kernel takes calls of up to 24 chains per SM (KDEB200_GIBBS_WARP_MAX overrides; 0 disables it).  Its prefix sums
+  // live in shared memory, which bounds the level size.
+  int nmax = 1;
+  for (int j = 0; j < ndens; ++j)
+    if (trees[j]->levels[trees[j]->depth].n > nmax) nmax = (int)trees[j]->levels[trees[j]->depth].n;
+  int64_t warp_max = (int64_t)24 * c.sm_count;
+  if (const char *ev = getenv("KDEB200_GIBBS_WARP_MAX")) warp_max = atoll(ev);
+  const bool warp_fits = gibbs_warp_smem(d, nmax) <= 96 * 1024;
+  if (literal && !warp_fits)
+    KDE_FAIL(8, "gibbs: a density has a zero, non-finite or out-of-range (variance outside [1e-30, 1e30]) bandwidth / mean / "
+                "weight and more than ~2900 components: the verbatim-arithmetic kernel cannot hold its level lists "
+                "(no CPU fallback)");
+  const bool warp = warp_fits && (literal || s1 - s0 <= warp_max);
+
+  Route r = ROUTE_K1;
+  if (!warp && gibbs_precision() == KDEB200_F32)
+    r = ROUTE_K1F;  // FP32 label probabilities (statistical mode only)
+  else if (!warp && exact_eligible(trees, ndens, masked, literal))
+    r = ROUTE_K1X;
+  SchedEntry key;
+  key.M = ndens;
+  key.T = Niter;
+  for (int j = 0; j < ndens; ++j) key.trees[j] = trees[j];
+  if (r != ROUTE_K1X) key.masked = masked;
+  if (r == ROUTE_K1) key.literal = literal;
+  if (r == ROUTE_K1F) std::memcpy(key.mask, P.mask, sizeof(key.mask));
   SchedEntry E;
   int *d_counter = nullptr;
-  if (literal) masked = true;  // the literal evaluation reads the activity flags in every mode
-  if (int rc = sched_get(trees, ndens, L, Niter, masked, literal, st, &E, &d_counter)) return rc;
+  if (int rc = sched_get(r, trees, L, key, &E, &d_counter)) return rc;
 
   P.draws = E.d_draws;
   P.tiles = E.d_tiles;
@@ -323,64 +331,21 @@ int gibbs_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, 
     P.labels[j] = t->d_labels;
     for (int k = 0; k < d; ++k) P.hvar[j][k] = t->hvar[k];
   }
-  // Few chains: one warp per chain (K1w).  The thread-per-chain kernel needs ~128 x 4 x SMs chains to fill the chip and
-  // costs the same 0.3 - 3 ms whether it runs 100 chains or 10 000; measured crossover (tools/gibbs_kernel_crossover.py,
-  // profiles/r02_gibbs_crossover.json): ~4 000 chains for 2 - 6 densities of 100 - 1000 components, so the warp
-  // kernel takes calls of up to 24 chains per SM (KDEB200_GIBBS_WARP_MAX overrides; 0 disables it).  Its prefix sums
-  // live in shared memory, which bounds the level size.
-  {
-    int nmax = 1;
-    for (int j = 0; j < ndens; ++j)
-      if (trees[j]->levels[trees[j]->depth].n > nmax) nmax = (int)trees[j]->levels[trees[j]->depth].n;
-    int64_t warp_max = (int64_t)24 * c.sm_count;
-    if (const char *ev = getenv("KDEB200_GIBBS_WARP_MAX")) warp_max = atoll(ev);
-    if (literal && gibbs_warp_smem(d, nmax) > 96 * 1024)
-      KDE_FAIL(8, "gibbs: a density has a zero, non-finite or out-of-range (variance outside [1e-30, 1e30]) bandwidth / mean / "
-                  "weight and more than ~2900 components: the verbatim-arithmetic kernel cannot hold its level lists "
-                  "(no CPU fallback)");
-    if ((literal || s1 - s0 <= warp_max) && gibbs_warp_smem(d, nmax) <= 96 * 1024) {
-      cudaError_t we = cudaErrorInvalidValue;
-      switch (d) {
-#ifdef GB_ONLY_D3
-        case 3: we = launch_gibbs_warp_d<3>(P, masked, nmax, st); break;
-#else
-        case 1: we = launch_gibbs_warp_d<1>(P, masked, nmax, st); break;
-        case 2: we = launch_gibbs_warp_d<2>(P, masked, nmax, st); break;
-        case 3: we = launch_gibbs_warp_d<3>(P, masked, nmax, st); break;
-        case 4: we = launch_gibbs_warp_d<4>(P, masked, nmax, st); break;
-        case 5: we = launch_gibbs_warp_d<5>(P, masked, nmax, st); break;
-        case 6: we = launch_gibbs_warp_d<6>(P, masked, nmax, st); break;
-        case 7: we = launch_gibbs_warp_d<7>(P, masked, nmax, st); break;
-        case 8: we = launch_gibbs_warp_d<8>(P, masked, nmax, st); break;
-#endif
-      }
-      if (we != cudaSuccess) KDE_FAIL(100 + (int)we, "gibbs (warp per chain) kernel launch: %s", cudaGetErrorString(we));
-      if (launches) *launches += 1;
-      return 0;
-    }
+
+  if (r == ROUTE_K1F) {
+    if (int rc = gibbs32_launch(P, E, d, st)) return rc;
+  } else if (r == ROUTE_K1X) {
+    if (int rc = gibbs_exact_launch(P, E, d, st)) return rc;
+  } else if (warp) {
+    const cudaError_t e = with_d(d, [&](auto D) { return launch_gibbs_warp_d<decltype(D)::value>(P, masked, nmax, st); });
+    if (e != cudaSuccess) KDE_FAIL(100 + (int)e, "gibbs (warp per chain) kernel launch: %s", cudaGetErrorString(e));
+  } else {
+    const size_t smem = GB_STAGES * GB_TILE_BYTES;
+    const cudaError_t e = with_d(d, [&](auto D) {
+      return launch_gibbs_d<decltype(D)::value>(P, masked, P.nbatches, smem, st, c.sm_count);
+    });
+    if (e != cudaSuccess) KDE_FAIL(100 + (int)e, "gibbs kernel launch: %s", cudaGetErrorString(e));
   }
-  if (gibbs_precision() == KDEB200_F32) {  // K1f: FP32 label probabilities (statistical mode only), gibbs_f32.cu
-    if (int rc = gibbs32_launch(trees, ndens, L, Niter, masked, P, st)) return rc;
-    if (launches) *launches += 1;
-    return 0;
-  }
-  const size_t smem = GB_STAGES * GB_TILE_BYTES;
-  cudaError_t e = cudaErrorInvalidValue;
-  switch (d) {
-#ifdef GB_ONLY_D3  // tuning builds: one instantiation
-    case 3: e = launch_gibbs_d<3>(P, masked, P.nbatches, smem, st, c.sm_count); break;
-#else
-    case 1: e = launch_gibbs_d<1>(P, masked, P.nbatches, smem, st, c.sm_count); break;
-    case 2: e = launch_gibbs_d<2>(P, masked, P.nbatches, smem, st, c.sm_count); break;
-    case 3: e = launch_gibbs_d<3>(P, masked, P.nbatches, smem, st, c.sm_count); break;
-    case 4: e = launch_gibbs_d<4>(P, masked, P.nbatches, smem, st, c.sm_count); break;
-    case 5: e = launch_gibbs_d<5>(P, masked, P.nbatches, smem, st, c.sm_count); break;
-    case 6: e = launch_gibbs_d<6>(P, masked, P.nbatches, smem, st, c.sm_count); break;
-    case 7: e = launch_gibbs_d<7>(P, masked, P.nbatches, smem, st, c.sm_count); break;
-    case 8: e = launch_gibbs_d<8>(P, masked, P.nbatches, smem, st, c.sm_count); break;
-#endif
-  }
-  if (e != cudaSuccess) KDE_FAIL(100 + (int)e, "gibbs kernel launch: %s", cudaGetErrorString(e));
   if (launches) *launches += 1;
   return 0;
 }

@@ -1,30 +1,20 @@
 // gibbs_f32.cu -- host side of K1f (FP32 Gibbs sampler): the FP32 pair records of a tree set under the call's shared affine
-// map, the schedule over them (cached like gibbs.cu's), launch.  The kernel lives in gibbs_f32_kernel.cuh and is
-// instantiated once per dimension in gibbs_f32_d<N>.cu.
+// map, the precision switch, launch.  The schedule is gibbs.cu's (cache) and gibbs_plan.cuh's (draws, chunks, tiles);
+// the kernel lives in gibbs_f32_kernel.cuh and is instantiated once per dimension in gibbs_f32_d<N>.cu.
 #include <atomic>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
-#include <list>
-#include <map>
-#include <mutex>
-#include <tuple>
 #include <vector>
 
-#include "gibbs_f32_kernel.cuh"
+#include "gibbs.cuh"
+#include "gibbs_plan.cuh"
 
 namespace kdeb200 {
 
-extern std::atomic<uint64_t> g_tree_epoch;
-
-extern template cudaError_t launch_gibbs_f32_d<1>(const GibbsParams &, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_f32_d<2>(const GibbsParams &, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_f32_d<3>(const GibbsParams &, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_f32_d<4>(const GibbsParams &, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_f32_d<5>(const GibbsParams &, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_f32_d<6>(const GibbsParams &, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_f32_d<7>(const GibbsParams &, int, size_t, cudaStream_t, int);
-extern template cudaError_t launch_gibbs_f32_d<8>(const GibbsParams &, int, size_t, cudaStream_t, int);
+#define GF_EXTERN(D) extern template cudaError_t launch_gibbs_f32_d<D>(const GibbsParams &, int, size_t, cudaStream_t, int);
+GF_EXTERN(1) GF_EXTERN(2) GF_EXTERN(3) GF_EXTERN(4) GF_EXTERN(5) GF_EXTERN(6) GF_EXTERN(7) GF_EXTERN(8)
+#undef GF_EXTERN
 
 // ---- FP64 level records -> FP32 pair records ----------------------------------------------------------------
 struct PrepDesc {
@@ -67,40 +57,8 @@ __global__ void gibbs_f32_prep_kernel(const PrepDesc *descs, int D, PrepMap mp) 
 
 // ---- host side ---------------------------------------------------------------------------------------------------
 namespace {
-struct Sched32 {
-  uint64_t epoch = 0;
-  int slot = 0, M = 0, T = 0;
-  bool masked = false;
-  kdeb200_tree_t trees[KDEB200_MAX_DENS] = {nullptr};
-  char *d_base = nullptr;  // draws | tiles | counters | FP32 records
-  Draw *d_draws = nullptr;
-  TileDesc *d_tiles = nullptr;
-  int *d_counters = nullptr;
-  int ndraws = 0, ntiles = 0;
-  unsigned next_counter = 0;
-  PrepMap map;
-  unsigned char mask[KDEB200_MAX_DENS][KDEB200_MAX_DIM];
-};
-constexpr int S32_COUNTERS = 256;
-constexpr size_t S32_KEEP = 4;
-std::mutex g32_mu;
-std::list<Sched32> g32_sched[KDEB200_MAX_GPUS];
-unsigned long long *g32_slow[KDEB200_MAX_GPUS] = {nullptr};
 std::atomic<int> g_gibbs_precision{KDEB200_F64};
-
-void s32_free(Sched32 &e, cudaStream_t st) {
-  if (e.d_base) cudaFreeAsync(e.d_base, st);
-  e.d_base = nullptr;
-}
 }  // namespace
-
-void gibbs32_drop_schedules(int slot) {
-  std::lock_guard<std::mutex> lk(g32_mu);
-  for (auto &e : g32_sched[slot]) s32_free(e, ctx_at(slot).stream);
-  g32_sched[slot].clear();
-  if (g32_slow[slot]) cudaFreeAsync(g32_slow[slot], ctx_at(slot).stream);
-  g32_slow[slot] = nullptr;
-}
 
 int gibbs_precision() {
   if (const char *ev = getenv("KDEB200_GIBBS_F32")) return atoi(ev) ? KDEB200_F32 : KDEB200_F64;
@@ -149,224 +107,60 @@ static int make_map(const kdeb200_tree_t *trees, int M, int d, const unsigned ch
   return 0;
 }
 
-static int s32_get(const kdeb200_tree_t *trees, int M, int L, int T, bool masked,
-                   const unsigned char (*mask)[KDEB200_MAX_DIM], Sched32 *out, int **counter) {
+// the FP32 pair records of every block of the plan, under the affine map of the entry's tree set and mask
+int gibbs32_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
   Context &c = ctx();
-  std::lock_guard<std::mutex> lk(g32_mu);
-  auto &lst = g32_sched[c.slot];
-  const uint64_t epoch = g_tree_epoch.load();
-  for (auto it = lst.begin(); it != lst.end();) {
-    if (it->epoch != epoch) {
-      s32_free(*it, c.stream);
-      it = lst.erase(it);
-    } else {
-      ++it;
-    }
-  }
-  for (auto it = lst.begin(); it != lst.end(); ++it) {
-    if (it->M != M || it->T != T || it->masked != masked) continue;
-    bool same = std::memcmp(it->mask, mask, sizeof(it->mask)) == 0;  // the affine map depends on the mask
-    for (int j = 0; j < M; ++j) same = same && it->trees[j] == trees[j];
-    if (!same) continue;
-    lst.splice(lst.begin(), lst, it);
-    *counter = it->d_counters + (it->next_counter++ % S32_COUNTERS);
-    *out = *it;
-    return 0;
-  }
   const int d = trees[0]->d;
-  Sched32 e;
-  if (int rc = make_map(trees, M, d, mask, e.map)) return rc;
-  std::memcpy(e.mask, mask, sizeof(e.mask));
-
-  // FP32 record blocks, one per (density slot, level, variant) the schedule touches
-  std::map<std::tuple<int, int, int>, size_t> block;  // -> offset in floats
+  PrepMap mp;
+  if (int rc = make_map(trees, e.M, d, e.mask, mp)) return rc;
+  std::memcpy(e.nctr, mp.ctr, sizeof(e.nctr));
+  std::memcpy(e.nisig, mp.isig, sizeof(e.nisig));
   std::vector<PrepDesc> preps;
-  std::vector<size_t> prep_off;
-  size_t nfloats = 0;
-  auto block_of = [&](int j, int li, int var) -> size_t {
-    const auto key = std::make_tuple(j, li, var);
-    auto it = block.find(key);
-    if (it != block.end()) return it->second;
-    const kdeb200_tree_s *t = trees[j];
-    const Level &lv = t->levels[li];
-    PrepDesc pd;
-    pd.src = t->d_buf + (var == VAR_A ? lv.offA : lv.offC);
-    pd.dst = nullptr;
-    pd.n = (int)lv.n;
-    pd.variant = var;
-    pd.src_stride = (var == VAR_A) ? t->SA : t->SC;
-    pd.dst_stride = gf_stride(d, var);
-    const size_t off = nfloats;
-    nfloats += (size_t)((lv.n + 1) / 2) * pd.dst_stride;
-    nfloats = (nfloats + 7) & ~(size_t)7;  // 32-byte aligned blocks: pass 2 reads them with 256-bit loads
-    preps.push_back(pd);
-    prep_off.push_back(off);
-    block[key] = off;
-    return off;
-  };
-  std::vector<Draw> draws;
-  struct TileRef { size_t off; uint32_t bytes; };
-  std::vector<TileRef> tiles;
-  std::vector<size_t> draw_off;
-  for (int l = 1; l <= L; ++l)
-    for (int pass = 0; pass <= T; ++pass)
-      for (int j = 0; j < M; ++j) {
-        const kdeb200_tree_s *t = trees[j];
-        const int li = l < t->depth ? l : t->depth;
-        const Level &lv = t->levels[li];
-        Draw dr;
-        std::memset(&dr, 0, sizeof(dr));
-        dr.j = (short)j;
-        dr.kind = pass == 0 ? 0 : 1;
-        dr.level = (short)l;
-        dr.new_level = (pass == 0 && j == 0) ? 1 : 0;
-        dr.n = (int)lv.n;
-        dr.wts = t->d_buf + lv.offW;
-        dr.levperm = t->d_levperm + lv.offP;
-        if (lv.cls == 0) {
-          dr.variant = VAR_A;
-          dr.rec_state = t->d_buf + lv.offA;
-          dr.state_stride = t->SA;
-          dr.state_has_bw = 0;
-        } else {
-          dr.variant = (pass == 0 && !masked) ? VAR_B : VAR_C;
-          dr.rec_state = t->d_buf + lv.offC;
-          dr.state_stride = t->SC;
-          dr.state_has_bw = 1;
-        }
-        dr.stride = gf_stride(d, dr.variant);
-        const size_t off = block_of(j, li, dr.variant);
-        int G = 2;
-        while ((int64_t)G * GB_MAXCK < lv.n) G *= 2;
-        const int want = 4 * gf_unr(d, dr.variant);  // at least two trips per chunk (x 1/2 and x 2 measured: +-1 %)
-        if (G < want && lv.n >= 2 * want) G = want;
-        dr.G = G;
-        dr.nchunks = (int)((lv.n + G - 1) / G);
-        int tn = 2;  // nodes per tile: the largest power of two whose pairs fit
-        while ((size_t)tn * dr.stride * sizeof(float) <= GB_TILE_BYTES) tn *= 2;
-        dr.tnodes = tn;
-        dr.ntiles = (int)((lv.n + tn - 1) / tn);
-        dr.tile0 = (int)tiles.size();
-        for (int qq = 0; qq < dr.ntiles; ++qq) {
-          const int64_t a = (int64_t)qq * tn;
-          const int64_t cnt = (lv.n - a < tn) ? (lv.n - a) : tn;
-          tiles.push_back(TileRef{off + (size_t)(a / 2) * dr.stride, (uint32_t)(((cnt + 1) / 2) * dr.stride * sizeof(float))});
-        }
-        draws.push_back(dr);
-        draw_off.push_back(off);
-      }
-
-  e.epoch = epoch;
-  e.slot = c.slot;
-  e.M = M;
-  e.T = T;
-  e.masked = masked;
-  for (int j = 0; j < M; ++j) e.trees[j] = trees[j];
-  e.ndraws = (int)draws.size();
-  e.ntiles = (int)tiles.size();
-  auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-  const size_t b_draws = up(sizeof(Draw) * draws.size()), b_tiles = up(sizeof(TileDesc) * tiles.size()),
-               b_cnt = up(sizeof(int) * S32_COUNTERS), b_prep = up(sizeof(PrepDesc) * preps.size()),
-               b_rec = up(sizeof(float) * nfloats);
-  KDE_CUDA(cudaMallocAsync(&e.d_base, b_draws + b_tiles + b_cnt + b_prep + b_rec, c.stream));
-  e.d_draws = reinterpret_cast<Draw *>(e.d_base);
-  e.d_tiles = reinterpret_cast<TileDesc *>(e.d_base + b_draws);
-  e.d_counters = reinterpret_cast<int *>(e.d_base + b_draws + b_tiles);
-  PrepDesc *d_prep = reinterpret_cast<PrepDesc *>(e.d_base + b_draws + b_tiles + b_cnt);
-  float *d_rec = reinterpret_cast<float *>(e.d_base + b_draws + b_tiles + b_cnt + b_prep);
-  std::vector<TileDesc> tds(tiles.size());
-  for (size_t i = 0; i < tiles.size(); ++i) {
-    tds[i].src = reinterpret_cast<const double *>(d_rec + tiles[i].off);
-    tds[i].bytes = tiles[i].bytes;
-    tds[i].pad = 0;
-  }
-  for (size_t i = 0; i < draws.size(); ++i) draws[i].rec = reinterpret_cast<const double *>(d_rec + draw_off[i]);
   int maxpairs = 1;
-  for (size_t i = 0; i < preps.size(); ++i) {
-    preps[i].dst = d_rec + prep_off[i];
-    if ((preps[i].n + 1) / 2 > maxpairs) maxpairs = (preps[i].n + 1) / 2;
+  for (const PlanBlock &b : S.blocks) {
+    const kdeb200_tree_s *t = trees[b.j];
+    const Level &lv = t->levels[b.level];
+    PrepDesc pd;
+    pd.src = t->d_buf + (b.variant == VAR_A ? lv.offA : lv.offC);
+    pd.dst = e.d_rec + b.off;
+    pd.n = (int)lv.n;
+    pd.variant = b.variant;
+    pd.src_stride = (b.variant == VAR_A) ? t->SA : t->SC;
+    pd.dst_stride = gf_stride(d, b.variant);
+    if ((pd.n + 1) / 2 > maxpairs) maxpairs = (pd.n + 1) / 2;
+    preps.push_back(pd);
   }
-  cudaError_t err = cudaMemcpyAsync(e.d_draws, draws.data(), sizeof(Draw) * draws.size(), cudaMemcpyHostToDevice, c.stream);
-  if (err == cudaSuccess) err = cudaMemcpyAsync(e.d_tiles, tds.data(), sizeof(TileDesc) * tds.size(), cudaMemcpyHostToDevice, c.stream);
-  if (err == cudaSuccess) err = cudaMemcpyAsync(d_prep, preps.data(), sizeof(PrepDesc) * preps.size(), cudaMemcpyHostToDevice, c.stream);
-  if (err == cudaSuccess) err = cudaMemsetAsync(e.d_counters, 0, b_cnt, c.stream);
+  for (size_t i = 0; i < S.draws.size(); ++i) {  // K1f reads every level from its pair records
+    S.draws[i].rec = reinterpret_cast<const double *>(e.d_rec + S.blocks[S.block[i]].off);
+    S.draws[i].stride = gf_stride(d, S.draws[i].variant);
+  }
+  PrepDesc *d_prep = nullptr;
+  KDE_CUDA(cudaMallocAsync(&d_prep, sizeof(PrepDesc) * preps.size(), c.stream));
+  cudaError_t err = cudaMemcpyAsync(d_prep, preps.data(), sizeof(PrepDesc) * preps.size(), cudaMemcpyHostToDevice, c.stream);
   if (err == cudaSuccess) {
-    gibbs_f32_prep_kernel<<<dim3((unsigned)((maxpairs + 127) / 128), (unsigned)preps.size()), 128, 0, c.stream>>>(d_prep, d, e.map);
+    gibbs_f32_prep_kernel<<<dim3((unsigned)((maxpairs + 127) / 128), (unsigned)preps.size()), 128, 0, c.stream>>>(d_prep, d, mp);
     err = cudaGetLastError();
   }
-  if (err == cudaSuccess) err = cudaStreamSynchronize(c.stream);
-  if (err != cudaSuccess) {
-    cudaFreeAsync(e.d_base, c.stream);
-    KDE_FAIL(100 + (int)err, "gibbs (FP32): building the schedule: %s", cudaGetErrorString(err));
-  }
-  lst.push_front(e);
-  while (lst.size() > S32_KEEP) {
-    cudaDeviceSynchronize();
-    s32_free(lst.back(), c.stream);
-    lst.pop_back();
-  }
-  *counter = lst.front().d_counters + (lst.front().next_counter++ % S32_COUNTERS);
-  *out = lst.front();
+  if (err == cudaSuccess) err = cudaStreamSynchronize(c.stream);  // preps is pageable host memory
+  cudaFreeAsync(d_prep, c.stream);
+  if (err != cudaSuccess) KDE_FAIL(100 + (int)err, "gibbs (FP32): building the schedule: %s", cudaGetErrorString(err));
   return 0;
 }
 
-static int slow_counter(unsigned long long **out) {
+// P arrives filled by gibbs_device with the entry's schedule; this adds the affine map and the slow-draw counter
+int gibbs32_launch(GibbsParams &P, const SchedEntry &E, int d, cudaStream_t st) {
   Context &c = ctx();
-  std::lock_guard<std::mutex> lk(g32_mu);
-  if (!g32_slow[c.slot]) {
-    KDE_CUDA(cudaMallocAsync(&g32_slow[c.slot], sizeof(unsigned long long), c.stream));
-    KDE_CUDA(cudaMemsetAsync(g32_slow[c.slot], 0, sizeof(unsigned long long), c.stream));
-    KDE_CUDA(cudaStreamSynchronize(c.stream));
-  }
-  *out = g32_slow[c.slot];
-  return 0;
-}
-
-// draws redone in FP64 on the calling context's device since the last call of this function (synchronises the device)
-int gibbs32_slow_draws(unsigned long long *out) {
-  unsigned long long *d = nullptr;
-  if (int rc = slow_counter(&d)) return rc;
-  KDE_CUDA(cudaDeviceSynchronize());
-  KDE_CUDA(cudaMemcpy(out, d, sizeof(*out), cudaMemcpyDeviceToHost));
-  KDE_CUDA(cudaMemset(d, 0, sizeof(*out)));
-  return 0;
-}
-
-// P arrives filled by gibbs_device (streams, outputs, masks, root records, labels, sizes); this adds the FP32 schedule
-int gibbs32_launch(const kdeb200_tree_t *trees, int ndens, int L, int Niter, bool masked, GibbsParams &P, cudaStream_t st) {
-  Context &c = ctx();
-  const int d = trees[0]->d;
-  Sched32 E;
-  int *d_counter = nullptr;
-  if (int rc = s32_get(trees, ndens, L, Niter, masked, P.mask, &E, &d_counter)) return rc;
-  unsigned long long *d_slow = nullptr;
-  if (int rc = slow_counter(&d_slow)) return rc;
-  P.draws = E.d_draws;
-  P.tiles = E.d_tiles;
-  P.counter = d_counter;
-  P.ndraws = E.ndraws;
-  P.ntiles = E.ntiles;
-  P.slow_draws = d_slow;
+  unsigned long long *d_count = nullptr;
+  if (int rc = gibbs_counters(&d_count)) return rc;
+  P.slow_draws = d_count;
   for (int k = 0; k < KDEB200_MAX_DIM; ++k) {
-    P.nctr[k] = E.map.ctr[k];
-    P.nisig[k] = E.map.isig[k];
+    P.nctr[k] = E.nctr[k];
+    P.nisig[k] = E.nisig[k];
   }
   const size_t smem = GB_STAGES * GB_TILE_BYTES;
-  cudaError_t e = cudaErrorInvalidValue;
-  switch (d) {
-#ifdef GF_ONLY_D3  // tuning builds: one instantiation
-    case 3: e = launch_gibbs_f32_d<3>(P, P.nbatches, smem, st, c.sm_count); break;
-#else
-    case 1: e = launch_gibbs_f32_d<1>(P, P.nbatches, smem, st, c.sm_count); break;
-    case 2: e = launch_gibbs_f32_d<2>(P, P.nbatches, smem, st, c.sm_count); break;
-    case 3: e = launch_gibbs_f32_d<3>(P, P.nbatches, smem, st, c.sm_count); break;
-    case 4: e = launch_gibbs_f32_d<4>(P, P.nbatches, smem, st, c.sm_count); break;
-    case 5: e = launch_gibbs_f32_d<5>(P, P.nbatches, smem, st, c.sm_count); break;
-    case 6: e = launch_gibbs_f32_d<6>(P, P.nbatches, smem, st, c.sm_count); break;
-    case 7: e = launch_gibbs_f32_d<7>(P, P.nbatches, smem, st, c.sm_count); break;
-    case 8: e = launch_gibbs_f32_d<8>(P, P.nbatches, smem, st, c.sm_count); break;
-#endif
-  }
+  const cudaError_t e = with_d(d, [&](auto D) {
+    return launch_gibbs_f32_d<decltype(D)::value>(P, P.nbatches, smem, st, c.sm_count);
+  });
   if (e != cudaSuccess) KDE_FAIL(100 + (int)e, "gibbs (FP32) kernel launch: %s", cudaGetErrorString(e));
   return 0;
 }

@@ -18,7 +18,7 @@
 #include <type_traits>
 #include <vector>
 
-#include "tree.cuh"
+#include "gibbs.cuh"
 
 namespace kdeb200 {
 
@@ -574,8 +574,6 @@ int tree_on(kdeb200_tree_t t, int slot, kdeb200_tree_t *out) {
   *out = r;
   return 0;
 }
-
-void gibbs_invalidate_schedules();  // gibbs.cu: cached schedules hold pointers into tree records
 
 int tree_destroy(kdeb200_tree_t t) {
   if (!t) return 0;

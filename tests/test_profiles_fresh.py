@@ -1,6 +1,6 @@
-"""The issued-instruction / DRAM-traffic figures that bench.py quotes come from profiles/ncu_issued.json, keyed by a hash
-of the kernel sources (tools/ncu_issued.py).  A kernel change without a new capture must fail loudly here, not let the
-bench line carry stale numbers (VERDICT r1: a hard-coded count had gone stale silently)."""
+"""The issued-instruction / DRAM-traffic figures that bench.py quotes come from profiles/ncu_issued.json, keyed by the
+profiled kernels' compiled code and launch sources (build.kernel_source_hash, tools/ncu_issued.py).  A kernel change
+without a new capture must fail loudly here, not let the bench line carry stale numbers (VERDICT r1: a hard-coded count had gone stale silently)."""
 import json
 import os
 

@@ -1,4 +1,5 @@
-"""Machine-readable issued-instruction / DRAM-traffic summary of the hot kernels, keyed by source hash.
+"""Machine-readable issued-instruction / DRAM-traffic summary of the hot kernels, keyed by build.kernel_source_hash
+(the profiled kernels' SASS and resource usage as compiled, plus their launch sources).
 
 Run ON THE GPU BOX right after the metric captures, so that the hashes describe the sources that were profiled:
 

@@ -11,5 +11,5 @@ for a in sys.argv[1:]:
     tag, defs = a.split(":")
     jobs.append((tag, ["GF_ONLY_D3"] + [d for d in defs.split(",") if d]))
 with ThreadPoolExecutor(max_workers=6) as ex:
-    for r in ex.map(lambda j: b.build_variant(j[0], j[1], tuned=["gibbs_f32.cu", "gibbs_f32_d3.cu"]), jobs):
+    for r in ex.map(lambda j: b.build_variant(*j), jobs):
         print("built", r)

@@ -124,6 +124,42 @@ int kdeb200_gibbs_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int
 int kdeb200_product_kde(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, int add_entropy,
                         const uint8_t *dimmask, uint64_t seed, double *points_out, int64_t *indices_out,
                         double *bw_std_out, int *nloo_calls_out);
+/* nprob independent prodAppxMSGibbsS problems (src/MSGibbs01.jl:645-703) in one blocking call (K1b: one launch per
+ * dimension and mask class, one CTA per 128 samples of one problem).  Problems are concatenated in order:
+ *   ndens[i]           densities of problem i (1..KDEB200_MAX_DENS)
+ *   trees              sum(ndens) handles, problem by problem; every problem's trees share its d (d may differ between
+ *                      problems); one handle may serve several problems
+ *   Np[i]              samples of problem i (0 allowed)
+ *   dimmask            NULL, or sum(ndens[i]*d_i) bytes, problem by problem, as kdeb200_gibbs's dimmask
+ *   randU/nU, randN/nN NULL, or concatenated per-problem streams with per-problem lengths; nU[i] == nN[i] == 0 means
+ *                      problem i draws from Philox4x32-10(seeds[i]); otherwise addressed exactly as kdeb200_gibbs does
+ *   seeds              nprob seeds (read only for Philox problems)
+ *   points_out         sum(d_i*Np[i]) doubles: problem i's block is laid out as kdeb200_gibbs's points_out
+ *   indices_out        sum(ndens[i]*Np[i]) int64: likewise (permutation + 1)
+ * Always FP64 (kdeb200_set_gibbs_precision does not apply).  Every problem's outputs are bit for bit those of
+ * kdeb200_gibbs called alone with the same arguments on the thread-per-chain kernel; against the warp-per-chain
+ * kernel that small single calls use, labels are identical and points agree to 1e-10.  Problems with a degenerate
+ * bandwidth run the single call's verbatim arithmetic and match it exactly; they go through the single-call path one
+ * by one (its schedule cache included, which synchronises when it builds or evicts an entry), so many distinct
+ * degenerate tree sets in one batch run serially after the batched launches.  Every problem is checked before anything
+ * runs, with the single call's error codes; the message names the problem.  Under kdeb200_init_multi the whole batch
+ * runs on the primary GPU.  kdeb200_last_kernel_ms covers all of the call's launches. */
+int kdeb200_gibbs_batch(int nprob, const int *ndens, const kdeb200_tree_t *trees, const int64_t *Np, int Niter,
+                        int add_entropy, const uint8_t *dimmask, const double *randU, const int64_t *nU,
+                        const double *randN, const int64_t *nN, const uint64_t *seeds,
+                        double *points_out, int64_t *indices_out);
+/* `*` for nprob problems (src/MSGibbs01.jl:707-726): the Gibbs step of kdeb200_gibbs_batch (Philox), then each
+ * problem's LOOCV refit as kdeb200_product_kde does it -- problems with Np <= 512 in one launch of one CTA per
+ * (problem, dimension), larger ones by the host bandwidth loop after the batch.  Equal outputs to kdeb200_product_kde
+ * under the same kernel, as above.  Np[i] >= 2.  bw_std_out and nloo_calls_out hold sum(d_i) entries; indices_out and
+ * nloo_calls_out may be NULL. */
+int kdeb200_product_kde_batch(int nprob, const int *ndens, const kdeb200_tree_t *trees, const int64_t *Np, int Niter,
+                              int add_entropy, const uint8_t *dimmask, const uint64_t *seeds, double *points_out,
+                              int64_t *indices_out, double *bw_std_out, int *nloo_calls_out);
+/* Diagnostic, like kdeb200_last_kernel_ms: where the last batch call (on the primary GPU) spent its time outside the
+ * kernels, in ms (any pointer may be NULL): host checks, schedule assembly and packing; the one host-to-device copy;
+ * the device-to-host copies.  The kernels are kdeb200_last_kernel_ms. */
+int kdeb200_gibbs_batch_split(double *plan_ms, double *h2d_ms, double *d2h_ms);
 /* Arithmetic of the label probabilities in kdeb200_gibbs / _gibbs_device / _product_kde (process-wide; default KDEB200_F64;
  * the environment variable KDEB200_GIBBS_F32=1/0 overrides):
  *   KDEB200_F64  parity mode (a): labels identical to the reference under injected variates.

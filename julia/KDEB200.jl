@@ -199,6 +199,83 @@ function product(trees::Vector{BallTreeDensity}; addEntropy::Bool=true, Niter::I
   return kde!(pts, bw)
 end
 
+# Many independent gibbs1 problems in one call (kdeb200_gibbs_batch: one launch per dimension, one CTA per 128 samples).
+# tree_lists[i], Np[i]: problem i.  pts[i] (d_i*Np[i]) and ind[i] (Ndens_i x Np[i]) are filled in place, each equal to
+# gibbs1!'s result for that problem alone.  partialDimMasks, randU, randN: nothing, or one entry (or nothing) per problem;
+# a problem without streams draws from Philox(seeds[i]).
+function gibbs1_batch!(tree_lists::Vector{Vector{BallTreeDensity}}, Np::Vector{Int}, Niter::Int,
+                       pts::Vector{Vector{Float64}}, ind::Vector{Matrix{Int}};
+                       addEntropy::Bool=true, partialDimMasks=nothing, randU=nothing, randN=nothing,
+                       seeds::Vector{UInt64}=rand(UInt64, length(tree_lists)))
+  n = length(tree_lists)
+  ndens = Cint[length(ts) for ts in tree_lists]
+  dims = [Ndim(ts[1]) for ts in tree_lists]
+  dts = [DeviceTree(t) for ts in tree_lists for t in ts]
+  hs = Ptr{Cvoid}[d.h for d in dts]
+  mask = partialDimMasks === nothing ? UInt8[] :
+    reduce(vcat, [m === nothing ? ones(UInt8, ndens[i] * dims[i]) :
+                  UInt8[m[j][k] ? 0x01 : 0x00 for k in 1:dims[i], j in 1:ndens[i]] for (i, m) in enumerate(partialDimMasks)])
+  U = randU === nothing ? Float64[] : reduce(vcat, [u === nothing ? Float64[] : u for u in randU]; init=Float64[])
+  G = randN === nothing ? Float64[] : reduce(vcat, [g === nothing ? Float64[] : g for g in randN]; init=Float64[])
+  nU = randU === nothing ? Int64[] : Int64[u === nothing ? 0 : length(u) for u in randU]
+  nN = randN === nothing ? Int64[] : Int64[g === nothing ? 0 : length(g) for g in randN]
+  P = zeros(sum(dims .* Np)); I = zeros(Int64, sum(ndens .* Np))
+  GC.@preserve dts hs mask U G nU nN P I begin
+    check(ccall((:kdeb200_gibbs_batch, LIB), Cint,
+                (Cint, Ptr{Cint}, Ptr{Ptr{Cvoid}}, Ptr{Int64}, Cint, Cint, Ptr{UInt8}, Ptr{Float64}, Ptr{Int64},
+                 Ptr{Float64}, Ptr{Int64}, Ptr{UInt64}, Ptr{Float64}, Ptr{Int64}),
+                n, ndens, hs, Int64.(Np), Niter, addEntropy, partialDimMasks === nothing ? C_NULL : mask,
+                randU === nothing ? C_NULL : U, randU === nothing ? C_NULL : nU,
+                randN === nothing ? C_NULL : G, randN === nothing ? C_NULL : nN, seeds, P, I))
+  end
+  p0 = 0; i0 = 0
+  for i in 1:n
+    pts[i] .= P[p0+1:p0+dims[i]*Np[i]]
+    ind[i] .= reshape(I[i0+1:i0+ndens[i]*Np[i]], Int(ndens[i]), Np[i])
+    p0 += dims[i] * Np[i]; i0 += ndens[i] * Np[i]
+  end
+  nothing
+end
+
+# [product(ts; addEntropy, seed=s) for (ts, s) in zip(tree_lists, seeds)] with the Gibbs steps and the LOOCV refits in
+# one call (kdeb200_product_kde_batch); what `*` answers on the host (one density without entropy, fewer than two
+# product samples) is answered the same way here.
+function product_batch(tree_lists::Vector{Vector{BallTreeDensity}}; addEntropy::Bool=true,
+                       seeds::Vector{UInt64}=rand(UInt64, length(tree_lists)))
+  res = Vector{BallTreeDensity}(undef, length(tree_lists))
+  dev = Int[]
+  for (i, ts) in enumerate(tree_lists)
+    numpts = round(Int, sum(Npts.(ts)) / length(ts))
+    if length(ts) == 1 && !addEntropy
+      res[i] = kde!(getPoints(ts[1]))
+    elseif numpts < 2
+      d = Ndim(ts[1]); pts = zeros(d * numpts); ind = zeros(Int, length(ts), numpts)
+      gibbs1!(length(ts), ts, numpts, 5, pts, ind, nothing, nothing; addEntropy=addEntropy, seed=seeds[i])
+      res[i] = kde!(reshape(pts, d, numpts))
+    else
+      push!(dev, i)
+    end
+  end
+  isempty(dev) && return res
+  ndens = Cint[length(tree_lists[i]) for i in dev]
+  dims = [Ndim(tree_lists[i][1]) for i in dev]
+  Np = Int64[round(Int, sum(Npts.(tree_lists[i])) / length(tree_lists[i])) for i in dev]
+  dts = [DeviceTree(t) for i in dev for t in tree_lists[i]]
+  hs = Ptr{Cvoid}[d.h for d in dts]
+  sd = seeds[dev]
+  P = zeros(sum(dims .* Np)); bw = zeros(sum(dims))
+  GC.@preserve dts hs sd P bw check(ccall((:kdeb200_product_kde_batch, LIB), Cint,
+    (Cint, Ptr{Cint}, Ptr{Ptr{Cvoid}}, Ptr{Int64}, Cint, Cint, Ptr{UInt8}, Ptr{UInt64}, Ptr{Float64}, Ptr{Int64},
+     Ptr{Float64}, Ptr{Cint}),
+    length(dev), ndens, hs, Np, 5, addEntropy, C_NULL, sd, P, C_NULL, bw, C_NULL))
+  p0 = 0; b0 = 0
+  for (k, i) in enumerate(dev)
+    res[i] = kde!(reshape(P[p0+1:p0+dims[k]*Np[k]], dims[k], Np[k]), bw[b0+1:b0+dims[k]])
+    p0 += dims[k] * Np[k]; b0 += dims[k]
+  end
+  return res
+end
+
 # sample(npd, Npts) (src/KDE01.jl:164-183) on the device; Philox(seed) variates (Julia's RNG streams can be injected as
 # randU (Npts) / randN (d x Npts) through the C entry point directly)
 function sample(npd::BallTreeDensity, Np::Int; seed::UInt64=rand(UInt64))

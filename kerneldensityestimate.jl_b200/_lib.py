@@ -40,6 +40,11 @@ SIGNATURES = {
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "kdeb200_product_kde": (C.c_int, [C.POINTER(tree_t), C.c_int, C.c_int64, C.c_int, C.c_int, u8p, C.c_uint64, f64p, i64p, f64p,
                                       C.POINTER(C.c_int)]),
+    "kdeb200_gibbs_batch": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(tree_t), i64p, C.c_int, C.c_int, u8p, f64p, i64p,
+                                      f64p, i64p, C.POINTER(C.c_uint64), f64p, i64p]),
+    "kdeb200_product_kde_batch": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(tree_t), i64p, C.c_int, C.c_int, u8p,
+                                            C.POINTER(C.c_uint64), f64p, i64p, f64p, C.POINTER(C.c_int)]),
+    "kdeb200_gibbs_batch_split": (C.c_int, [f64p, f64p, f64p]),
     "kdeb200_gibbs_sizes": (C.c_int, [C.POINTER(tree_t), C.c_int, C.c_int, C.POINTER(C.c_int), i64p, i64p, i64p]),
     "kdeb200_philox_streams": (C.c_int, [C.c_uint64, C.c_int64, C.c_int64, C.c_int64, f64p, f64p]),
     "kdeb200_eval": (C.c_int, [tree_t, f64p, C.c_int64, C.c_int, C.c_int, f64p]),

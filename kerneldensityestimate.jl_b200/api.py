@@ -28,7 +28,7 @@ from ._lib import KDEError, check, fptr, iptr, lib
 __all__ = [
     "KDEError", "BallTree", "BallTreeDensity", "kde", "kde_bang", "getPoints", "getBW", "getWeights", "marginal",
     "sample", "rand", "resample", "evaluateDualTree", "evalAvgLogL", "entropy", "kld", "minkld", "nLOO_LL", "golden",
-    "ksize", "neighborMinMax", "lcv_bandwidths", "updateBandwidth", "prodAppxMSGibbsS", "Ndim", "Npts", "init", "init_multi", "multi_count", "gibbs_sizes",
+    "ksize", "neighborMinMax", "lcv_bandwidths", "updateBandwidth", "prodAppxMSGibbsS", "prodAppxMSGibbsS_batch", "prod_batch", "gibbs_batch_split", "Ndim", "Npts", "init", "init_multi", "multi_count", "gibbs_sizes",
     "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
     "getKDEMax", "getKDEMean", "getKDEfit", "intersIntgAppxIS", "eval_marginals", "to_string", "from_string",
 ]
@@ -752,6 +752,113 @@ def prod(trees, glbs=None, addEntropy=True, seed=None, recordLabels=False):
     check(lib().kdeb200_product_kde(_handles(trees), len(trees), numpts, 5, int(bool(addEntropy)), None,
                                     int(seed) & 0xFFFFFFFFFFFFFFFF, fptr(pts), None, fptr(bw), None))
     return kde(pts.T, bw)
+
+
+def _batch_handles(tree_lists):
+    lists = [list(t) for t in tree_lists]
+    ndens = np.array([len(t) for t in lists], dtype=np.int32)
+    flat = [t for ts in lists for t in ts]
+    for i, ts in enumerate(lists):
+        if ts and any(Ndim(t) != Ndim(ts[0]) for t in ts):
+            raise KDEError("problem %d: kdes must have same dimension" % i)
+    dims = [Ndim(ts[0]) if ts else 0 for ts in lists]
+    return lists, ndens, _handles(flat), dims
+
+
+def _seeds(seeds, n):
+    if seeds is None:
+        return np.frombuffer(os.urandom(8 * n), dtype=np.uint64).copy() if n else np.zeros(0, dtype=np.uint64)
+    s = np.array([int(x) & 0xFFFFFFFFFFFFFFFF for x in seeds], dtype=np.uint64)
+    if s.size != n:
+        raise KDEError("need one seed per problem")
+    return s
+
+
+def prodAppxMSGibbsS_batch(tree_lists, Np, Niter=3, addEntropy=True, partialDimMasks=None, randU=None, randN=None,
+                           seeds=None):
+    """Many independent prodAppxMSGibbsS problems in one library call (kdeb200_gibbs_batch, one launch per dimension).
+
+    tree_lists[i] are the densities of problem i and Np[i] its number of samples.  partialDimMasks, randU, randN are
+    None or one entry per problem (an entry may be None: all dimensions, resp. Philox(seeds[i])).  Returns a list of
+    (points d x Np, indices Ndens x Np), each equal to what prodAppxMSGibbsS returns for that problem alone."""
+    lists, ndens, handles, dims = _batch_handles(tree_lists)
+    n = len(lists)
+    Np = np.array([int(x) for x in Np], dtype=np.int64)
+    if Np.size != n:
+        raise KDEError("need one Np per problem")
+    mask = None
+    if partialDimMasks is not None:
+        if len(partialDimMasks) != n:
+            raise KDEError("need one partialDimMask (or None) per problem")
+        mask = np.concatenate([np.ones(ndens[i] * dims[i], dtype=np.uint8) if m is None else
+                               np.asarray(m, dtype=bool).reshape(ndens[i], dims[i]).astype(np.uint8).ravel()
+                               for i, m in enumerate(partialDimMasks)] or [np.zeros(0, dtype=np.uint8)])
+    U = G = nU = nN = None
+    if (randU is None) != (randN is None):
+        raise KDEError("prodAppxMSGibbsS_batch: pass both randU and randN or neither")
+    if randU is not None:
+        if len(randU) != n or len(randN) != n:
+            raise KDEError("need one randU / randN entry (or None) per problem")
+        us = [np.zeros(0) if u is None else np.ascontiguousarray(u, dtype=np.float64).ravel() for u in randU]
+        gs = [np.zeros(0) if g is None else np.ascontiguousarray(g, dtype=np.float64).ravel() for g in randN]
+        nU = np.array([u.size for u in us], dtype=np.int64)
+        nN = np.array([g.size for g in gs], dtype=np.int64)
+        U = np.concatenate(us + [np.zeros(1)])
+        G = np.concatenate(gs + [np.zeros(1)])
+    sd = _seeds(seeds, n)
+    points = np.zeros(int(sum(dims[i] * Np[i] for i in range(n))) + 1)
+    indices = np.zeros(int(sum(ndens[i] * Np[i] for i in range(n))) + 1, dtype=np.int64)
+    check(lib().kdeb200_gibbs_batch(n, ndens.ctypes.data_as(C.POINTER(C.c_int)), handles, iptr(Np), int(Niter),
+                                    int(bool(addEntropy)), None if mask is None else mask.ctypes.data_as(_lib.u8p),
+                                    fptr(U), iptr(nU), fptr(G), iptr(nN), sd.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                    fptr(points), iptr(indices)))
+    out, p0, i0 = [], 0, 0
+    for i in range(n):
+        d, M, m = dims[i], int(ndens[i]), int(Np[i])
+        out.append((points[p0:p0 + d * m].reshape(m, d).T.copy(), indices[i0:i0 + M * m].reshape(m, M).T.copy()))
+        p0 += d * m
+        i0 += M * m
+    return out
+
+
+def prod_batch(tree_lists, addEntropy=True, seeds=None):
+    """[prod(trees, addEntropy=addEntropy, seed=s) for trees, s in zip(tree_lists, seeds)] with the Gibbs steps and the
+    LOOCV refits of all problems in one library call (kdeb200_product_kde_batch).  The problems prod answers on the host
+    (one density without entropy, fewer than two product samples) are answered the same way here."""
+    lists = [list(t) for t in tree_lists]
+    n = len(lists)
+    sd = _seeds(seeds, n)
+    res = [None] * n
+    dev = []
+    for i, ts in enumerate(lists):
+        numpts = int(round(float(np.mean([Npts(t) for t in ts])))) if ts else 0
+        if (len(ts) == 1 and not addEntropy) or numpts < 2:
+            res[i] = prod(ts, addEntropy=addEntropy, seed=int(sd[i]))
+        else:
+            dev.append((i, numpts))
+    if dev:
+        lists_d, ndens, handles, dims = _batch_handles([lists[i] for i, _ in dev])
+        Np = np.array([m for _, m in dev], dtype=np.int64)
+        sdd = np.ascontiguousarray(sd[[i for i, _ in dev]])
+        pts = np.zeros(int(sum(dims[k] * Np[k] for k in range(len(dev)))))
+        bw = np.zeros(int(sum(dims)))
+        check(lib().kdeb200_product_kde_batch(len(dev), ndens.ctypes.data_as(C.POINTER(C.c_int)), handles, iptr(Np), 5,
+                                              int(bool(addEntropy)), None, sdd.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                              fptr(pts), None, fptr(bw), None))
+        p0 = b0 = 0
+        for k, (i, m) in enumerate(dev):
+            d = dims[k]
+            res[i] = kde(pts[p0:p0 + d * m].reshape(m, d).T, bw[b0:b0 + d])
+            p0 += d * m
+            b0 += d
+    return res
+
+
+def gibbs_batch_split():
+    """(host checks + planning + packing, host-to-device copy, device-to-host copies) of the last batch call, in ms."""
+    a, b, c = C.c_double(0), C.c_double(0), C.c_double(0)
+    check(lib().kdeb200_gibbs_batch_split(C.byref(a), C.byref(b), C.byref(c)))
+    return a.value, b.value, c.value
 
 
 # ------------------------------------------------------------------------- measurement -------

@@ -49,19 +49,6 @@ int dfma_probe(int ilp, int blocks_per_sm, int threads, int iters, double *lane_
 static std::recursive_mutex g_call_mu;
 #define KDE_SERIALISE() std::lock_guard<std::recursive_mutex> kde_lock__(::kdeb200::g_call_mu)
 
-// RAII device buffer on a stream
-struct DevBuf {
-  void *p = nullptr;
-  cudaStream_t st;
-  explicit DevBuf(cudaStream_t s) : st(s) {}
-  cudaError_t alloc(size_t bytes) { return cudaMallocAsync(&p, bytes ? bytes : 16, st); }
-  ~DevBuf() {
-    if (p) cudaFreeAsync(p, st);
-  }
-  template <class T>
-  T *as() { return static_cast<T *>(p); }
-};
-
 struct Timer {  // CUDA-event bracket on the library stream, result readable via kdeb200_last_kernel_ms
   Context &c;
   explicit Timer(Context &cc) : c(cc) {
@@ -534,6 +521,40 @@ int kdeb200_product_kde(const kdeb200_tree_t *trees, int ndens, int64_t Np, int 
   int rc = kde_lcv(d, Np, points_out, 0, Np, nullptr, nullptr, bw_std_out, nloo_calls_out);
   c.last_ms += ms_gibbs;
   return rc;
+}
+
+int kdeb200_gibbs_batch(int nprob, const int *ndens, const kdeb200_tree_t *trees, const int64_t *Np, int Niter,
+                        int add_entropy, const uint8_t *dimmask, const double *randU, const int64_t *nU,
+                        const double *randN, const int64_t *nN, const uint64_t *seeds, double *points_out,
+                        int64_t *indices_out) {
+  KDE_SERIALISE();
+  if (int rc = ensure_init()) return rc;
+  if (nprob < 0) KDE_FAIL(3, "gibbs_batch: nprob=%d < 0", nprob);
+  if (nprob == 0) return 0;
+  if (!ndens || !trees || !Np || !points_out || !indices_out) KDE_FAIL(2, "gibbs_batch: NULL argument");
+  ScopedDevice sd(0);
+  const GibbsBatchArgs a{nprob, ndens, trees, Np, Niter, add_entropy, dimmask, randU, nU, randN, nN, seeds};
+  return gibbs_batch(a, points_out, indices_out, nullptr, nullptr);
+}
+
+int kdeb200_product_kde_batch(int nprob, const int *ndens, const kdeb200_tree_t *trees, const int64_t *Np, int Niter,
+                              int add_entropy, const uint8_t *dimmask, const uint64_t *seeds, double *points_out,
+                              int64_t *indices_out, double *bw_std_out, int *nloo_calls_out) {
+  KDE_SERIALISE();
+  if (int rc = ensure_init()) return rc;
+  if (nprob < 0) KDE_FAIL(3, "product_kde_batch: nprob=%d < 0", nprob);
+  if (nprob == 0) return 0;
+  if (!ndens || !trees || !Np || !seeds || !points_out || !bw_std_out) KDE_FAIL(2, "product_kde_batch: NULL argument");
+  ScopedDevice sd(0);
+  const GibbsBatchArgs a{nprob, ndens, trees, Np, Niter, add_entropy, dimmask, nullptr, nullptr, nullptr, nullptr, seeds};
+  return gibbs_batch(a, points_out, indices_out, bw_std_out, nloo_calls_out);
+}
+
+int kdeb200_gibbs_batch_split(double *plan_ms, double *h2d_ms, double *d2h_ms) {
+  KDE_SERIALISE();
+  if (int rc = ensure_init()) return rc;
+  ScopedDevice sd(0);
+  return gibbs_batch_split(plan_ms, h2d_ms, d2h_ms);
 }
 
 int kdeb200_eval_marginals(kdeb200_tree_t bd, const double *grids, int64_t G, double *out) {

@@ -48,6 +48,7 @@ static void drop_context(Context &c) {
   cudaSetDevice(c.device);
   cudaDeviceSynchronize();
   gibbs_drop_schedules(c.slot);
+  gibbs_batch_drop(c.slot);
   cudaStreamSynchronize(c.stream);
   cudaFree(c.d_exptab);
   cudaEventDestroy(c.ev0);

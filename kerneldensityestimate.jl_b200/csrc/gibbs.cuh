@@ -31,6 +31,25 @@ int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, 
 void gibbs_invalidate_schedules();  // a tree is destroyed: cached schedules point into tree records
 void gibbs_drop_schedules(int slot);  // a context goes away: frees its schedules and counters
 
+// ---- batched problems (gibbs_batch.cu): the arguments of kdeb200_gibbs_batch, problem by problem
+struct GibbsBatchArgs {
+  int nprob;
+  const int *ndens;
+  const kdeb200_tree_t *trees;
+  const int64_t *Np;
+  int Niter, add_entropy;
+  const uint8_t *dimmask;
+  const double *randU;
+  const int64_t *nU;
+  const double *randN;
+  const int64_t *nN;
+  const uint64_t *seeds;
+};
+// Blocking, on the calling context.  bw_std_out != null adds the LOOCV refit of kdeb200_product_kde_batch.
+int gibbs_batch(const GibbsBatchArgs &a, double *points_out, int64_t *indices_out, double *bw_std_out, int *nloo_out);
+int gibbs_batch_split(double *plan_ms, double *h2d_ms, double *d2h_ms);  // of the context's last batch
+void gibbs_batch_drop(int slot);  // a context goes away: frees its staging buffer
+
 // ---- the schedule cache (gibbs.cu) ------------------------------------------------------------------------------
 enum Route : int { ROUTE_K1 = 0, ROUTE_K1F = 1, ROUTE_K1X = 2, NROUTES = 3 };  // K1 also serves K1w
 

@@ -1,0 +1,5 @@
+// gibbs_batch_d2.cu -- explicit instantiation of the batched Gibbs kernel (K1b) for d = 2.
+#include "gibbs_batch_kernel.cuh"
+namespace kdeb200 {
+template cudaError_t launch_gibbs_batch_d<2>(const BatchParams &, bool, int, int, cudaStream_t);
+}

@@ -22,6 +22,7 @@
 #include <vector>
 
 #include "eval_shared.cuh"
+#include "lcv.cuh"
 #include "tree.cuh"
 
 namespace kdeb200 {
@@ -44,7 +45,6 @@ int loo_sym_combine_device(kdeb200_tree_t bd, const double *bw_var, const double
 int loglik_reduce_device(kdeb200_tree_t bd, const double *d_L, int64_t q0, int64_t n, double *d_sum, int *d_flag,
                          cudaStream_t st, int *launches);
 
-constexpr int LCV_FUSED_MAX = 512;  // one row per thread and a single component tile: the sums of eval.cu at S = 1
 constexpr int LCV_THREADS = 1024;   // == the block of loglik_reduce_kernel (same reduction tree)
 
 struct LcvDim {
@@ -165,12 +165,13 @@ struct LcvPointsParams {
   double norm0, tol, Cg, Rg;
 };
 
-__global__ void __launch_bounds__(LCV_THREADS) lcv_golden_points_kernel(const __grid_constant__ LcvPointsParams P) {
+// the whole search for dimension `dim` of the points at P.pts, by one CTA of LCV_THREADS threads
+__device__ __forceinline__ void lcv_golden_points_cta(const LcvPointsParams &P, int dim) {
   __shared__ __align__(16) double tab[KDE_EXP_TAB];  // prologue: the heap (centres | half-ranges), then the exp table
   __shared__ __align__(16) double rec[2 * LCV_FUSED_MAX];
   __shared__ double sh[LCV_THREADS];
   __shared__ int shf[LCV_THREADS];
-  const int dim = blockIdx.x, N = P.N, tid = threadIdx.x;
+  const int N = P.N, tid = threadIdx.x;
   // ---- sort (bitonic, 512 slots padded with +inf)
   double *sb = sh;
   if (tid < LCV_FUSED_MAX) sb[tid] = (tid < N) ? P.pts[(size_t)tid * P.d + dim] : INFINITY;
@@ -259,6 +260,24 @@ __global__ void __launch_bounds__(LCV_THREADS) lcv_golden_points_kernel(const __
   }
 }
 
+__global__ void __launch_bounds__(LCV_THREADS) lcv_golden_points_kernel(const __grid_constant__ LcvPointsParams P) {
+  lcv_golden_points_cta(P, blockIdx.x);
+}
+
+// The same for many point sets in one launch (kdeb200_product_kde_batch): CTA b runs dimension items[b].dim of
+// problem items[b].  Every item carries its own points, N, d, w2 and output block; the constants are the launch's.
+__global__ void __launch_bounds__(LCV_THREADS) lcv_golden_points_batch_kernel(const LcvBatchItem *__restrict__ items,
+                                                                              const __grid_constant__ LcvPointsParams C) {
+  const LcvBatchItem it = items[blockIdx.x];
+  LcvPointsParams P = C;
+  P.pts = it.pts;
+  P.out = it.out;
+  P.N = it.N;
+  P.d = it.d;
+  P.w2 = it.w2;
+  lcv_golden_points_cta(P, it.dim);
+}
+
 namespace {
 
 // everything ksize needs from one dimension's marginal, in the reference's order of operations
@@ -311,6 +330,20 @@ struct Golden {
   }
 };
 
+// the launch constants of the device-points search (everything but the points, N, d and w2)
+LcvPointsParams lcv_points_consts() {
+  const Golden G_;
+  LcvPointsParams P;
+  std::memset(&P, 0, sizeof(P));
+  P.exptab = ctx().d_exptab;
+  P.ec = make_exp_consts();
+  P.norm0 = std::pow(2.0 * M_PI, 0.5);
+  P.tol = 1e-2;
+  P.Cg = G_.Cg;
+  P.Rg = G_.Rg;
+  return P;
+}
+
 }  // namespace
 
 // kde!(points) bandwidths for N <= LCV_FUSED_MAX points resident on the device (point i at d_points + i * d): one launch on
@@ -318,8 +351,18 @@ struct Golden {
 // together with its other results; lcv_points_finish turns it into the standard deviations.
 int kde_lcv_points_device(int d, int64_t N, const double *d_points, double *d_out5, cudaStream_t st) {
   if (N < 2 || N > LCV_FUSED_MAX) KDE_FAIL(3, "kde_lcv (device points): needs 2 <= N <= %d", LCV_FUSED_MAX);
-  Context &c = ctx();
-  const Golden G_;
+  LcvPointsParams P = lcv_points_consts();
+  P.pts = d_points;
+  P.out = d_out5;
+  P.N = (int)N;
+  P.d = d;
+  P.w2 = lcv_points_w2(N);
+  lcv_golden_points_kernel<<<d, LCV_THREADS, 0, st>>>(P);
+  KDE_CUDA(cudaGetLastError());
+  return 0;
+}
+
+double lcv_points_w2(int64_t N) {
   // the weights of the working density, exactly as the host route derives them: kde!(points, [1.0]) -> 1/N, marginal()
   // renormalises by the sequential sum, ksize's kde! renormalises once more
   double w1 = 1.0 / (double)N;
@@ -334,19 +377,12 @@ int kde_lcv_points_device(int d, int64_t N, const double *d_points, double *d_ou
     for (int64_t i = 0; i < N; ++i) ssum += w1;
     w2 = w1 / ssum;
   }
-  LcvPointsParams P;
-  P.pts = d_points;
-  P.out = d_out5;
-  P.exptab = c.d_exptab;
-  P.ec = make_exp_consts();
-  P.N = (int)N;
-  P.d = d;
-  P.w2 = w2;
-  P.norm0 = std::pow(2.0 * M_PI, 0.5);
-  P.tol = 1e-2;
-  P.Cg = G_.Cg;
-  P.Rg = G_.Rg;
-  lcv_golden_points_kernel<<<d, LCV_THREADS, 0, st>>>(P);
+  return w2;
+}
+
+int kde_lcv_points_batch_device(int nitems, const LcvBatchItem *d_items, cudaStream_t st) {
+  if (nitems <= 0) return 0;
+  lcv_golden_points_batch_kernel<<<nitems, LCV_THREADS, 0, st>>>(d_items, lcv_points_consts());
   KDE_CUDA(cudaGetLastError());
   return 0;
 }

@@ -1,6 +1,7 @@
 // tree.cuh -- device-resident BallTreeDensity: level-ordered SoA/AoS records (K3).
 #pragma once
 #include <cstdint>
+#include <memory>
 #include <vector>
 
 #include "common.cuh"
@@ -20,6 +21,10 @@ struct Level {
 };
 
 }  // namespace kdeb200
+
+namespace kdeb200 {
+struct TreeDraws;  // gibbs_batch.cu
+}
 
 struct kdeb200_tree_s {
   int d = 0;
@@ -51,6 +56,7 @@ struct kdeb200_tree_s {
   int device = 0;               // ... and its CUDA device
   std::vector<int64_t> h_perm;  // host copy of d_perm (scatter of sharded LOO rows)
   kdeb200_tree_s *replica[KDEB200_MAX_GPUS] = {nullptr};  // copies on the other GPUs of the in-process set (lazy)
+  std::shared_ptr<kdeb200::TreeDraws> batch_draws[2];  // lazily built Gibbs draw templates, [b_records] (gibbs_batch.cu)
 };
 
 namespace kdeb200 {

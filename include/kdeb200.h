@@ -198,6 +198,21 @@ int kdeb200_philox_streams(uint64_t seed, int64_t Np, int64_t uniforms_per_sampl
  * evaluates bd at its own points leaving each one out (bd === locations), output in original
  * point order. */
 int kdeb200_eval(kdeb200_tree_t bd, const double *pos, int64_t M, int loo, int precision, double *p_out);
+/* nprob independent evaluate(bd, locations) problems (src/DualTree01.jl:303-346) in one blocking call (K2b: one
+ * brute-force launch per (d, loo) class present, one finalize launch for the problems whose components are split).
+ *   trees    nprob handles (the same handle may serve several problems)
+ *   M        nprob query counts; ignored (taken as N_i) where loo[i] != 0; M[i] == 0 is allowed
+ *   loo      nprob flags, or NULL for none
+ *   pos      the d_i x M_i query blocks of the non-LOO problems, concatenated in order, each laid out as kdeb200_eval's
+ *   p_out    M_i results per problem, concatenated; LOO results in original point order
+ * precision must be KDEB200_F64 (the others are refused with code 3).  Each problem's results are bit for bit those of
+ * kdeb200_eval(..., KDEB200_F64) alone on one GPU under pruning modes 0 and 1.  Under mode 2 the single call may take
+ * the pruned kernel (large N and M), the batch always sums by brute force: results then agree to that kernel's 1e-13
+ * bound.  Every problem is checked before anything runs, with the single call's error codes; the message names the
+ * problem.  Under kdeb200_init_multi the whole batch runs on the primary GPU.  kdeb200_last_kernel_ms covers all of
+ * the call's launches. */
+int kdeb200_eval_batch(int nprob, const kdeb200_tree_t *trees, const int64_t *M, const int *loo, const double *pos,
+                       int precision, double *p_out);
 /* Pruning policy (replaces setForceEvalDirect! / FORCE_EVAL_DIRECT src/DualTree01.jl:3-9, and the dual-tree recursion
  * evaluate :248-299 + recurseMinMax :164-242 it switches on).  The pruned kernel drops (query block, component tile)
  * pairs whose bounding boxes are so far apart that each kernel value is below 1e-26, and recomputes over all
@@ -246,6 +261,13 @@ int kdeb200_loo_partial(kdeb200_tree_t bd, const double *bw_var, int64_t j0, int
  * golden-section search in ONE kernel launch; larger N loops on the host over the tiled LOO
  * kernel.  Both give the bits of the call-by-call route through kdeb200_loo_entropy. */
 int kdeb200_kde_lcv(int d, int64_t N, const double *points, double *bw_std_out, int *nloo_calls_out);
+/* kde!(points) bandwidths (src/KDE01.jl:13-23) of nprob independent point sets in one call.  points holds the d[i] x N[i]
+ * sets concatenated in order; bw_std_out and nloo_calls_out (may be NULL) hold sum(d[i]) entries.  Sets with
+ * N[i] <= 512 run in one copy and one launch (one CTA per (set, dimension)); larger sets run kdeb200_kde_lcv's bandwidth
+ * loop one after the other.  Each set's results are bit for bit kdeb200_kde_lcv's.  Every set is checked first, with the
+ * single call's error codes; the message names the set. */
+int kdeb200_kde_lcv_batch(int nprob, const int *d, const int64_t *N, const double *points, double *bw_std_out,
+                          int *nloo_calls_out);
 
 /* The same with the leaf rows [j0, j1) of every nLOO_LL evaluation owned by this process (one process
  * per GPU): after each partial evaluation the library calls allreduce(&sum, &zero_flag, user), which

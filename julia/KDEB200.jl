@@ -276,6 +276,52 @@ function product_batch(tree_lists::Vector{Vector{BallTreeDensity}}; addEntropy::
   return res
 end
 
+# [evaluateDualTree(bd, pos, lv) for (bd, pos, lv) in zip(densities, positions, lvFlags)] in one call (kdeb200_eval_batch:
+# one brute-force launch per dimension and leave-one-out flag).  positions[i] is d_i x M_i; a leave-one-out problem
+# ignores its entry.  Each result is bit for bit the single call's (pruning modes 0 and 1).
+function evaluate_batch(densities::Vector{BallTreeDensity}, positions::Vector{Matrix{Float64}},
+                        lvFlags::Vector{Bool}=fill(false, length(densities)))
+  n = length(densities)
+  for i in 1:n
+    lvFlags[i] || Ndim(densities[i]) == size(positions[i], 1) ||
+      error("evaluate_batch: problem $(i-1): bd and pos must have the same dimension")
+  end
+  dts = [DeviceTree(bd; gibbs=false) for bd in densities]
+  hs = Ptr{Cvoid}[d.h for d in dts]
+  M = Int64[lvFlags[i] ? Npts(densities[i]) : size(positions[i], 2) for i in 1:n]
+  loo = Cint[lv ? 1 : 0 for lv in lvFlags]
+  Q = reduce(vcat, [vec(positions[i]) for i in 1:n if !lvFlags[i]]; init=Float64[])
+  P = zeros(sum(M; init=0))
+  GC.@preserve dts hs M loo Q P check(ccall((:kdeb200_eval_batch, LIB), Cint,
+    (Cint, Ptr{Ptr{Cvoid}}, Ptr{Int64}, Ptr{Cint}, Ptr{Float64}, Cint, Ptr{Float64}), n, hs, M, loo, Q, 0, P))
+  res = Vector{Vector{Float64}}(undef, n)
+  o = 0
+  for i in 1:n
+    res[i] = P[o+1:o+M[i]]
+    o += M[i]
+  end
+  return res
+end
+
+# [lcv_bandwidths(p) for p in point_sets] in one call (kdeb200_kde_lcv_batch): sets of at most 512 points in one launch,
+# larger ones by the bandwidth loop one after the other.  kde!(p, bw) then builds each density as kde!(p) does.
+function kde_lcv_batch(point_sets::Vector{Matrix{Float64}})
+  n = length(point_sets)
+  d = Cint[size(p, 1) for p in point_sets]
+  N = Int64[size(p, 2) for p in point_sets]
+  pts = reduce(vcat, [vec(p) for p in point_sets]; init=Float64[])
+  bw = zeros(sum(d; init=0))
+  GC.@preserve d N pts bw check(ccall((:kdeb200_kde_lcv_batch, LIB), Cint,
+    (Cint, Ptr{Cint}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}), n, d, N, pts, bw, C_NULL))
+  res = Vector{Vector{Float64}}(undef, n)
+  b0 = 0
+  for i in 1:n
+    res[i] = bw[b0+1:b0+d[i]]
+    b0 += d[i]
+  end
+  return res
+end
+
 # sample(npd, Npts) (src/KDE01.jl:164-183) on the device; Philox(seed) variates (Julia's RNG streams can be injected as
 # randU (Npts) / randN (d x Npts) through the C entry point directly)
 function sample(npd::BallTreeDensity, Np::Int; seed::UInt64=rand(UInt64))

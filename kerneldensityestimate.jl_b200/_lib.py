@@ -48,10 +48,12 @@ SIGNATURES = {
     "kdeb200_gibbs_sizes": (C.c_int, [C.POINTER(tree_t), C.c_int, C.c_int, C.POINTER(C.c_int), i64p, i64p, i64p]),
     "kdeb200_philox_streams": (C.c_int, [C.c_uint64, C.c_int64, C.c_int64, C.c_int64, f64p, f64p]),
     "kdeb200_eval": (C.c_int, [tree_t, f64p, C.c_int64, C.c_int, C.c_int, f64p]),
+    "kdeb200_eval_batch": (C.c_int, [C.c_int, C.POINTER(tree_t), i64p, C.POINTER(C.c_int), f64p, C.c_int, f64p]),
     "kdeb200_eval_device": (C.c_int, [tree_t, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "kdeb200_loo_entropy": (C.c_int, [tree_t, f64p, f64p]),
     "kdeb200_loo_partial": (C.c_int, [tree_t, f64p, C.c_int64, C.c_int64, f64p, C.POINTER(C.c_int)]),
     "kdeb200_kde_lcv": (C.c_int, [C.c_int, C.c_int64, f64p, f64p, C.POINTER(C.c_int)]),
+    "kdeb200_kde_lcv_batch": (C.c_int, [C.c_int, C.POINTER(C.c_int), i64p, f64p, f64p, C.POINTER(C.c_int)]),
     "kdeb200_kde_lcv_sharded": (C.c_int, [C.c_int, C.c_int64, f64p, C.c_int64, C.c_int64, allreduce_fn, C.c_void_p, f64p,
                                           C.POINTER(C.c_int)]),
     "kdeb200_kde_lcv_sharded_v": (C.c_int, [C.c_int, C.c_int64, f64p, C.c_int64, C.c_int64, allreduce_v_fn, C.c_void_p, f64p,

@@ -27,7 +27,7 @@ from ._lib import KDEError, check, fptr, iptr, lib
 
 __all__ = [
     "KDEError", "BallTree", "BallTreeDensity", "kde", "kde_bang", "getPoints", "getBW", "getWeights", "marginal",
-    "sample", "rand", "resample", "evaluateDualTree", "evalAvgLogL", "entropy", "kld", "minkld", "nLOO_LL", "golden",
+    "sample", "rand", "resample", "evaluateDualTree", "evaluateDualTree_batch", "kde_batch", "lcv_bandwidths_batch", "evalAvgLogL", "entropy", "kld", "minkld", "nLOO_LL", "golden",
     "ksize", "neighborMinMax", "lcv_bandwidths", "updateBandwidth", "prodAppxMSGibbsS", "prodAppxMSGibbsS_batch", "prod_batch", "gibbs_batch_split", "Ndim", "Npts", "init", "init_multi", "multi_count", "gibbs_sizes",
     "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
     "getKDEMax", "getKDEMean", "getKDEfit", "intersIntgAppxIS", "eval_marginals", "to_string", "from_string",
@@ -259,6 +259,38 @@ def lcv_bandwidths(points, _count=None):
     return bw
 
 
+def lcv_bandwidths_batch(point_sets, _count=None):
+    """[lcv_bandwidths(p) for p in point_sets] in one library call (kdeb200_kde_lcv_batch): every set of at most 512
+    points in one kernel launch, larger sets by the bandwidth loop one after the other.  Returns a list of arrays of d_i
+    standard deviations, bit for bit those of lcv_bandwidths; _count, if given, receives one list of nLOO_LL call counts
+    per set."""
+    sets = [_as_matrix(p) for p in point_sets]
+    n = len(sets)
+    d = np.array([p.shape[0] for p in sets], dtype=np.int32)
+    N = np.array([p.shape[1] for p in sets], dtype=np.int64)
+    flat = np.concatenate([np.ascontiguousarray(p.T).ravel() for p in sets] + [np.zeros(1)])
+    nb = int(d.sum())
+    bw = np.zeros(nb + 1)
+    calls = np.zeros(nb + 1, dtype=np.int32)
+    check(lib().kdeb200_kde_lcv_batch(n, d.ctypes.data_as(C.POINTER(C.c_int)), iptr(N), fptr(flat), fptr(bw),
+                                      calls.ctypes.data_as(C.POINTER(C.c_int))))
+    res, b0 = [], 0
+    for k in d:
+        res.append(bw[b0:b0 + int(k)].copy())
+        if _count is not None:
+            _count.append([int(c) for c in calls[b0:b0 + int(k)]])
+        b0 += int(k)
+    return res
+
+
+def kde_batch(point_sets):
+    """[kde(p) for p in point_sets]: the leave-one-out bandwidths of all sets from one library call
+    (lcv_bandwidths_batch), then each density built on the host as kde(p) builds it.  Equal bandwidths and identical
+    tree arrays."""
+    sets = [_as_matrix(p) for p in point_sets]
+    return [kde(p, bw) for p, bw in zip(sets, lcv_bandwidths_batch(sets))]
+
+
 def kde(points, ks=None, weights=None, addop=None, diffop=None, native_lcv=True):
     """kde!(points) / kde!(points, ks) / kde!(points, ks, weights)  (src/KDE01.jl:3-84).
 
@@ -413,6 +445,63 @@ def evaluateDualTree(bd, pos, lvFlag=False, errTol=1e-3, addop=None, diffop=None
     if lvFlag:
         return _eval_loo(bd, precision)
     return _eval_points(bd, pos, precision)
+
+
+def _eval_problem(i, bd, pos, lvFlag):
+    """(loo, d x M query matrix or None) of one evaluateDualTree_batch problem, read as evaluateDualTree reads it"""
+    if isinstance(pos, BallTreeDensity):
+        if bd.bt.dims != pos.bt.dims:
+            raise KDEError("evaluateDualTree_batch: problem %d: bd and pos must have the same dimension" % i)
+        if lvFlag or pos is bd:
+            return True, None
+        return False, getPoints(pos)
+    pos = np.asarray(pos, dtype=np.float64)
+    if pos.ndim == 1:
+        pos = pos.reshape(1, -1)
+    if pos.ndim != 2 or bd.bt.dims != pos.shape[0]:
+        raise KDEError("evaluateDualTree_batch: problem %d: bd and pos must have the same dimension" % i)
+    if lvFlag:
+        return True, None
+    return False, pos
+
+
+def evaluateDualTree_batch(densities, positions, lvFlags=None, precision=F64):
+    """[evaluateDualTree(b, p, lv) for b, p, lv in zip(densities, positions, lvFlags)] in one library call
+    (kdeb200_eval_batch: one brute-force launch per dimension and leave-one-out flag).  Each entry of positions takes
+    what evaluateDualTree's pos takes (a d x M matrix, a vector of 1-D points, another BallTreeDensity; lvFlag or pos is
+    the density itself selects leave-one-out).  Every result is bit for bit what evaluateDualTree returns for that
+    problem alone with pruning modes 0 and 1 (within 1e-13 under mode 2).  FP64 only."""
+    dens = list(densities)
+    poss = list(positions)
+    n = len(dens)
+    if len(poss) != n:
+        raise KDEError("evaluateDualTree_batch: need one position set per density")
+    lvs = [False] * n if lvFlags is None else [bool(x) for x in lvFlags]
+    if len(lvs) != n:
+        raise KDEError("evaluateDualTree_batch: need one lvFlag per density")
+    M = np.zeros(n, dtype=np.int64)
+    loo = np.zeros(n, dtype=np.int32)
+    blocks = []
+    for i, (bd, pos, lv) in enumerate(zip(dens, poss, lvs)):
+        is_loo, q = _eval_problem(i, bd, pos, lv)
+        loo[i] = 1 if is_loo else 0
+        if is_loo:
+            M[i] = bd.bt.num_points
+        else:
+            M[i] = q.shape[1]
+            blocks.append(np.ascontiguousarray(q.T).ravel())
+    handles = (_lib.tree_t * max(n, 1))()
+    for i, bd in enumerate(dens):
+        handles[i] = bd._dev()
+    q = np.concatenate(blocks + [np.zeros(1)])
+    out = np.zeros(int(M.sum()) + 1)
+    check(lib().kdeb200_eval_batch(n, handles, iptr(M), loo.ctypes.data_as(C.POINTER(C.c_int)), fptr(q), int(precision),
+                                   fptr(out)))
+    res, o = [], 0
+    for m in M:
+        res.append(out[o:o + int(m)].copy())
+        o += int(m)
+    return res
 
 
 def evalAvgLogL(bd1, bd2, addop=None, diffop=None):

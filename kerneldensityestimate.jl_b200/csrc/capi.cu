@@ -41,6 +41,9 @@ int eval_device_f32(kdeb200_tree_t bd, const double *d_pos, int64_t M, int loo, 
                     int *launches);
 int loo_partial_device(kdeb200_tree_t bd, const double *bw_var, int64_t j0, int64_t j1, double *d_sum, int *d_flag,
                        cudaStream_t st, int *launches);
+int eval_batch(int nprob, const kdeb200_tree_t *trees, const int64_t *M, const int *loo, const double *pos,
+               int precision, double *p_out);
+int kde_lcv_batch(int nprob, const int *d, const int64_t *N, const double *points, double *bw_std_out, int *nloo_out);
 int pipe_peak(int which, int iters, double *lane_ops_per_s, double *ms_out);
 int dfma_probe(int ilp, int blocks_per_sm, int threads, int iters, double *lane_ops_per_s);
 
@@ -402,6 +405,14 @@ int kdeb200_eval(kdeb200_tree_t bd, const double *pos, int64_t M, int loo, int p
   return 0;
 }
 
+int kdeb200_eval_batch(int nprob, const kdeb200_tree_t *trees, const int64_t *M, const int *loo, const double *pos,
+                       int precision, double *p_out) {
+  KDE_SERIALISE();
+  if (int rc = ensure_init()) return rc;
+  ScopedDevice sd(0);
+  return eval_batch(nprob, trees, M, loo, pos, precision, p_out);
+}
+
 int kdeb200_loo_partial(kdeb200_tree_t bd, const double *bw_var, int64_t j0, int64_t j1, double *sum_out,
                         int *zero_flag_out) {
   KDE_SERIALISE();
@@ -447,6 +458,14 @@ int kdeb200_kde_lcv(int d, int64_t N, const double *points, double *bw_std_out, 
   KDE_SERIALISE();
   if (!points || !bw_std_out) KDE_FAIL(2, "kde_lcv: NULL argument");
   return kde_lcv(d, N, points, 0, N, nullptr, nullptr, bw_std_out, nloo_calls_out);
+}
+
+int kdeb200_kde_lcv_batch(int nprob, const int *d, const int64_t *N, const double *points, double *bw_std_out,
+                          int *nloo_calls_out) {
+  KDE_SERIALISE();
+  if (int rc = ensure_init()) return rc;
+  ScopedDevice sd(0);
+  return kde_lcv_batch(nprob, d, N, points, bw_std_out, nloo_calls_out);
 }
 
 int kdeb200_kde_lcv_sharded_v(int d, int64_t N, const double *points, int64_t j0, int64_t j1,

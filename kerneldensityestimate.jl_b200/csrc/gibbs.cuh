@@ -49,6 +49,9 @@ struct GibbsBatchArgs {
 int gibbs_batch(const GibbsBatchArgs &a, double *points_out, int64_t *indices_out, double *bw_std_out, int *nloo_out);
 int gibbs_batch_split(double *plan_ms, double *h2d_ms, double *d2h_ms);  // of the context's last batch
 void gibbs_batch_drop(int slot);  // a context goes away: frees its staging buffer
+// the calling context's pinned staging buffer of the batch calls (gibbs_batch.cu, eval_batch.cu), at least `bytes` long;
+// a batch call synchronises its stream before it returns, so the next call may reuse it
+int batch_stage(size_t bytes, char **out);
 
 // ---- the schedule cache (gibbs.cu) ------------------------------------------------------------------------------
 enum Route : int { ROUTE_K1 = 0, ROUTE_K1F = 1, ROUTE_K1X = 2, NROUTES = 3 };  // K1 also serves K1w

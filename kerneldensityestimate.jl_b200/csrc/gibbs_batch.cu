@@ -110,6 +110,19 @@ void gibbs_batch_drop(int slot) {
   b = BatchState();
 }
 
+int batch_stage(size_t bytes, char **out) {
+  BatchState &bs = g_batch[ctx().slot];
+  if (bs.stage_bytes < bytes) {
+    if (bs.stage) cudaFreeHost(bs.stage);
+    bs.stage = nullptr;
+    bs.stage_bytes = 0;
+    KDE_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&bs.stage), bytes, cudaHostAllocDefault));
+    bs.stage_bytes = bytes;
+  }
+  *out = bs.stage;
+  return 0;
+}
+
 int gibbs_batch_split(double *plan_ms, double *h2d_ms, double *d2h_ms) {
   const BatchState &b = g_batch[ctx().slot];
   if (plan_ms) *plan_ms = b.plan_ms;
@@ -238,13 +251,8 @@ int gibbs_batch(const GibbsBatchArgs &a, double *points_out, int64_t *indices_ou
   const size_t n_at = bytes;
   bytes += up256(sizeof(double) * offN);
 
-  if (bs.stage_bytes < bytes) {
-    if (bs.stage) cudaFreeHost(bs.stage);
-    bs.stage = nullptr;
-    bs.stage_bytes = 0;
-    KDE_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&bs.stage), bytes, cudaHostAllocDefault));
-    bs.stage_bytes = bytes;
-  }
+  char *h = nullptr;
+  if (int rc = batch_stage(bytes, &h)) return rc;
   if (!bs.ev_h2d) KDE_CUDA(cudaEventCreate(&bs.ev_h2d));
   if (!bs.ev_d2h) KDE_CUDA(cudaEventCreate(&bs.ev_d2h));
   DevBuf dBlob(c.stream), dP(c.stream), dI(c.stream), dO(c.stream);
@@ -252,7 +260,7 @@ int gibbs_batch(const GibbsBatchArgs &a, double *points_out, int64_t *indices_ou
   KDE_CUDA(dP.alloc(sizeof(double) * offP));
   KDE_CUDA(dI.alloc(sizeof(int64_t) * offI));
   KDE_CUDA(dO.alloc(sizeof(double) * 5 * offB));
-  char *h = bs.stage, *dv = dBlob.as<char>();
+  char *dv = dBlob.as<char>();
   const double *d_U = reinterpret_cast<const double *>(dv + u_at), *d_N = reinterpret_cast<const double *>(dv + n_at);
 
   for (size_t k = 0; k < nplans; ++k) {

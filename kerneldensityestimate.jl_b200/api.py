@@ -29,7 +29,7 @@ __all__ = [
     "KDEError", "BallTree", "BallTreeDensity", "kde", "kde_bang", "getPoints", "getBW", "getWeights", "marginal",
     "sample", "rand", "resample", "evaluateDualTree", "evaluateDualTree_batch", "kde_batch", "lcv_bandwidths_batch", "evalAvgLogL", "entropy", "kld", "minkld", "nLOO_LL", "golden",
     "ksize", "neighborMinMax", "lcv_bandwidths", "updateBandwidth", "prodAppxMSGibbsS", "prodAppxMSGibbsS_batch", "prod_batch", "gibbs_batch_split", "Ndim", "Npts", "init", "init_multi", "multi_count", "gibbs_sizes",
-    "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
+    "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "gibbs_exact_redone_internal", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
     "getKDEMax", "getKDEMean", "getKDEfit", "intersIntgAppxIS", "eval_marginals", "to_string", "from_string",
 ]
 
@@ -90,6 +90,14 @@ def gibbs_exact_redone():
     that were redone in FP64, since the last call"""
     n, w = C.c_ulonglong(0), C.c_ulonglong(0)
     check(lib().kdeb200_gibbs_exact_redone(C.byref(n), C.byref(w)))
+    return int(n.value), int(w.value)
+
+
+def gibbs_exact_redone_internal():
+    """(lane-draws, warp-draws) of the FP64 sampler whose label on an internal level the certified FP32 bound could not
+    decide and that were redone in FP64, since the last call"""
+    n, w = C.c_ulonglong(0), C.c_ulonglong(0)
+    check(lib().kdeb200_gibbs_exact_redone_internal(C.byref(n), C.byref(w)))
     return int(n.value), int(w.value)
 
 

@@ -78,7 +78,7 @@ constexpr size_t SCHED_KEEP[NROUTES] = {8, 4, 4};
 std::mutex g_sched_mu;
 std::list<SchedEntry> g_sched[NROUTES][KDEB200_MAX_GPUS];
 unsigned long long *g_counters[KDEB200_MAX_GPUS] = {nullptr};
-constexpr int NCOUNTERS = 3;
+constexpr int NCOUNTERS = 5;
 
 void sched_free(SchedEntry &e, cudaStream_t st) {
   if (e.d_base) cudaFreeAsync(e.d_base, st);
@@ -103,6 +103,7 @@ int sched_build(Route r, const kdeb200_tree_t *trees, int L, SchedEntry &e) {
   Context &c = ctx();
   Plan S;
   plan_schedule(trees, e.M, L, e.T, !e.masked && !e.literal, r != ROUTE_K1, r == ROUTE_K1F, S);
+  if (r == ROUTE_K1X) gibbs_exact_plan(trees, S);
   const size_t b_draws = up256(sizeof(Draw) * S.draws.size()), b_tiles = up256(sizeof(TileDesc) * S.tiles.size()),
                b_cnt = up256(sizeof(int) * SCHED_COUNTERS),
                b_rec = S.blocks.empty() ? 0 : up256(sizeof(float) * (S.nfloats + 8));
@@ -205,10 +206,17 @@ static int take_counters(int first, int n, unsigned long long *h) {
 // K1f draws redone in FP64 since the last call
 int gibbs32_slow_draws(unsigned long long *out) { return take_counters(0, 1, out); }
 
-// K1x lane-draws and warp-draws redone in FP64 since the last call
+// K1x lane-draws and warp-draws redone in FP64 since the last call: leaf levels, certified internal levels
 int gibbs_exact_redone(unsigned long long *lanes, unsigned long long *warps) {
   unsigned long long h[2] = {0, 0};
   if (int rc = take_counters(1, 2, h)) return rc;
+  if (lanes) *lanes = h[0];
+  if (warps) *warps = h[1];
+  return 0;
+}
+int gibbs_exact_redone_internal(unsigned long long *lanes, unsigned long long *warps) {
+  unsigned long long h[2] = {0, 0};
+  if (int rc = take_counters(3, 2, h)) return rc;
   if (lanes) *lanes = h[0];
   if (warps) *warps = h[1];
   return 0;

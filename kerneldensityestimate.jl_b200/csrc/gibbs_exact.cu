@@ -1,6 +1,7 @@
-// gibbs_exact.cu -- host side of K1x (gibbs_exact_kernel.cuh): the FP32 leaf records laid out for accuracy (per-tile
-// centres, log-weights relative to the level's largest), the XDraws over them, launch, and the bound probe.  Routing is
-// gibbs_device's (gibbs.cu), the schedule gibbs.cu's (cache) and gibbs_plan.cuh's (draws, chunks, tiles).
+// gibbs_exact.cu -- host side of K1x (gibbs_exact_kernel.cuh): which draws are certified (leaf levels, large internal
+// sampleIndex levels), their FP32 records laid out for accuracy (per-tile centres, log-weights relative to the level's
+// largest), the XDraws over them, launch, and the bound probe.  Routing is gibbs_device's (gibbs.cu), the schedule
+// gibbs.cu's (cache) and gibbs_plan.cuh's (draws, chunks, tiles), which gibbs_exact_plan adjusts.
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -22,31 +23,36 @@ GX_EXTERN(1) GX_EXTERN(2) GX_EXTERN(3) GX_EXTERN(4) GX_EXTERN(5) GX_EXTERN(6) GX
 // Relative error bound of ex2.approx.ftz.f32 over the exponents K1x feeds it, [-126, 0]: 2^-21 = 4.8e-7, more than three
 // times the maximum measured over every float of that range on a B200, 1.44e-7 (tools/ulp_mufu.py, profiles/mufu_ulp.json).
 constexpr double GX_EX2_ERR = 0x1.0p-21;
+// The same margin for rsqrt.approx.ftz.f32 over every positive normal float: measured maximum 1.25e-7 (same sources).
+constexpr double GX_RSQ_ERR = 0x1.0p-21;
 
-// ---- FP32 leaf records ------------------------------------------------------------------------------------------
+// ---- FP32 records -------------------------------------------------------------------------------------------------
 struct XPrep {
-  const double *src;  // [m.., ln w] records, stride SA
-  float *dst;         // pair records, stride gf_stride(d, VAR_A)
-  double *stats;      // per tile: min[MAX_DIM] | max[MAX_DIM] | max ln w  (pass a) -> centre[MAX_DIM] (pass b reads)
-  int n, src_stride, tnodes;
+  const double *src;  // A: [m.., ln w], C: [m.., b.., ln w] records, stride src_stride
+  float *dst;         // pair records, stride gf_stride(d, var)
+  double *stats;      // per tile (GX_STATS doubles): min m | max m | min b | max b (C) | max ln w
+  int n, src_stride, tnodes, var;
   double lw2max;
 };
+constexpr int GX_STATS = 4 * KDEB200_MAX_DIM + 1;
 
-// pass a: one CTA per tile, per-dimension min / max and the largest ln w of the tile's nodes
+// pass a: one CTA per tile, per-dimension min / max of the means (and, variant C, of the variances) and the largest ln w
 __global__ void gibbs_exact_stats_kernel(const XPrep *preps, int D) {
   const XPrep pd = preps[blockIdx.y];
   const int t = blockIdx.x;
   const int z0 = t * pd.tnodes;
   if (z0 >= pd.n) return;
   const int z1 = min(z0 + pd.tnodes, pd.n);
-  __shared__ double red[2 * KDEB200_MAX_DIM + 1][4];
+  const int nb = pd.var == VAR_C ? 2 * D : 0;  // min / max of b
+  const int nq = 2 * D + nb + 1;
+  __shared__ double red[GX_STATS][4];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  for (int k = 0; k <= 2 * D; ++k) {
-    const bool isw = k == 2 * D, ismax = k >= D;
-    const int kk = isw ? D : (k % D);
+  for (int k = 0; k < nq; ++k) {
+    const bool isw = k == nq - 1, ismax = isw || (k % (2 * D)) >= D;
+    const int col = isw ? (pd.var == VAR_C ? 2 * D : D) : (k < 2 * D ? k % D : D + k % D);
     double v = ismax ? -INFINITY : INFINITY;
     for (int z = z0 + threadIdx.x; z < z1; z += blockDim.x) {
-      const double x = pd.src[(size_t)z * pd.src_stride + kk];
+      const double x = pd.src[(size_t)z * pd.src_stride + col];
       v = ismax ? fmax(v, x) : fmin(v, x);
     }
     for (int o = 16; o; o >>= 1) {
@@ -56,23 +62,25 @@ __global__ void gibbs_exact_stats_kernel(const XPrep *preps, int D) {
     if (lane == 0) red[k][warp] = v;
   }
   __syncthreads();
-  if (threadIdx.x <= 2 * D) {
+  if (threadIdx.x < nq) {
     const int k = threadIdx.x;
-    const bool ismax = k >= D;
+    const bool isw = k == nq - 1, ismax = isw || (k % (2 * D)) >= D;
     double v = red[k][0];
     for (int w = 1; w < 4; ++w) v = ismax ? fmax(v, red[k][w]) : fmin(v, red[k][w]);
-    double *o = pd.stats + (size_t)t * (2 * KDEB200_MAX_DIM + 1);
-    o[k == 2 * D ? 2 * KDEB200_MAX_DIM : (ismax ? KDEB200_MAX_DIM + k - D : k)] = v;
+    // slot: the (2 k / D)-th block of KDEB200_MAX_DIM, dimension k % D
+    pd.stats[(size_t)t * GX_STATS + (isw ? 4 * KDEB200_MAX_DIM : (k / D) * KDEB200_MAX_DIM + k % D)] = v;
   }
 }
 
-// pass b: pair records [m'_0(a), m'_0(b), .., lw'(a), lw'(b), pad], m' = m - centre(tile), lw' = lw2max - log2 w >= 0
+// pass b: pair records, m' = m - centre(tile), lw' = lw2max - log2 w >= 0:
+//   A: [m'_0(a), m'_0(b), .., lw'(a), lw'(b), pad];  C: [m'_0(a), m'_0(b), .., b_0(a), b_0(b), .., lw'(a), lw'(b), pad]
 __global__ void gibbs_exact_rec_kernel(const XPrep *preps, const double *ctrs_base, const size_t *ctr_off, int D) {
   const XPrep pd = preps[blockIdx.y];
   const double *ctr = ctrs_base + ctr_off[blockIdx.y];
   const int p = blockIdx.x * blockDim.x + threadIdx.x;
   if (2 * p >= pd.n) return;
-  const int stride = gf_stride(D, VAR_A);
+  const int stride = gf_stride(D, pd.var);
+  const int nb = pd.var == VAR_C ? D : 0;
   float *o = pd.dst + (size_t)p * stride;
   const double *c = ctr + (size_t)((2 * p) / pd.tnodes) * KDEB200_MAX_DIM;
   for (int hh = 0; hh < 2; ++hh) {
@@ -80,26 +88,67 @@ __global__ void gibbs_exact_rec_kernel(const XPrep *preps, const double *ctrs_ba
     const bool ok = z < pd.n;  // an odd level is padded with a node of probability zero (finite: no 0 * inf)
     const double *r = pd.src + (size_t)(ok ? z : 0) * pd.src_stride;
     for (int k = 0; k < D; ++k) o[2 * k + hh] = ok ? (float)(r[k] - c[k]) : 0.f;
-    o[2 * D + hh] = ok ? (float)fmax(pd.lw2max - r[D] * GF_LOG2E, 0.0) : 1e30f;
+    for (int k = 0; k < nb; ++k) o[2 * (D + k) + hh] = ok ? (float)r[D + k] : 1.f;
+    o[2 * (D + nb) + hh] = ok ? (float)fmax(pd.lw2max - r[D + nb] * GF_LOG2E, 0.0) : 1e30f;
   }
-  for (int k = 2 * (D + 1); k < stride; ++k) o[k] = 0.f;
+  for (int k = 2 * (D + nb + 1); k < stride; ++k) o[k] = 0.f;
 }
 
-// ---- schedule: the FP32 leaf records and the XDraws ---------------------------------------------------------------
-// Every block of the plan is a leaf level (K1x plans FP32 records on leaf levels only).  Pass a on the device, tile
-// centres / radii / largest weights on the host, pass b on the device; the persistent XDraws and centres go to e.d_extra.
+// ---- schedule ---------------------------------------------------------------------------------------------------
+// plan_schedule(.., f32_leaf = true, f32_internal = false) gives every leaf draw FP32 records; this moves the sampleIndex
+// draws (variant C) of internal levels of at least GX_NMIN nodes onto FP32 records as well, with K1f's chunk and tile
+// rule, and rebuilds the tile stream.  Smaller internal levels and every sampleIndices! draw (variant B) keep K1's
+// FP64 tiles: those levels hold a few per cent of the nodes.
+void gibbs_exact_plan(const kdeb200_tree_t *trees, Plan &S) {
+  const int d = trees[0]->d;
+  const int stride = gf_stride(d, VAR_C);
+  std::vector<PlanTile> tiles;
+  for (size_t i = 0; i < S.draws.size(); ++i) {
+    Draw &dr = S.draws[i];
+    const int t0 = dr.tile0;
+    dr.tile0 = (int)tiles.size();
+    if (S.block[i] >= 0 || dr.variant != VAR_C || dr.n < GX_NMIN) {
+      tiles.insert(tiles.end(), S.tiles.begin() + t0, S.tiles.begin() + t0 + dr.ntiles);
+      continue;
+    }
+    const kdeb200_tree_s *t = trees[dr.j];
+    int G = 2;
+    while ((int64_t)G * GB_MAXCK < dr.n) G *= 2;
+    const int want = 4 * gf_unr(d, VAR_C);
+    if (G < want && dr.n >= 2 * want) G = want;
+    int tn = 2;
+    while ((size_t)tn * stride * sizeof(float) <= GB_TILE_BYTES) tn *= 2;
+    dr.G = G;
+    dr.tnodes = tn;
+    dr.nchunks = (dr.n + G - 1) / G;
+    dr.ntiles = (dr.n + tn - 1) / tn;
+    const int blk = plan_block(S, dr.j, dr.level < t->depth ? dr.level : t->depth, VAR_C, dr.n, stride, tn);
+    S.block[i] = blk;
+    for (int a = 0; a < dr.n; a += tn) {
+      const int cnt = (dr.n - a < tn) ? (dr.n - a) : tn;
+      tiles.push_back(PlanTile{nullptr, S.blocks[blk].off + (size_t)(a / 2) * stride,
+                               (uint32_t)(((cnt + 1) / 2) * stride * sizeof(float))});
+    }
+  }
+  S.tiles.swap(tiles);
+}
+
+// Every block of the plan holds FP32 records (a leaf level, or a certified internal level).  Pass a on the device, tile
+// centres / radii / variance ranges / largest weights on the host, pass b on the device; the persistent XDraws and
+// centres go to e.d_extra.
 int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
   Context &c = ctx();
   const int d = trees[0]->d;
-  const size_t SW = 2 * KDEB200_MAX_DIM + 1;  // statistics per tile
-  struct LeafBlock {
+  const size_t SW = GX_STATS;
+  struct XBlock {
     size_t ctr_off = 0, stats_off = 0;  // doubles into the centres / statistics
     int ntiles = 0;
     double rad[KDEB200_MAX_DIM] = {0};
+    double bmin[KDEB200_MAX_DIM] = {0};
     double lw2max = 0.0;
     bool fp32 = true;
   };
-  std::vector<LeafBlock> leaf(S.blocks.size());
+  std::vector<XBlock> blk(S.blocks.size());
   std::vector<XPrep> preps(S.blocks.size());
   std::vector<size_t> coff(S.blocks.size());
   size_t nctr = 0, nstats = 0;
@@ -107,19 +156,21 @@ int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
   for (size_t i = 0; i < S.blocks.size(); ++i) {
     const kdeb200_tree_s *t = trees[S.blocks[i].j];
     const Level &lv = t->levels[S.blocks[i].level];
-    LeafBlock &b = leaf[i];
+    const bool isC = S.blocks[i].variant == VAR_C;
+    XBlock &b = blk[i];
     b.ntiles = (int)((lv.n + S.blocks[i].tnodes - 1) / S.blocks[i].tnodes);
     b.ctr_off = coff[i] = nctr;
     b.stats_off = nstats;
     nctr += (size_t)b.ntiles * KDEB200_MAX_DIM;
     nstats += (size_t)b.ntiles * SW;
     XPrep &xp = preps[i];
-    xp.src = t->d_buf + lv.offA;
+    xp.src = t->d_buf + (isC ? lv.offC : lv.offA);
     xp.dst = e.d_rec + S.blocks[i].off;
     xp.stats = nullptr;
     xp.n = (int)lv.n;
-    xp.src_stride = t->SA;
+    xp.src_stride = isC ? t->SC : t->SA;
     xp.tnodes = S.blocks[i].tnodes;
+    xp.var = S.blocks[i].variant;
     xp.lw2max = 0.0;
     if (b.ntiles > maxt) maxt = b.ntiles;
     if ((lv.n + 1) / 2 > maxpairs) maxpairs = (int)((lv.n + 1) / 2);
@@ -137,7 +188,7 @@ int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
     if (err == cudaSuccess) {
       XPrep *d_prep = reinterpret_cast<XPrep *>(reinterpret_cast<char *>(d_stats) + sizeof(double) * nstats);
       size_t *d_coff = reinterpret_cast<size_t *>(reinterpret_cast<char *>(d_prep) + up(sizeof(XPrep) * preps.size()));
-      for (size_t i = 0; i < preps.size(); ++i) preps[i].stats = d_stats + leaf[i].stats_off;
+      for (size_t i = 0; i < preps.size(); ++i) preps[i].stats = d_stats + blk[i].stats_off;
       err = cudaMemcpyAsync(d_prep, preps.data(), sizeof(XPrep) * preps.size(), cudaMemcpyHostToDevice, c.stream);
       if (err == cudaSuccess) {
         gibbs_exact_stats_kernel<<<dim3((unsigned)maxt, (unsigned)preps.size()), 128, 0, c.stream>>>(d_prep, d);
@@ -148,9 +199,11 @@ int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
       if (err == cudaSuccess) err = cudaStreamSynchronize(c.stream);
       std::vector<double> ctr(nctr + 1, 0.0);
       if (err == cudaSuccess) {
-        for (size_t i = 0; i < leaf.size(); ++i) {
-          LeafBlock &b = leaf[i];
+        for (size_t i = 0; i < blk.size(); ++i) {
+          XBlock &b = blk[i];
           double lwmax = -INFINITY;
+          if (preps[i].var == VAR_C)
+            for (int k = 0; k < d; ++k) b.bmin[k] = INFINITY;
           for (int tt = 0; tt < b.ntiles; ++tt) {
             const double *sv = &st[b.stats_off + (size_t)tt * SW];
             for (int k = 0; k < d; ++k) {
@@ -161,8 +214,14 @@ int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
               const double r = std::fmax(hi - cc, cc - lo) * (1.0 + 1e-15) + std::fabs(cc) * 0x1.0p-51;
               if (!(r <= 1e20)) b.fp32 = false;  // outside FP32's comfortable range: FP64 redo for the whole level
               if (r > b.rad[k]) b.rad[k] = r;
+              if (preps[i].var == VAR_C) {
+                // c_k = b_k + Calmost_k in FP32 needs b_k in (0, 2^29]; the kernel checks Calmost per chain
+                const double bl = sv[2 * KDEB200_MAX_DIM + k], bh = sv[3 * KDEB200_MAX_DIM + k];
+                if (!(bl > 0.0) || !(bh <= 0x1.0p29)) b.fp32 = false;
+                b.bmin[k] = std::fmin(b.bmin[k], bl);
+              }
             }
-            lwmax = std::fmax(lwmax, sv[2 * KDEB200_MAX_DIM]);
+            lwmax = std::fmax(lwmax, sv[4 * KDEB200_MAX_DIM]);
           }
           b.lw2max = lwmax * GF_LOG2E;
           if (!std::isfinite(b.lw2max)) b.fp32 = false, b.lw2max = 0.0;
@@ -185,15 +244,17 @@ int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
   std::memset(xds.data(), 0, sizeof(XDraw) * xds.size());
   for (size_t i = 0; i < S.draws.size(); ++i) {
     if (S.block[i] < 0) continue;
-    const LeafBlock &b = leaf[S.block[i]];
+    const XBlock &b = blk[S.block[i]];
     XDraw &xd = xds[i];
     xd.rec32 = e.d_rec + S.blocks[S.block[i]].off;
     xd.ctr = d_ctr + b.ctr_off;
-    for (int k = 0; k < KDEB200_MAX_DIM; ++k) xd.rad[k] = b.rad[k];
+    for (int k = 0; k < KDEB200_MAX_DIM; ++k) xd.rad[k] = b.rad[k], xd.bmin[k] = b.bmin[k];
     xd.lw2max = b.lw2max;
     xd.G = S.draws[i].G;
     xd.nchunks = S.draws[i].nchunks;
     xd.fp32 = b.fp32 ? 1 : 0;
+    const int nb = (S.draws[i].n + GX_SCR - 1) / GX_SCR;
+    if (nb > e.redo_blocks) e.redo_blocks = nb;
   }
   if (err == cudaSuccess) err = cudaMemcpyAsync(e.d_xd, xds.data(), sizeof(XDraw) * xds.size(), cudaMemcpyHostToDevice, c.stream);
   if (err == cudaSuccess) err = cudaStreamSynchronize(c.stream);
@@ -216,16 +277,20 @@ int gibbs_exact_launch(GibbsParams &P, const SchedEntry &E, int d, cudaStream_t 
   XParams X;
   X.xd = E.d_xd;
   X.ex2_err = GX_EX2_ERR;
+  X.rsq_err = GX_RSQ_ERR;
   X.inflate = 1.0;
   if (const char *ev = getenv("KDEB200_GIBBS_EXACT_INFLATE")) X.inflate = atof(ev);  // tests: force the FP64 redo
   unsigned long long *d_count = nullptr;
   if (int rc = gibbs_counters(&d_count)) return rc;
   X.redone = d_count + 1;
   X.warp_redone = d_count + 2;
+  X.redone_int = d_count + 3;
+  X.warp_redone_int = d_count + 4;
+  X.scr_stride = GX_SCR + E.redo_blocks;
   // The redo scratch belongs to this launch alone, stream-ordered on `st`: launches on other streams may be in flight
   // at the same time, and a warp that shared its (block, warp) slot with another launch would sum foreign terms.
   X.scratch = nullptr;
-  KDE_CUDA(cudaMallocAsync(&X.scratch, sizeof(double) * (size_t)grid * (GB_THREADS / 32) * GX_SCR, st));
+  KDE_CUDA(cudaMallocAsync(&X.scratch, sizeof(double) * (size_t)grid * (GB_THREADS / 32) * X.scr_stride, st));
   e = with_d(d, [&](auto D) { return launch_gibbs_exact_d<decltype(D)::value>(P, X, grid, smem, st); });
   cudaFreeAsync(X.scratch, st);  // released once the kernel ahead of it on `st` has finished
   if (e != cudaSuccess) KDE_FAIL(100 + (int)e, "gibbs (exact) kernel launch: %s", cudaGetErrorString(e));
@@ -233,18 +298,19 @@ int gibbs_exact_launch(GibbsParams &P, const SchedEntry &E, int d, cudaStream_t 
 }
 
 // ---- bound probe (tests) ------------------------------------------------------------------------------------------
-// For query conditionals (mu, Calmost) of one variant-A draw: every node's FP32 term as K1x computes it, its bound, K1's
-// FP64 term, K1's prefix sums, and the intervals K1x would claim for them -- per node as xa_decide forms them, and at
-// checkpoints as xa_pass1 forms them (trip sums in FP32, Q in FP32 per chunk).  One CTA per query.
-// out per query: [A, B, aabs, ok, lw2max, n, G, 0] then per node [p32, acc32, p64, S64, lo, hi, lo_ck, hi_ck]
-// (lo_ck / hi_ck are NaN except at chunk ends).
+// For query conditionals (mu, Calmost) of one certified draw (the leaf draw, variant A, or the first sampleIndex draw of
+// an internal level, variant C): every node's FP32 term as K1x computes it, its bound, K1's FP64 term, K1's prefix sums,
+// and the intervals K1x would claim for them -- per node as xa_decide forms them, and at checkpoints as xa_pass1 forms
+// them (trip sums in FP32, Q in FP32 per chunk).  One CTA per query.
+// out per query: [A, B, aabs, ok, lw2max, n, G, W] then per node [p32, acc32, p64, S64, lo, hi, lo_ck, hi_ck]
+// (lo_ck / hi_ck are NaN except at chunk ends; the intervals bound S64 / W).
 constexpr int GX_PROBE_HDR = 8, GX_PROBE_NODE = 8;
 
-template <int D>
+template <int D, int VAR>
 __global__ void gibbs_exact_probe_kernel(Draw dr, XDraw xd, const double *mu_all, const double *cadd_all, GibbsParams P,
                                          int j, double *out_all) {
-  constexpr int stride = gf_stride(D, VAR_A);
-  constexpr int UNR = gf_unr(D, VAR_A);
+  constexpr int stride = gf_stride(D, VAR);
+  constexpr int UNR = gf_unr(D, VAR);
   const int qi = blockIdx.x;
   double *out = out_all + (size_t)qi * (GX_PROBE_HDR + (size_t)GX_PROBE_NODE * dr.n);
   double mu[D];
@@ -259,20 +325,20 @@ __global__ void gibbs_exact_probe_kernel(Draw dr, XDraw xd, const double *mu_all
     h.ich[k] = sqrt(0.5 / c);
     s32[k] = (float)sqrt(GF_HL2E / c);
   }
-  const XBound bd = xa_bound<D>(xd, s32, dr.n, GX_EX2_ERR, 1.0);
   Hoist32<D> g;
-  for (int k = 0; k < D; ++k) g.a[k] = gf_pack(s32[k], s32[k]);
+  float ks[D], sv[D];
+  double rsmax;
+  const bool rok = x_chain<D, VAR>(xd, h, s32, ks, sv, g, rsmax);
+  XBound bd = xa_bound<D, VAR>(xd, ks, rsmax, dr.n, GX_EX2_ERR, GX_RSQ_ERR, 1.0);
+  bd.ok = bd.ok && rok;
   for (int z = threadIdx.x; z < dr.n; z += blockDim.x) {
-    xa_tile_hoist<D>(xd.ctr + (size_t)(z / dr.tnodes) * KDEB200_MAX_DIM, mu, s32, g);
-    f32x2 acc, sc;
-    gf_pre<D, VAR_A, true>(xd.rec32 + (size_t)(z >> 1) * stride, g, acc, sc);
-    float al, ah;
-    gf_unpack(acc, al, ah);
-    const float a = (z & 1) ? ah : al;
+    xa_tile_hoist<D, VAR>(xd.ctr + (size_t)(z / dr.tnodes) * KDEB200_MAX_DIM, mu, sv, g);
+    float al, ah, pa, pb;
+    xa_pair<D, VAR, true>(xd.rec32 + (size_t)(z >> 1) * stride, g, pa, pb, al, ah);
     double *o = out + GX_PROBE_HDR + (size_t)GX_PROBE_NODE * z;
-    o[0] = (double)gf_ex2_neg(a);
-    o[1] = (double)a;
-    o[2] = eval_node<D, false, VAR_A, true>(dr.rec + (size_t)z * dr.stride, h, P.exptab, P.ec);
+    o[0] = (double)((z & 1) ? pb : pa);
+    o[1] = (double)((z & 1) ? ah : al);
+    o[2] = eval_node<D, false, VAR, true>(dr.rec + (size_t)z * dr.stride, h, P.exptab, P.ec);
   }
   __syncthreads();
   if (threadIdx.x != 0) return;
@@ -283,7 +349,7 @@ __global__ void gibbs_exact_probe_kernel(Draw dr, XDraw xd, const double *mu_all
   out[4] = xd.lw2max;
   out[5] = dr.n;
   out[6] = xd.G;
-  out[7] = 0.0;
+  out[7] = exp2(xd.lw2max);
   double S64 = 0.0, S = 0.0, Q = 0.0, S1 = 0.0, Q1 = 0.0;
   float s = 0.f, qf = 0.f;
   int intrip = 0;
@@ -338,8 +404,9 @@ int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, 
   KDE_CUDA(cudaMemcpy(xds.data(), E.d_xd, sizeof(XDraw) * E.ndraws, cudaMemcpyDeviceToHost));
   int di = -1;
   for (int i = 0; i < E.ndraws && di < 0; ++i)
-    if (draws[i].j == j && draws[i].level == level && draws[i].variant == VAR_A) di = i;
-  if (di < 0) KDE_FAIL(3, "gibbs_exact_probe: level %d of density %d is not a leaf level", level, j + 1);
+    if (draws[i].j == j && draws[i].level == level && (draws[i].variant == VAR_A || (draws[i].kind == 1 && xds[i].rec32)))
+      di = i;
+  if (di < 0) KDE_FAIL(3, "gibbs_exact_probe: level %d of density %d has no certified draw", level, j + 1);
   const size_t per = GX_PROBE_HDR + (size_t)GX_PROBE_NODE * draws[di].n;
   if ((int64_t)(per * nq) > out_len) KDE_FAIL(3, "gibbs_exact_probe: out needs %lld doubles", (long long)(per * nq));
   GibbsParams P;
@@ -353,7 +420,10 @@ int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, 
   cudaError_t err = cudaMemcpy(d_mu, mu, sizeof(double) * nq * d, cudaMemcpyHostToDevice);
   if (err == cudaSuccess) err = cudaMemcpy(d_mu + nq * d, cadd, sizeof(double) * nq * d, cudaMemcpyHostToDevice);
   if (err == cudaSuccess) {
-    gibbs_exact_probe_kernel<3><<<nq, 128, 0, c.stream>>>(draws[di], xds[di], d_mu, d_mu + nq * d, P, j, d_out);
+    if (draws[di].variant == VAR_A)
+      gibbs_exact_probe_kernel<3, VAR_A><<<nq, 128, 0, c.stream>>>(draws[di], xds[di], d_mu, d_mu + nq * d, P, j, d_out);
+    else
+      gibbs_exact_probe_kernel<3, VAR_C><<<nq, 128, 0, c.stream>>>(draws[di], xds[di], d_mu, d_mu + nq * d, P, j, d_out);
     err = cudaGetLastError();
   }
   if (err == cudaSuccess) err = cudaStreamSynchronize(c.stream);

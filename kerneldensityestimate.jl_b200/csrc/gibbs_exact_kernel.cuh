@@ -1,27 +1,33 @@
 // gibbs_exact_kernel.cuh -- K1x (device code and launch template; gibbs_exact.cu holds the host side,
-// gibbs_exact_d<N>.cu one explicit instantiation per d): the FP64 Gibbs sampler with the labels of the leaf levels
-// DECIDED from certified FP32 prefix sums.
+// gibbs_exact_d<N>.cu one explicit instantiation per d): the FP64 Gibbs sampler with the labels of the leaf levels and of
+// the large internal sampleIndex levels DECIDED from certified FP32 prefix sums.
 //
 // Same schedule, chain state, RNG addressing and outputs as gibbs_kernel (K1), bit for bit.  K1 picks on every level
 // the first z with target = fl(u * pT) <= S_z, S_z its sequential FP64 prefix sums (else n - 1).  On the leaf levels
-// (variant A, two thirds of K1's FP64 work at C4) K1x instead evaluates the nodes in packed FP32 (gibbs_f32_kernel.cuh's
-// pair records and arithmetic) and carries next to every FP32 prefix sum S'_z a bound E_z on |S'_z - S_z / W|
-// (W: the level's largest weight; DESIGN.md "K1x" derives it).  A lane's label is taken only when the intervals prove
-// it:  hi(S_{z-1}) < lo(target)  and  hi(target) <= lo(S_z).  A lane that cannot prove its label is redone by its
-// warp with K1's FP64 arithmetic (K1w's scheme: lanes evaluate, one lane sums in node order, the result is K1's
-// label by construction).  Internal levels (variants B, C) run K1's own pass1 / pass2 unchanged.
+// (variant A) and on the sampleIndex draws of internal levels of at least GX_NMIN nodes (variant C) K1x instead
+// evaluates the nodes in packed FP32 (gibbs_f32_kernel.cuh's pair records and arithmetic) and carries next to every FP32
+// prefix sum S'_z a bound E_z on |S'_z - S_z / W| (W: the level's largest weight; DESIGN.md "K1x" derives it).  A lane's
+// label is taken only when the intervals prove it:  hi(S_{z-1}) < lo(target)  and  hi(target) <= lo(S_z).  A lane that
+// cannot prove its label is redone by its warp with K1's FP64 arithmetic (K1w's scheme: lanes evaluate, one lane sums
+// in node order, the result is K1's label by construction).  The other internal draws (variant B, small levels) run
+// K1's own pass1 / pass2 unchanged.
 #pragma once
+#include <type_traits>
+
 #include "gibbs_f32_kernel.cuh"
 
 namespace kdeb200 {
 
-constexpr int GX_SCR = 256;  // doubles of global scratch per warp (the cooperative FP64 redo)
+constexpr int GX_SCR = 256;   // nodes per block of the cooperative FP64 redo (its per-warp global scratch: GX_SCR doubles
+                              // of terms, then one running sum per block)
+constexpr int GX_NMIN = 256;  // internal sampleIndex levels of at least this many nodes are certified in FP32
 
-// per-draw extras of K1x (variant-A draws only; zero elsewhere)
+// per-draw extras of K1x (certified draws only; zero elsewhere)
 struct alignas(16) XDraw {
   const float *rec32;                 // FP32 pair records, coordinates relative to the tile centre
   const double *ctr;                  // tile centres, KDEB200_MAX_DIM doubles per tile of this draw
   double rad[KDEB200_MAX_DIM];        // max over the level of |m - centre| per dimension (FP64, rounded up)
+  double bmin[KDEB200_MAX_DIM];       // variant C: the level's smallest node variance b_k per dimension
   double lw2max;                      // log2 of the level's largest weight (records hold lw2max - log2 w >= 0)
   int G, nchunks;                     // K1x's own checkpoint chunks (nodes, power of two)
   int fp32;                           // 0: the level is outside the FP32 range guard, every lane takes the FP64 redo
@@ -30,32 +36,72 @@ struct alignas(16) XDraw {
 
 struct XParams {
   const XDraw *xd;
-  double *scratch;                    // GX_SCR doubles per warp of the grid
-  unsigned long long *redone;         // lane-draws redone in FP64 (live chains only)
-  unsigned long long *warp_redone;    // warp-draws with at least one redone lane
+  double *scratch;                    // scr_stride doubles per warp of the grid
+  unsigned long long *redone;         // leaf lane-draws redone in FP64 (live chains only)
+  unsigned long long *warp_redone;    // leaf warp-draws with at least one redone lane
+  unsigned long long *redone_int;     // the same two for the certified internal draws
+  unsigned long long *warp_redone_int;
   double ex2_err;                     // relative error bound of ex2.approx.ftz.f32 on [-126, 0]
+  double rsq_err;                     // relative error bound of rsqrt.approx.ftz.f32 on normal floats
   double inflate;                     // test hook: multiplies the bound (1 in production)
+  int scr_stride;                     // GX_SCR + the largest number of redo blocks of a level
 };
 
-// The bound of one variant-A draw: |p32 - p64 / W| <= p32 (A + B acc32) per node, plus aabs; prefix sums add the
+// The bound of one certified draw: |p32 - p64 / W| <= p32 (A + B acc32) per node, plus aabs; prefix sums add the
 // summation terms.  DESIGN.md "K1x" derives every constant.
 struct XBound {
   double A, B, aabs, eta;
   bool ok;
 };
 
-template <int D>
-__device__ __forceinline__ XBound xa_bound(const XDraw &xd, const float (&s32)[D], int n, double ex2_err, double inflate) {
+// The per-chain FP32 constants of a certified draw, from K1's FP64 conditionals h:
+//   ks: kernel-width scale per dimension (A: s_k = sqrt(0.5 log2e / c_k); C: the same for the level's narrowest
+//       c_k = b_min,k + Calmost_k), which measures the tile radii of the bound;
+//   sv: what the tile hoist clamps with (A: s_k; C: |mu - centre| <= 1e12 kernel widths);
+//   g.a, g.c: A: s_k; C: 1 and Calmost_k, so that gf_pre forms c_k = b_k + Calmost_k and d_k = m'_k - (mu_k - centre_k);
+//   rsmax: C: the largest normaliser prod_k c_k^-1/2 of the level (1 for A).
+// Returns false when a variant-C chain's c_k could leave [2^-30, 2^30] (FP32 products of three of them stay normal).
+template <int D, int VAR>
+__device__ __forceinline__ bool x_chain(const XDraw &xd, const Hoist<D, false> &h, const float (&s32)[D], float (&ks)[D],
+                                        float (&sv)[D], Hoist32<D> &g, double &rsmax) {
+  bool ok = true;
+  rsmax = 1.0;
+#pragma unroll
+  for (int k = 0; k < D; ++k) {
+    if (VAR == VAR_A) {
+      ks[k] = sv[k] = s32[k];
+      g.a[k] = gf_pack(s32[k], s32[k]);
+    } else {
+      const double cm = xd.bmin[k] + h.cadd[k];  // <= every node's c_k
+      ok = ok && cm >= 0x1.0p-30 && h.cadd[k] <= 0x1.0p29;  // the host keeps b_k <= 2^29
+      ks[k] = (float)sqrt(GF_HL2E / fmax(cm, 0x1.0p-30));
+      sv[k] = (float)(1e12 / (double)ks[k]);
+      rsmax *= cm;
+      const float cf = (float)h.cadd[k];
+      g.a[k] = gf_pack(1.f, 1.f);
+      g.c[k] = gf_pack(cf, cf);
+    }
+  }
+  if (VAR == VAR_C) rsmax = 1.0 / sqrt(fmax(rsmax, 1e-300));
+  return ok;
+}
+
+template <int D, int VAR>
+__device__ __forceinline__ XBound xa_bound(const XDraw &xd, const float (&ks)[D], double rsmax, int n, double ex2_err,
+                                           double rsq_err, double inflate) {
   const double u = 0x1.0p-24 * (1.0 + 0x1.0p-20);
   double Rmax = 0.0, Rsum = 0.0, R2 = 0.0;
 #pragma unroll
   for (int k = 0; k < D; ++k) {
-    const double R = xd.rad[k] * (double)s32[k] * (1.0 + 3.0 * u);
+    const double R = xd.rad[k] * (double)ks[k] * (1.0 + 3.0 * u);
     Rmax = fmax(Rmax, R);
     Rsum += R;
     R2 += R * R;
   }
-  const double a1 = (D + 7.2) * u + 2.05 * u * Rmax;
+  // variant C: d_k is one FFMA (4.02u on t^2 instead of A's 6.02u), c_k = b_k + Calmost_k 2.01u, the reciprocals from
+  // rs^2 and two products 2 eps_rsq + 5u, D + 3 roundings of the non-negative sum
+  constexpr int ng = (D + 3) / 4;  // rsqrt groups of gf_pre
+  const double a1 = (VAR == VAR_A ? (D + 7.2) * u : (D + 14.2) * u + 2.02 * rsq_err) + 2.05 * u * Rmax;
   const double a0 = 2.05 * u * Rsum + 1e-13 * R2;
   XBound b;
   b.ok = xd.fp32 && (a1 * 130.0 + a0 <= 1e-3) && (R2 == R2);
@@ -66,10 +112,15 @@ __device__ __forceinline__ XBound xa_bound(const XDraw &xd, const float (&s32)[D
   const double qsum = 1.0 / (1.0 - (double)xd.G * u);
   b.ok = b.ok && (double)xd.G * u < 0.1;
   b.B = inflate * qsum * (1.003 * ln2 * 1.001 * a1 + 5e-15);
-  b.A = inflate * (1.003 * (ln2 * (a0 + 1.001 * a1 * a0) + 1.01 * ex2_err) + 2.0 * gf_unr(D, VAR_A) * 1.01 * u +
+  // variant C: the normaliser rs32 = fl(rsqrt(fl(prod c32))) against prod c^-1/2, and the product ex2 * rs32; K1's
+  // own FP64 rsqrt, products and reciprocals as a further relative 1e-14
+  const double norm = (VAR == VAR_A) ? 0.0 : 1.01 * (ng * rsq_err + (1.51 * D + 2.0 * ng) * u) + 1e-14;
+  b.A = inflate * (1.003 * (ln2 * (a0 + 1.001 * a1 * a0) + 1.01 * ex2_err + norm) + 2.0 * gf_unr(D, VAR) * 1.01 * u +
                    (double)n * 0x1.0p-52 + 1e-15 * (6.0 + lwm));
-  // ex2.approx.ftz flushes 2^-acc below 2^-126 to zero; K1 clamps exponents below -700 (kde_exp_flush)
-  b.aabs = 0x1.0p-125 + exp(-699.0 - xd.lw2max * ln2);
+  // ex2.approx.ftz flushes 2^-acc below 2^-126 to zero (variant C: times the normaliser, and the FP32 product may be
+  // subnormal); K1 clamps exponents below -700 (kde_exp_flush)
+  b.aabs = (VAR == VAR_A) ? 0x1.0p-125 + exp(-699.0 - xd.lw2max * ln2)
+                          : 1.01 * (0x1.0p-125 * (1.0 + rsmax) + exp(-699.0 - xd.lw2max * ln2) * rsmax);
   b.eta = (double)n * 1.2e-16 + 1e-15;
   return b;
 }
@@ -78,28 +129,38 @@ __device__ __forceinline__ double xa_err(const XBound &b, double S, double Q, in
   return 1.01 * (b.A * S + b.B * Q) + (double)cnt * b.aabs;
 }
 
-// b_k = (mu_k - centre_k) s_k in FP64 once per tile, clamped so that FP32 never sees an infinity
-template <int D>
-__device__ __forceinline__ void xa_tile_hoist(const double *__restrict__ ctr, const double (&mu)[D], const float (&s32)[D],
+// per tile: A: b_k = (mu_k - centre_k) s_k in FP64, clamped so that FP32 never sees an infinity; C: mu_k - centre_k,
+// clamped to 1e12 kernel widths (sv)
+template <int D, int VAR>
+__device__ __forceinline__ void xa_tile_hoist(const double *__restrict__ ctr, const double (&mu)[D], const float (&sv)[D],
                                               Hoist32<D> &g) {
 #pragma unroll
   for (int k = 0; k < D; ++k) {
-    const double bk = fmin(fmax((mu[k] - ctr[k]) * (double)s32[k], -1e12), 1e12);
+    const double bk = (VAR == VAR_A) ? fmin(fmax((mu[k] - ctr[k]) * (double)sv[k], -1e12), 1e12)
+                                     : fmin(fmax(mu[k] - ctr[k], -(double)sv[k]), (double)sv[k]);
     const float fb = (float)(-bk);
     g.b[k] = gf_pack(fb, fb);
   }
 }
 
-// pass 1 over the FP32 tiles of a variant-A draw: trip sums of 2 UNR terms in FP32 folded into an FP64 running sum,
+// one record pair -> the two FP32 terms and their exponents
+template <int D, int VAR, bool NC>
+__device__ __forceinline__ void xa_pair(const float *__restrict__ r, const Hoist32<D> &g, float &pa, float &pb, float &al,
+                                        float &ah) {
+  f32x2 acc, sc;
+  gf_pre<D, VAR, NC>(r, g, acc, sc);
+  gf_unpack(acc, al, ah);
+  gf_fin<VAR>(acc, sc, pa, pb);
+}
+
+// pass 1 over the FP32 tiles of a certified draw: trip sums of 2 UNR terms in FP32 folded into an FP64 running sum,
 // Q = sum p32 acc32 (the exponent-proportional part of the bound), both checkpointed every G nodes
-template <int D>
-__device__ __forceinline__ double xa_pass1(const Draw &dr, const XDraw &xd, const double (&mu)[D], const float (&s32)[D],
-                                           Ring &R, int64_t &q, double *__restrict__ ck, float *__restrict__ ckq, double &Qout) {
-  constexpr int UNR = gf_unr(D, VAR_A);
-  constexpr int stride = gf_stride(D, VAR_A);
-  Hoist32<D> g;
-#pragma unroll
-  for (int k = 0; k < D; ++k) g.a[k] = gf_pack(s32[k], s32[k]);
+template <int D, int VAR>
+__device__ __forceinline__ double xa_pass1(const Draw &dr, const XDraw &xd, const double (&mu)[D], const float (&sv)[D],
+                                           Hoist32<D> &g, Ring &R, int64_t &q, double *__restrict__ ck,
+                                           float *__restrict__ ckq, double &Qout) {
+  constexpr int UNR = gf_unr(D, VAR);
+  constexpr int stride = gf_stride(D, VAR);
   const int npt = (dr.n + 1) >> 1;
   const int Gp = xd.G >> 1;
   const int tp = dr.tnodes >> 1;
@@ -107,7 +168,7 @@ __device__ __forceinline__ double xa_pass1(const Draw &dr, const XDraw &xd, cons
   float qf = 0.f;
   int c = 0, done = 0, left = Gp;
   for (int t = 0; t < dr.ntiles; ++t, ++q) {
-    xa_tile_hoist<D>(xd.ctr + (size_t)t * KDEB200_MAX_DIM, mu, s32, g);
+    xa_tile_hoist<D, VAR>(xd.ctr + (size_t)t * KDEB200_MAX_DIM, mu, sv, g);
     const int np = (npt - done < tp) ? (npt - done) : tp;
     mbar_wait(&R.bars[q % GB_STAGES], (uint32_t)((q / GB_STAGES) & 1));
     const float *rec = reinterpret_cast<const float *>(R.tiles + (size_t)(q % GB_STAGES) * (GB_TILE_BYTES / 8));
@@ -118,13 +179,13 @@ __device__ __forceinline__ double xa_pass1(const Draw &dr, const XDraw &xd, cons
       int i = 0;
       for (; i + UNR <= run; i += UNR) {
         f32x2 acc[UNR], sc[UNR];
-        gf_trip_pre<D, VAR_A, UNR>(r + (size_t)i * stride, g, acc, sc);
+        gf_trip_pre<D, VAR, UNR>(r + (size_t)i * stride, g, acc, sc);
         float s = 0.f;
 #pragma unroll
         for (int uu = 0; uu < UNR; ++uu) {
-          float al, ah;
+          float al, ah, pa, pb;
           gf_unpack(acc[uu], al, ah);
-          const float pa = gf_ex2_neg(al), pb = gf_ex2_neg(ah);
+          gf_fin<VAR>(acc[uu], sc[uu], pa, pb);
           s = __fadd_rn(s, pa);
           s = __fadd_rn(s, pb);
           qf = __fmaf_rn(pa, al, qf);
@@ -133,11 +194,8 @@ __device__ __forceinline__ double xa_pass1(const Draw &dr, const XDraw &xd, cons
         S = __dadd_rn(S, (double)s);
       }
       for (; i < run; ++i) {
-        f32x2 acc[1], sc[1];
-        gf_trip_pre<D, VAR_A, 1>(r + (size_t)i * stride, g, acc, sc);
-        float al, ah;
-        gf_unpack(acc[0], al, ah);
-        const float pa = gf_ex2_neg(al), pb = gf_ex2_neg(ah);
+        float al, ah, pa, pb;
+        xa_pair<D, VAR, false>(r + (size_t)i * stride, g, pa, pb, al, ah);
         S = __dadd_rn(S, (double)__fadd_rn(pa, pb));
         qf = __fmaf_rn(pa, al, qf);
         qf = __fmaf_rn(pb, ah, qf);
@@ -163,11 +221,11 @@ __device__ __forceinline__ double xa_pass1(const Draw &dr, const XDraw &xd, cons
 
 // decision: chunk from the central checkpoint values, then per-node intervals over that chunk (FP32 terms from global
 // memory, FP64 running sums).  Returns the certified label or -1.
-template <int D>
+template <int D, int VAR>
 __device__ __forceinline__ int xa_decide(const Draw &dr, const XDraw &xd, const XBound &bd, const double (&mu)[D],
-                                         const float (&s32)[D], const double *__restrict__ ck, const float *__restrict__ ckq,
-                                         double tc, double tLo, double tHi) {
-  constexpr int stride = gf_stride(D, VAR_A);
+                                         const float (&sv)[D], Hoist32<D> &g, const double *__restrict__ ck,
+                                         const float *__restrict__ ckq, double tc, double tLo, double tHi) {
+  constexpr int stride = gf_stride(D, VAR);
   const int n = dr.n;
   int lo = 0, hi = xd.nchunks;
   while (lo < hi) {
@@ -183,21 +241,16 @@ __device__ __forceinline__ int xa_decide(const Draw &dr, const XDraw &xd, const 
     Q = (double)ckq[lo - 1];
     prevHi = (S + xa_err(bd, S, Q, z0)) * (1.0 + bd.eta);
   }
-  Hoist32<D> g;
-#pragma unroll
-  for (int k = 0; k < D; ++k) g.a[k] = gf_pack(s32[k], s32[k]);
   int cur = -1;
   for (int z = z0; z < z1; z += 2) {
     const int t = z / dr.tnodes;
     if (t != cur) {
-      xa_tile_hoist<D>(xd.ctr + (size_t)t * KDEB200_MAX_DIM, mu, s32, g);
+      xa_tile_hoist<D, VAR>(xd.ctr + (size_t)t * KDEB200_MAX_DIM, mu, sv, g);
       cur = t;
     }
-    f32x2 acc, sc;
-    gf_pre<D, VAR_A, true>(xd.rec32 + (size_t)(z >> 1) * stride, g, acc, sc);
-    float al, ah;
-    gf_unpack(acc, al, ah);
-    const float pp[2] = {gf_ex2_neg(al), gf_ex2_neg(ah)};
+    float al, ah, pa, pb;
+    xa_pair<D, VAR, true>(xd.rec32 + (size_t)(z >> 1) * stride, g, pa, pb, al, ah);
+    const float pp[2] = {pa, pb};
     const float aa[2] = {al, ah};
 #pragma unroll
     for (int hh = 0; hh < 2; ++hh) {
@@ -214,21 +267,27 @@ __device__ __forceinline__ int xa_decide(const Draw &dr, const XDraw &xd, const 
   return -1;
 }
 
-// K1's label for one lane's variant-A draw, computed by the whole warp: lanes evaluate the nodes with K1's eval_node,
-// lane 0 adds them in node order (the same additions as K1's pass 1 and pass 2), pT < 1e-99 rule included.
-template <int D>
+// K1's label for one lane's certified draw, computed by the whole warp: lanes evaluate the nodes with K1's eval_node,
+// lane 0 adds them in node order (the same additions as K1's pass 1 and pass 2), pT < 1e-99 rule included.  The first
+// sweep records the running sum at the end of every block of GX_SCR nodes (scr[GX_SCR + b]); the second sweep
+// re-evaluates only the block whose end-sum first reaches the target, continuing from the exact sum before it.
+template <int D, int VAR>
 __device__ __noinline__ int xa_redo(const Draw &dr, const Hoist<D, false> &h, double scale, double u,
                                     const double *__restrict__ tab, const ExpConsts &ec, double *__restrict__ scr) {
   const unsigned FULL = 0xffffffffu;
   const int lane = threadIdx.x & 31;
   const int n = dr.n;
+  const int nb = (n + GX_SCR - 1) / GX_SCR;
   double S = 0.0;
-  for (int base = 0; base < n; base += GX_SCR) {
+  for (int b = 0; b < nb; ++b) {
+    const int base = b * GX_SCR;
     const int cnt = (n - base < GX_SCR) ? n - base : GX_SCR;
-    for (int i = lane; i < cnt; i += 32) scr[i] = eval_node<D, false, VAR_A, true>(dr.rec + (size_t)(base + i) * dr.stride, h, tab, ec);
+    for (int i = lane; i < cnt; i += 32) scr[i] = eval_node<D, false, VAR, true>(dr.rec + (size_t)(base + i) * dr.stride, h, tab, ec);
     __syncwarp();
-    if (lane == 0)
+    if (lane == 0) {
       for (int i = 0; i < cnt; ++i) S = __dadd_rn(S, scr[i]);
+      scr[GX_SCR + b] = S;
+    }
     __syncwarp();
   }
   const double pT = __shfl_sync(FULL, S, 0);
@@ -252,25 +311,31 @@ __device__ __noinline__ int xa_redo(const Draw &dr, const Hoist<D, false> &h, do
     return __shfl_sync(FULL, zs, 0);
   }
   const double target = u * pT;
-  S = 0.0;
-  for (int base = 0; base < n; base += GX_SCR) {
-    const int cnt = (n - base < GX_SCR) ? n - base : GX_SCR;
-    for (int i = lane; i < cnt; i += 32) scr[i] = eval_node<D, false, VAR_A, true>(dr.rec + (size_t)(base + i) * dr.stride, h, tab, ec);
-    __syncwarp();
-    int f = -1;
-    if (lane == 0)
-      for (int i = 0; i < cnt; ++i) {
-        S = __dadd_rn(S, scr[i]);
-        if (target <= S) {
-          f = base + i;
-          break;
-        }
+  unsigned bf = (unsigned)nb;  // first block whose end-sum reaches the target
+  for (int b = lane; b < nb; b += 32)
+    if (target <= scr[GX_SCR + b]) {
+      bf = (unsigned)b;
+      break;
+    }
+  bf = __reduce_min_sync(FULL, bf);
+  if (bf >= (unsigned)nb) return zs;
+  const int base = (int)bf * GX_SCR;
+  const int cnt = (n - base < GX_SCR) ? n - base : GX_SCR;
+  S = bf ? scr[GX_SCR + bf - 1] : 0.0;
+  for (int i = lane; i < cnt; i += 32) scr[i] = eval_node<D, false, VAR, true>(dr.rec + (size_t)(base + i) * dr.stride, h, tab, ec);
+  __syncwarp();
+  int f = base + cnt - 1;
+  if (lane == 0)
+    for (int i = 0; i < cnt; ++i) {
+      S = __dadd_rn(S, scr[i]);
+      if (target <= S) {
+        f = base + i;
+        break;
       }
-    f = __shfl_sync(FULL, f, 0);
-    __syncwarp();
-    if (f >= 0) return f;
-  }
-  return zs;
+    }
+  f = __shfl_sync(FULL, f, 0);
+  __syncwarp();
+  return f;
 }
 
 template <int D, int MD>
@@ -284,7 +349,7 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_exact_kernel(c
   const int tid = threadIdx.x, lane = tid & 31;
   const int M = P.M;
   const unsigned FULL = 0xffffffffu;
-  double *scr = X.scratch + ((size_t)blockIdx.x * (GB_THREADS / 32) + (tid >> 5)) * GX_SCR;
+  double *scr = X.scratch + ((size_t)blockIdx.x * (GB_THREADS / 32) + (tid >> 5)) * X.scr_stride;
 
   for (int i = tid; i < KDE_EXP_TAB; i += GB_THREADS) tab[i] = P.exptab[i];
   if (tid == 0) {
@@ -319,7 +384,7 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_exact_kernel(c
   double ck[GB_MAXCK];
   float ckq[GB_MAXCK];
   int selpos[MD];
-  unsigned redone = 0, wredone = 0;
+  unsigned redone = 0, wredone = 0, redone_i = 0, wredone_i = 0;
 
   while (batch < P.nbatches) {
     int64_t s = P.s0 + (int64_t)batch * GB_THREADS + tid;
@@ -404,31 +469,39 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_exact_kernel(c
         scale = kde_rsqrt(prod);
       }
 
-      int zs = 0;
-      if (dr.variant == VAR_A) {
+      // a certified draw: FP32 pass 1, the bound, the FP32 decision, the FP64 redo of the lanes it leaves undecided
+      auto certified = [&](auto var) -> int {
+        constexpr int VAR = decltype(var)::value;
         const XDraw xd = X.xd[di];
+        Hoist32<D> g;
+        float ks[D], sv[D];
+        double rsmax;
+        const bool rok = x_chain<D, VAR>(xd, h, s32, ks, sv, g, rsmax);
         double Qt;
-        const double pT = xa_pass1<D>(dr, xd, h.mu, s32, R, q, ck, ckq, Qt);
+        const double pT = xa_pass1<D, VAR>(dr, xd, h.mu, sv, g, R, q, ck, ckq, Qt);
+        int z = 0;
         bool und = false;
         double u = 0.0;
         if (dr.n > 1) {
           const uint32_t c = (uint32_t)(M + di);
           u = P.randU ? P.randU[s * P.perU + c - 1] : philox_uniform(P.seed, (uint64_t)s, c);
-          const XBound bd = xa_bound<D>(xd, s32, dr.n, X.ex2_err, X.inflate);
+          XBound bd = xa_bound<D, VAR>(xd, ks, rsmax, dr.n, X.ex2_err, X.rsq_err, X.inflate);
+          bd.ok = bd.ok && rok;
           const double E = xa_err(bd, pT, Qt, dr.n);
           const double pLo = (pT - E) * (1.0 - bd.eta), pHi = (pT + E) * (1.0 + bd.eta);
-          // K1's pT * scale < 1e-99 rule must provably not fire; u in [0, 1) keeps the target interval ordered
+          // K1's pT * scale < 1e-99 rule (scale = 1 on internal levels) must provably not fire; u in [0, 1) keeps the
+          // target interval ordered
           und = !(bd.ok && u >= 0.0 && u < 1.0 && pLo > 0.0 && pLo * exp2(xd.lw2max) * scale >= 1.000001e-99);
           if (!und) {
             const double tLo = u * pLo * (1.0 - 0x1.0p-50), tHi = u * pHi * (1.0 + 0x1.0p-50);
-            zs = xa_decide<D>(dr, xd, bd, h.mu, s32, ck, ckq, u * pT, tLo, tHi);
-            und = zs < 0;
+            z = xa_decide<D, VAR>(dr, xd, bd, h.mu, sv, g, ck, ckq, u * pT, tLo, tHi);
+            und = z < 0;
           }
         }
         unsigned ub = __ballot_sync(FULL, und);
         if (ub) {
-          if (live && und) ++redone;
-          if (lane == 0) ++wredone;
+          if (live && und) ++(VAR == VAR_A ? redone : redone_i);
+          if (lane == 0) ++(VAR == VAR_A ? wredone : wredone_i);
         }
         while (ub) {
           const int L = __ffs(ub) - 1;
@@ -438,12 +511,19 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_exact_kernel(c
           for (int k = 0; k < D; ++k) {
             hl.mu[k] = __shfl_sync(FULL, h.mu[k], L);
             hl.ich[k] = __shfl_sync(FULL, h.ich[k], L);
-            hl.cadd[k] = 0.0;
+            hl.cadd[k] = __shfl_sync(FULL, h.cadd[k], L);
             hl.act[k] = true;
           }
-          const int zl = xa_redo<D>(dr, hl, __shfl_sync(FULL, scale, L), __shfl_sync(FULL, u, L), tab, P.ec, scr);
-          if (lane == L) zs = zl;
+          const int zl = xa_redo<D, VAR>(dr, hl, __shfl_sync(FULL, scale, L), __shfl_sync(FULL, u, L), tab, P.ec, scr);
+          if (lane == L) z = zl;
         }
+        return z;
+      };
+      int zs = 0;
+      if (dr.variant == VAR_A) {
+        zs = certified(std::integral_constant<int, VAR_A>());
+      } else if (dr.variant == VAR_C && X.xd[di].rec32) {
+        zs = certified(std::integral_constant<int, VAR_C>());
       } else {  // internal levels: K1's own arithmetic
         double pT;
         if (dr.variant == VAR_B)
@@ -530,6 +610,8 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_exact_kernel(c
   }
   if (redone) atomicAdd(X.redone, (unsigned long long)redone);
   if (wredone) atomicAdd(X.warp_redone, (unsigned long long)wredone);
+  if (redone_i) atomicAdd(X.redone_int, (unsigned long long)redone_i);
+  if (wredone_i) atomicAdd(X.warp_redone_int, (unsigned long long)wredone_i);
 }
 
 template <int D>

@@ -1,7 +1,8 @@
 """K1x (certified FP32 decisions, FP64 results) against K1 (all FP64), alternating in one process:
 python tools/bench_gibbs_exact.py [Np] [dims] [reps] -> one JSON object.  dims is a comma list (default 3 = the C4 shape:
 8 densities x 4096 components, Niter 5).  Kernel times are the library's own CUDA-event times.  `redone_*` are the
-lane-draws / warp-draws K1x redid in FP64 per leaf-level draw; `identical` compares points and labels bit for bit.
+lane-draws / warp-draws K1x redid in FP64 per leaf-level draw, `redone_int_*` the same per certified internal draw
+(sampleIndex on the levels of 256 to 2048 nodes); `identical` compares points and labels bit for bit.
 Also reports the card's name and power limit: the times belong to them."""
 import json, os, subprocess, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -38,6 +39,7 @@ for d in dims:
     r = {"k1_ms": [], "k1x_ms": []}
     run("1", trees)  # schedule, records and scratch are built on the first call
     K.gibbs_exact_redone()
+    K.gibbs_exact_redone_internal()
     for _ in range(reps):
         ref, ms = run("0", trees)
         r["k1_ms"].append(ms)
@@ -49,6 +51,10 @@ for d in dims:
     leaf_draws = reps * Np * 8 * 6 * leaf_levels
     r["redone_lane_frac"] = lanes / leaf_draws
     r["redone_warp_frac"] = warps / (leaf_draws / 32)
+    lanes, warps = K.gibbs_exact_redone_internal()
+    int_draws = reps * Np * 8 * 5 * sum(1 for l in range(1, L + 1) if 256 <= 2 ** l < 4096)
+    r["redone_int_lane_frac"] = lanes / int_draws
+    r["redone_int_warp_frac"] = warps / (int_draws / 32)
     r["identical"] = bool(all(np.array_equal(a, b) for a, b in zip(ref, new)))
     r["k1_samples_per_s"] = Np / min(r["k1_ms"]) * 1e3
     r["k1x_samples_per_s"] = Np / min(r["k1x_ms"]) * 1e3

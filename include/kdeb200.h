@@ -244,6 +244,33 @@ int kdeb200_eval_marginals(kdeb200_tree_t bd, const double *grids, int64_t G, do
  * randN (d x Np, column-major) inject the variates; NULL draws them from Philox4x32-10(seed).  ind_out is 1-based. */
 int kdeb200_sample(kdeb200_tree_t bd, int64_t Np, uint64_t seed, const double *randU, const double *randN,
                    double *points_out, int64_t *ind_out);
+/* nprob independent sample(npd, Npts) problems (src/KDE01.jl:164-183) in one blocking call (one launch for every
+ * problem with Np[i] <= 2048: one CTA each sorts its uniforms in shared memory; larger problems run kdeb200_sample's
+ * device-wide route one by one after it).
+ *   trees              nprob handles; one handle may serve several problems
+ *   Np[i]              samples of problem i, in [0, 2^31) (0 allowed)
+ *   seeds              nprob seeds (read only for problems with a Philox stream; may be NULL if there is none)
+ *   randU/nU           NULL, or the per-problem uniforms concatenated in order; nU[i] is 0 (Philox(seeds[i])) or Np[i]
+ *   randN/nN           NULL, or the per-problem normals concatenated; nN[i] is 0 or d_i*Np[i], laid out as
+ *                      kdeb200_sample's randN.  U and N are injected independently of each other.
+ *   points_out         sum(d_i*Np[i]) doubles: problem i's block laid out as kdeb200_sample's points_out
+ *   ind_out            sum(Np[i]) 1-based indices
+ * Each problem's points and indices are bit for bit those of kdeb200_sample called alone with the same handle, seed and
+ * streams.  The cumulative-weight tables of all handles that have none yet are built together (two synchronises for the
+ * batch).  Every problem is checked before anything runs, with the single call's error codes (a stream length that is
+ * neither 0 nor the full length: code 7); the message names the problem.  Under kdeb200_init_multi the whole batch runs
+ * on the primary GPU.  kdeb200_last_kernel_ms covers all of the call's launches. */
+int kdeb200_sample_batch(int nprob, const kdeb200_tree_t *trees, const int64_t *Np, const uint64_t *seeds,
+                         const double *randU, const int64_t *nU, const double *randN, const int64_t *nN,
+                         double *points_out, int64_t *ind_out);
+/* resample(p, Np) (src/BallTreeDensity01.jl:312-334) for nprob problems: the samples above, then the kde! LOOCV
+ * bandwidths of every sample set -- without the samples leaving the device (Np <= 512: one launch of one CTA per
+ * (problem, dimension)), or by kdeb200_kde_lcv's host route.  Np[i] >= 2 (code 3).  bw_std_out and nloo_calls_out hold
+ * sum(d_i) entries; ind_out and nloo_calls_out may be NULL.  Each problem's bandwidths and nLOO_LL counts are bit for
+ * bit those of kdeb200_kde_lcv on its points. */
+int kdeb200_resample_batch(int nprob, const kdeb200_tree_t *trees, const int64_t *Np, const uint64_t *seeds,
+                           const double *randU, const int64_t *nU, const double *randN, const int64_t *nN,
+                           double *points_out, int64_t *ind_out, double *bw_std_out, int *nloo_calls_out);
 
 /* ---- S3: leave-one-out likelihood (fused) --------------------------------------------------
  * Replaces entropy(bd) src/DualTree01.jl:505-508 / evalAvgLogL :450-470 as called from

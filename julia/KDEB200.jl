@@ -332,6 +332,53 @@ function sample(npd::BallTreeDensity, Np::Int; seed::UInt64=rand(UInt64))
   return pts, ind
 end
 
+# [sample(p, n; seed=s) for (p, n, s) in zip(densities, Np, seeds)] in one call (kdeb200_sample_batch: one launch for
+# every problem of at most 2048 samples).  Each result is bit for bit the single call's.
+function sample_batch(densities::Vector{BallTreeDensity}, Np::Vector{Int};
+                      seeds::Vector{UInt64}=rand(UInt64, length(densities)))
+  n = length(densities)
+  (length(Np) == n && length(seeds) == n) || error("sample_batch: need one Np and one seed per density")
+  dts = [DeviceTree(p; gibbs=false) for p in densities]
+  hs = Ptr{Cvoid}[d.h for d in dts]
+  dims = [Ndim(p) for p in densities]
+  N64 = Int64.(Np)
+  P = zeros(sum(dims .* N64; init=0)); ind = zeros(Int64, sum(N64; init=0))
+  GC.@preserve dts hs N64 seeds P ind check(ccall((:kdeb200_sample_batch, LIB), Cint,
+    (Cint, Ptr{Ptr{Cvoid}}, Ptr{Int64}, Ptr{UInt64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64},
+     Ptr{Int64}), n, hs, N64, seeds, C_NULL, C_NULL, C_NULL, C_NULL, P, ind))
+  res = Vector{Tuple{Matrix{Float64},Vector{Int}}}(undef, n)
+  p0 = 0; i0 = 0
+  for i in 1:n
+    res[i] = (reshape(P[p0+1:p0+dims[i]*N64[i]], dims[i], N64[i]), Int.(ind[i0+1:i0+N64[i]]))
+    p0 += dims[i] * N64[i]; i0 += N64[i]
+  end
+  return res
+end
+
+# [resample(p, n) with Philox(seed)] for many densities in one call (kdeb200_resample_batch): the samples as
+# sample_batch draws them, then the kde! LOOCV bandwidths of every sample set (Np <= 512 without the samples leaving the
+# device); kde!(points, bw) then builds each density as kde!(points) does.
+function resample_batch(densities::Vector{BallTreeDensity}, Np::Vector{Int}=[Npts(p) for p in densities];
+                        seeds::Vector{UInt64}=rand(UInt64, length(densities)))
+  n = length(densities)
+  (length(Np) == n && length(seeds) == n) || error("resample_batch: need one Np and one seed per density")
+  dts = [DeviceTree(p; gibbs=false) for p in densities]
+  hs = Ptr{Cvoid}[d.h for d in dts]
+  dims = [Ndim(p) for p in densities]
+  N64 = Int64.(Np)
+  P = zeros(sum(dims .* N64; init=0)); bw = zeros(sum(dims; init=0))
+  GC.@preserve dts hs N64 seeds P bw check(ccall((:kdeb200_resample_batch, LIB), Cint,
+    (Cint, Ptr{Ptr{Cvoid}}, Ptr{Int64}, Ptr{UInt64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64},
+     Ptr{Int64}, Ptr{Float64}, Ptr{Cint}), n, hs, N64, seeds, C_NULL, C_NULL, C_NULL, C_NULL, P, C_NULL, bw, C_NULL))
+  res = Vector{BallTreeDensity}(undef, n)
+  p0 = 0; b0 = 0
+  for i in 1:n
+    res[i] = kde!(reshape(P[p0+1:p0+dims[i]*N64[i]], dims[i], N64[i]), bw[b0+1:b0+dims[i]])
+    p0 += dims[i] * N64[i]; b0 += dims[i]
+  end
+  return res
+end
+
 # every 1-D marginal on its own grid in one launch (getKDEMax, src/DualTree01.jl:558-569): grids is G x d (column k = the
 # abscissae of dimension k, i.e. the C side's d x G row-major), result likewise
 function eval_marginals(p::BallTreeDensity, grids::Matrix{Float64})

@@ -60,6 +60,10 @@ SIGNATURES = {
                                             C.POINTER(C.c_int)]),
     "kdeb200_eval_marginals": (C.c_int, [tree_t, f64p, C.c_int64, f64p]),
     "kdeb200_sample": (C.c_int, [tree_t, C.c_int64, C.c_uint64, f64p, f64p, f64p, i64p]),
+    "kdeb200_sample_batch": (C.c_int, [C.c_int, C.POINTER(tree_t), i64p, C.POINTER(C.c_uint64), f64p, i64p, f64p, i64p,
+                                       f64p, i64p]),
+    "kdeb200_resample_batch": (C.c_int, [C.c_int, C.POINTER(tree_t), i64p, C.POINTER(C.c_uint64), f64p, i64p, f64p,
+                                         i64p, f64p, i64p, f64p, C.POINTER(C.c_int)]),
     "kdeb200_set_pruning": (C.c_int, [C.c_int]),
     "kdeb200_set_gibbs_precision": (C.c_int, [C.c_int]),
     "kdeb200_gibbs_f32_slow_draws": (C.c_int, [C.POINTER(C.c_ulonglong)]),

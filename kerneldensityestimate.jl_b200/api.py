@@ -27,7 +27,7 @@ from ._lib import KDEError, check, fptr, iptr, lib
 
 __all__ = [
     "KDEError", "BallTree", "BallTreeDensity", "kde", "kde_bang", "getPoints", "getBW", "getWeights", "marginal",
-    "sample", "rand", "resample", "evaluateDualTree", "evaluateDualTree_batch", "kde_batch", "lcv_bandwidths_batch", "evalAvgLogL", "entropy", "kld", "minkld", "nLOO_LL", "golden",
+    "sample", "rand", "resample", "sample_batch", "rand_batch", "resample_batch", "evaluateDualTree", "evaluateDualTree_batch", "kde_batch", "lcv_bandwidths_batch", "evalAvgLogL", "entropy", "kld", "minkld", "nLOO_LL", "golden",
     "ksize", "neighborMinMax", "lcv_bandwidths", "updateBandwidth", "prodAppxMSGibbsS", "prodAppxMSGibbsS_batch", "prod_batch", "gibbs_batch_split", "Ndim", "Npts", "init", "init_multi", "multi_count", "gibbs_sizes",
     "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "gibbs_exact_redone_internal", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
     "getKDEMax", "getKDEMean", "getKDEfit", "intersIntgAppxIS", "eval_marginals", "to_string", "from_string",
@@ -411,6 +411,91 @@ def resample(p, Np=-1, ksType="lcv", rng=None, seed=None):
         raise KDEError("resample: ksType=:discrete is broken in the reference (undefined getDim) and not provided")
     samplePts, _ = sample(p, Np, rng=rng, seed=seed)
     return kde(samplePts)
+
+
+def _sample_batch_args(fn, densities, Np, seeds, randU, randN):
+    """handles, Np, seeds and the concatenated injected streams (or None) of a sample_batch / resample_batch call"""
+    dens = list(densities)
+    n = len(dens)
+    Np = np.array([int(x) for x in Np], dtype=np.int64)
+    if Np.size != n:
+        raise KDEError("%s: need one Np per density" % fn)
+    sd = _seeds(seeds, n)
+    streams = []
+    for name, arg, per in (("randU", randU, [1] * n), ("randN", randN, [Ndim(p) for p in dens])):
+        if arg is None:
+            streams += [None, None]
+            continue
+        if len(arg) != n:
+            raise KDEError("%s: need one %s entry (or None) per density" % (fn, name))
+        parts = []
+        for i, a in enumerate(arg):
+            if a is None:
+                parts.append(np.zeros(0))
+            elif name == "randU":
+                parts.append(np.ascontiguousarray(a, dtype=np.float64).ravel())
+            else:  # d x Np, column-major as sample takes it: point ii at [ii*d, ii*d + d)
+                g = np.asarray(a, dtype=np.float64)
+                if g.ndim != 2 or g.shape[0] != per[i]:
+                    raise KDEError("%s: problem %d: randN must be d x Np" % (fn, i))
+                parts.append(np.ascontiguousarray(g.T).ravel())
+        streams += [np.concatenate(parts + [np.zeros(1)]), np.array([q.size for q in parts], dtype=np.int64)]
+    handles = (_lib.tree_t * max(n, 1))()
+    for i, p in enumerate(dens):
+        handles[i] = p._dev()
+    return dens, n, Np, sd, handles, streams
+
+
+def sample_batch(densities, Np, seeds=None, randU=None, randN=None):
+    """[sample(p, n, seed=s) for p, n, s in zip(densities, Np, seeds)] in one library call (kdeb200_sample_batch: one
+    launch for every problem of at most 2048 samples, larger ones by the single call's route after it).  randU / randN are
+    None or one entry per density, and an entry may be None (Philox(seeds[i])); randU[i] holds Np[i] uniforms, randN[i]
+    is d x Np[i].  Returns a list of (points d x Np, ind), each bit for bit what sample returns for that problem alone
+    with the same seed or injected streams."""
+    dens, n, Np, sd, handles, (U, nU, G, nN) = _sample_batch_args("sample_batch", densities, Np, seeds, randU, randN)
+    dims = [Ndim(p) for p in dens]
+    pts = np.zeros(int(sum(dims[i] * Np[i] for i in range(n))) + 1)
+    idx = np.zeros(int(Np.sum()) + 1, dtype=np.int64)
+    check(lib().kdeb200_sample_batch(n, handles, iptr(Np), sd.ctypes.data_as(C.POINTER(C.c_uint64)), fptr(U), iptr(nU),
+                                     fptr(G), iptr(nN), fptr(pts), iptr(idx)))
+    out, p0, i0 = [], 0, 0
+    for d, m in zip(dims, Np):
+        m = int(m)
+        out.append((pts[p0:p0 + d * m].reshape(m, d).T.copy(), idx[i0:i0 + m].copy()))
+        p0 += d * m
+        i0 += m
+    return out
+
+
+def rand_batch(densities, N=1, seeds=None):
+    """[rand(p, N, seed=s) for p, s in zip(densities, seeds)]; N may be one count or one per density."""
+    dens = list(densities)
+    Ns = [int(N)] * len(dens) if np.isscalar(N) else list(N)
+    return [pts for pts, _ in sample_batch(dens, Ns, seeds=seeds)]
+
+
+def resample_batch(densities, Np=None, ksType="lcv", seeds=None):
+    """[resample(p, n, seed=s) for p, n, s in zip(densities, Np, seeds)] in one library call (kdeb200_resample_batch):
+    the samples as sample_batch draws them, then the kde! bandwidths of every sample set -- sets of at most 512 samples
+    without leaving the device, in one launch.  Np = None means each density's Npts; :discrete is refused as resample
+    refuses it.  Returns the densities built on the host as kde(points, bw), like kde_batch."""
+    if ksType in ("discrete", ":discrete"):
+        raise KDEError("resample: ksType=:discrete is broken in the reference (undefined getDim) and not provided")
+    dens = list(densities)
+    Ns = [Npts(p) for p in dens] if Np is None else Np
+    dens, n, Nps, sd, handles, _ = _sample_batch_args("resample_batch", dens, Ns, seeds, None, None)
+    dims = [Ndim(p) for p in dens]
+    pts = np.zeros(int(sum(dims[i] * Nps[i] for i in range(n))) + 1)
+    bw = np.zeros(int(sum(dims)) + 1)
+    check(lib().kdeb200_resample_batch(n, handles, iptr(Nps), sd.ctypes.data_as(C.POINTER(C.c_uint64)), None, None, None,
+                                       None, fptr(pts), None, fptr(bw), None))
+    out, p0, b0 = [], 0, 0
+    for d, m in zip(dims, Nps):
+        m = int(m)
+        out.append(kde(pts[p0:p0 + d * m].reshape(m, d).T, bw[b0:b0 + d].copy()))
+        p0 += d * m
+        b0 += d
+    return out
 
 
 # ------------------------------------------------------------------------- evaluation -------

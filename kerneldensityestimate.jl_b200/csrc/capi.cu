@@ -44,6 +44,9 @@ int loo_partial_device(kdeb200_tree_t bd, const double *bw_var, int64_t j0, int6
 int eval_batch(int nprob, const kdeb200_tree_t *trees, const int64_t *M, const int *loo, const double *pos,
                int precision, double *p_out);
 int kde_lcv_batch(int nprob, const int *d, const int64_t *N, const double *points, double *bw_std_out, int *nloo_out);
+int sample_batch(bool resample, int nprob, const kdeb200_tree_t *trees, const int64_t *Np, const uint64_t *seeds,
+                 const double *randU, const int64_t *nU, const double *randN, const int64_t *nN, double *points_out,
+                 int64_t *ind_out, double *bw_std_out, int *nloo_out);
 int pipe_peak(int which, int iters, double *lane_ops_per_s, double *ms_out);
 int dfma_probe(int ilp, int blocks_per_sm, int threads, int iters, double *lane_ops_per_s);
 
@@ -630,6 +633,25 @@ int kdeb200_sample(kdeb200_tree_t bd, int64_t Np, uint64_t seed, const double *r
   KDE_CUDA(cudaMemcpyAsync(ind_out, dI.p, sizeof(int64_t) * Np, cudaMemcpyDeviceToHost, c.stream));
   KDE_CUDA(cudaStreamSynchronize(c.stream));
   return 0;
+}
+
+int kdeb200_sample_batch(int nprob, const kdeb200_tree_t *trees, const int64_t *Np, const uint64_t *seeds,
+                         const double *randU, const int64_t *nU, const double *randN, const int64_t *nN,
+                         double *points_out, int64_t *ind_out) {
+  KDE_SERIALISE();
+  if (int rc = ensure_init()) return rc;
+  ScopedDevice sd(0);
+  return sample_batch(false, nprob, trees, Np, seeds, randU, nU, randN, nN, points_out, ind_out, nullptr, nullptr);
+}
+
+int kdeb200_resample_batch(int nprob, const kdeb200_tree_t *trees, const int64_t *Np, const uint64_t *seeds,
+                           const double *randU, const int64_t *nU, const double *randN, const int64_t *nN,
+                           double *points_out, int64_t *ind_out, double *bw_std_out, int *nloo_calls_out) {
+  KDE_SERIALISE();
+  if (int rc = ensure_init()) return rc;
+  ScopedDevice sd(0);
+  return sample_batch(true, nprob, trees, Np, seeds, randU, nU, randN, nN, points_out, ind_out, bw_std_out,
+                      nloo_calls_out);
 }
 
 int kdeb200_set_pruning(int mode) {

@@ -9,9 +9,12 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include <cmath>
+#include <unordered_set>
 #include <vector>
 
 #include "eval_shared.cuh"
+#include "gibbs.cuh"
+#include "sample.cuh"
 #include "tree.cuh"
 
 namespace kdeb200 {
@@ -86,46 +89,57 @@ __global__ void sample_uniforms_kernel(uint64_t seed, int64_t Np, double *__rest
   if (i < Np) u[i] = philox_uniform(seed ^ 0x9E3779B97F4A7C15ull, (uint64_t)i, 0u);
 }
 
-// t: SORTED uniforms; cw: cumulative weights in original point order, normalised (cw[N-1] == 1); for sample ii the
-// reference's scan picks the first i with cw[i] > t[ii] (src/KDE01.jl:176-181)
+// t: SORTED uniforms; the body is sample_one (sample.cuh), shared with the batched kernel (sample_batch.cu)
 __global__ void sample_kernel(const double *__restrict__ t, const double *__restrict__ cw, const int64_t *__restrict__ leaf_of,
                               const double *__restrict__ leaf, int SE, int d, int64_t N, int64_t Np,
                               const double *__restrict__ randn_in, uint64_t seed, const double *__restrict__ bw_std,
                               double *__restrict__ points, int64_t *__restrict__ idx) {
   const int64_t ii = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (ii >= Np) return;
-  const double tv = t[ii];
-  int64_t lo = 0, hi = N - 1;  // first i with cw[i] > tv; cw[N-1] = 1 > tv always (tv < 1)
-  while (lo < hi) {
-    const int64_t mid = (lo + hi) >> 1;
-    if (cw[mid] > tv) hi = mid; else lo = mid + 1;
-  }
-  const double *r = leaf + leaf_of[lo] * SE;
-  for (int k = 0; k < d; ++k) {
-    const double g = randn_in ? randn_in[ii * d + k] : philox_normal(seed, (uint64_t)ii, (uint32_t)k);
-    points[ii * d + k] = r[k] + bw_std[k] * g;
-  }
-  idx[ii] = lo + 1;  // 1-based like the reference
+  sample_one(t[ii], ii, cw, leaf_of, leaf, SE, d, N, randn_in, seed, bw_std, points, idx);
 }
 
-// h_cw / d_cw: built on first use from the weights the tree was created with (sequential cumsum in original order, the
-// reference's cumsum(w) ./ w[end])
-int sample_device(kdeb200_tree_t bd, int64_t Np, uint64_t seed, const double *d_randU, const double *d_randN,
-                  double *d_points, int64_t *d_idx, cudaStream_t st, int *launches) {
-  if (Np <= 0) return 0;
+namespace {
+struct Drain {  // an error return after the first enqueue waits for the enqueued work: the staging buffer is reused
+  cudaStream_t st;
+  ~Drain() { cudaStreamSynchronize(st); }
+};
+}  // namespace
+
+int sample_tables(const kdeb200_tree_t *trees, int n) {
   Context &c = ctx();
-  const int d = bd->d;
-  const int64_t N = bd->N;
-  if (!bd->d_cw) {
-    std::vector<double> leafw(N);
-    KDE_CUDA(cudaMemcpy2DAsync(leafw.data(), sizeof(double), bd->d_leaf + d, sizeof(double) * bd->SE, sizeof(double), N,
+  std::vector<kdeb200_tree_t> todo;
+  std::unordered_set<kdeb200_tree_t> seen;
+  int64_t tot = 0;
+  for (int i = 0; i < n; ++i) {
+    const kdeb200_tree_t t = trees[i];
+    if (!t || t->d_cw || !seen.insert(t).second) continue;
+    todo.push_back(t);
+    tot += t->N;
+  }
+  if (todo.empty()) return 0;
+  // pinned staging: leaf weights of every handle (tot doubles), then per handle its [cw | leaf_of] table (2 N words)
+  char *h = nullptr;
+  if (int rc = batch_stage(24 * (size_t)tot, &h)) return rc;
+  double *w = reinterpret_cast<double *>(h);
+  char *tab = h + 8 * (size_t)tot;
+  Drain drain{c.stream};
+  int64_t off = 0;
+  for (const kdeb200_tree_t t : todo) {
+    KDE_CUDA(cudaMemcpy2DAsync(w + off, sizeof(double), t->d_leaf + t->d, sizeof(double) * t->SE, sizeof(double), t->N,
                                cudaMemcpyDeviceToHost, c.stream));
-    KDE_CUDA(cudaStreamSynchronize(c.stream));
-    std::vector<double> cw(N);
-    std::vector<int64_t> leaf_of(N);
+    off += t->N;
+  }
+  KDE_CUDA(cudaStreamSynchronize(c.stream));
+  off = 0;
+  for (const kdeb200_tree_t t : todo) {
+    const int64_t N = t->N;
+    const double *leafw = w + off;
+    double *cw = reinterpret_cast<double *>(tab + 16 * (size_t)off);
+    int64_t *leaf_of = reinterpret_cast<int64_t *>(tab + 16 * (size_t)off + 8 * (size_t)N);
     for (int64_t s = 0; s < N; ++s) {
-      cw[bd->h_perm[s]] = leafw[s];
-      leaf_of[bd->h_perm[s]] = s;
+      cw[t->h_perm[s]] = leafw[s];
+      leaf_of[t->h_perm[s]] = s;
     }
     double run = 0.0;
     for (int64_t i = 0; i < N; ++i) {
@@ -133,14 +147,33 @@ int sample_device(kdeb200_tree_t bd, int64_t Np, uint64_t seed, const double *d_
       cw[i] = run;
     }
     for (int64_t i = 0; i < N; ++i) cw[i] = cw[i] / run;
+    off += N;
+  }
+  off = 0;
+  for (const kdeb200_tree_t t : todo) {
+    const int64_t N = t->N;
     char *base = nullptr;
     KDE_CUDA(cudaMallocAsync(&base, 16 * (size_t)N, c.stream));
-    bd->d_cw = reinterpret_cast<double *>(base);
-    bd->d_leaf_of = reinterpret_cast<int64_t *>(base + 8 * (size_t)N);
-    KDE_CUDA(cudaMemcpyAsync(bd->d_cw, cw.data(), 8 * (size_t)N, cudaMemcpyHostToDevice, c.stream));
-    KDE_CUDA(cudaMemcpyAsync(bd->d_leaf_of, leaf_of.data(), 8 * (size_t)N, cudaMemcpyHostToDevice, c.stream));
-    KDE_CUDA(cudaStreamSynchronize(c.stream));
+    const cudaError_t e = cudaMemcpyAsync(base, tab + 16 * (size_t)off, 16 * (size_t)N, cudaMemcpyHostToDevice, c.stream);
+    if (e != cudaSuccess) {
+      cudaFreeAsync(base, c.stream);
+      KDE_FAIL(100 + (int)e, "sample: uploading the cumulative weights: %s", cudaGetErrorString(e));
+    }
+    t->d_cw = reinterpret_cast<double *>(base);
+    t->d_leaf_of = reinterpret_cast<int64_t *>(base + 8 * (size_t)N);
+    off += N;
   }
+  KDE_CUDA(cudaStreamSynchronize(c.stream));
+  return 0;
+}
+
+// d_cw / d_leaf_of: built on first use from the weights the tree was created with (sample_tables)
+int sample_device(kdeb200_tree_t bd, int64_t Np, uint64_t seed, const double *d_randU, const double *d_randN,
+                  double *d_points, int64_t *d_idx, cudaStream_t st, int *launches) {
+  if (Np <= 0) return 0;
+  const int d = bd->d;
+  const int64_t N = bd->N;
+  if (int rc = sample_tables(&bd, 1)) return rc;
   double bw[KDEB200_MAX_DIM];
   for (int k = 0; k < d; ++k) bw[k] = std::sqrt(bd->hvar[k]);  // getBW = sqrt of the leaf variances
   size_t tmp_bytes = 0;

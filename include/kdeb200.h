@@ -171,21 +171,24 @@ int kdeb200_gibbs_batch_split(double *plan_ms, double *h2d_ms, double *d2h_ms);
  *                its last call).  Refused (code 8) when a bandwidth is below 1e-4 of the data spread. */
 int kdeb200_set_gibbs_precision(int precision);
 int kdeb200_gibbs_f32_slow_draws(unsigned long long *count_out);
-/* KDEB200_F64 calls of the thread-per-chain sampler decide the leaf-level labels, and the sampleIndex labels of internal
- * levels of at least 256 nodes, from FP32 prefix sums with a proven error bound and redo in FP64 only the draws the
- * bound cannot decide; the labels and points are those of the FP64 arithmetic bit for bit (KDEB200_GIBBS_EXACT=0 forces
- * the all-FP64 kernel).  Counts the redone leaf-level lane-draws and the warp-draws that contained one (warps_out may be
- * NULL) on the calling context's device since the last call; kdeb200_gibbs_exact_redone_internal counts the same for
- * the internal levels. */
+/* KDEB200_F64 calls of the thread-per-chain sampler decide every label -- leaf levels, and on internal levels both the
+ * sampleIndices! and the sampleIndex draws -- from FP32 prefix sums with a proven error bound and redo in FP64 only the
+ * draws the bound cannot decide; the labels and points are those of the FP64 arithmetic bit for bit
+ * (KDEB200_GIBBS_EXACT=0 forces the all-FP64 kernel).  Counts the redone leaf-level lane-draws and the warp-draws that
+ * contained one (warps_out may be NULL) on the calling context's device since the last call;
+ * kdeb200_gibbs_exact_redone_internal counts the same for the sampleIndex draws of every internal level, and
+ * kdeb200_gibbs_exact_redone_b for the sampleIndices! draws (one per internal level and density). */
 int kdeb200_gibbs_exact_redone(unsigned long long *lanes_out, unsigned long long *warps_out);
 int kdeb200_gibbs_exact_redone_internal(unsigned long long *lanes_out, unsigned long long *warps_out);
+int kdeb200_gibbs_exact_redone_b(unsigned long long *lanes_out, unsigned long long *warps_out);
 /* Diagnostic for tests of the bound above (d = 3): for nq query conditionals (mu, Calmost: nq x d each, row-major) of the
  * certified draw of density `density` (0-based) on schedule level `level` (1-based) -- the leaf-level draw, or on an
- * internal level the first sampleIndex draw -- writes per query a header [A, B, aabs, ok, log2 w_max, n, G, W] and per
+ * internal level the first sampleIndex draw, or with pass0 != 0 the sampleIndices! draw (which evaluates against mu alone
+ * and ignores cadd) -- writes per query a header [A, B, aabs, ok, log2 w_max, n, G, W] and per
  * node [p32, acc32, p64, S64, lo, hi, lo_ck, hi_ck]: the FP32 term and its exponent, the FP64 term and prefix sum, and
  * the intervals claimed for S64 / W per node and at checkpoints (NaN between checkpoints), W = w_max the level's
  * largest weight.  out_len: capacity of out in doubles. */
-int kdeb200_gibbs_exact_bound_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int density, int level,
+int kdeb200_gibbs_exact_bound_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int density, int level, int pass0,
                                     const double *mu, const double *cadd, int nq, double *out, int64_t out_len);
 /* glbs.Nlevels (src/MSGibbs01.jl:555-568) and the per-sample stream consumption. */
 int kdeb200_gibbs_sizes(const kdeb200_tree_t *trees, int ndens, int Niter, int *nlevels,

@@ -29,7 +29,7 @@ __all__ = [
     "KDEError", "BallTree", "BallTreeDensity", "kde", "kde_bang", "getPoints", "getBW", "getWeights", "marginal",
     "sample", "rand", "resample", "sample_batch", "rand_batch", "resample_batch", "evaluateDualTree", "evaluateDualTree_batch", "kde_batch", "lcv_bandwidths_batch", "evalAvgLogL", "entropy", "kld", "minkld", "nLOO_LL", "golden",
     "ksize", "neighborMinMax", "lcv_bandwidths", "updateBandwidth", "prodAppxMSGibbsS", "prodAppxMSGibbsS_batch", "prod_batch", "gibbs_batch_split", "Ndim", "Npts", "init", "init_multi", "multi_count", "gibbs_sizes",
-    "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "gibbs_exact_redone_internal", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
+    "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "gibbs_exact_redone_internal", "gibbs_exact_redone_b", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
     "getKDEMax", "getKDEMean", "getKDEfit", "intersIntgAppxIS", "eval_marginals", "to_string", "from_string",
 ]
 
@@ -94,23 +94,31 @@ def gibbs_exact_redone():
 
 
 def gibbs_exact_redone_internal():
-    """(lane-draws, warp-draws) of the FP64 sampler whose label on an internal level the certified FP32 bound could not
-    decide and that were redone in FP64, since the last call"""
+    """(lane-draws, warp-draws) of the FP64 sampler whose sampleIndex label on an internal level (any size) the certified
+    FP32 bound could not decide and that were redone in FP64, since the last call"""
     n, w = C.c_ulonglong(0), C.c_ulonglong(0)
     check(lib().kdeb200_gibbs_exact_redone_internal(C.byref(n), C.byref(w)))
     return int(n.value), int(w.value)
 
 
-def _gibbs_exact_bound_probe(trees, Niter, density, level, mu, cadd):
+def gibbs_exact_redone_b():
+    """(lane-draws, warp-draws) of the FP64 sampler whose sampleIndices! label on an internal level the certified FP32
+    bound could not decide and that were redone in FP64, since the last call"""
+    n, w = C.c_ulonglong(0), C.c_ulonglong(0)
+    check(lib().kdeb200_gibbs_exact_redone_b(C.byref(n), C.byref(w)))
+    return int(n.value), int(w.value)
+
+
+def _gibbs_exact_bound_probe(trees, Niter, density, level, mu, cadd, pass0=False):
     """tests: per query conditional (rows of mu, cadd) the header and per-node table of kdeb200_gibbs_exact_bound_probe,
-    as (headers [nq, 8], nodes [nq, n, 8])"""
+    as (headers [nq, 8], nodes [nq, n, 8]); pass0 probes an internal level's sampleIndices! draw (cadd unused)"""
     mu = np.ascontiguousarray(mu, dtype=np.float64)
     cadd = np.ascontiguousarray(cadd, dtype=np.float64)
     nq = mu.shape[0]
     n = max(Npts(t) for t in trees)
     out = np.zeros(nq * (8 + 8 * n))
     check(lib().kdeb200_gibbs_exact_bound_probe(_handles(trees), len(trees), int(Niter), int(density), int(level),
-                                                fptr(mu), fptr(cadd), nq, fptr(out), out.size))
+                                                int(bool(pass0)), fptr(mu), fptr(cadd), nq, fptr(out), out.size))
     n = int(out[5])
     per = 8 + 8 * n
     out = out[:nq * per].reshape(nq, per)

@@ -687,11 +687,18 @@ int kdeb200_gibbs_exact_redone_internal(unsigned long long *lanes_out, unsigned 
   return gibbs_exact_redone_internal(lanes_out, warps_out);
 }
 
-int kdeb200_gibbs_exact_bound_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int density, int level,
+int kdeb200_gibbs_exact_redone_b(unsigned long long *lanes_out, unsigned long long *warps_out) {
+  KDE_SERIALISE();
+  if (!lanes_out) KDE_FAIL(2, "gibbs_exact_redone_b: NULL argument");
+  if (int rc = ensure_init()) return rc;
+  return gibbs_exact_redone_b(lanes_out, warps_out);
+}
+
+int kdeb200_gibbs_exact_bound_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int density, int level, int pass0,
                                     const double *mu, const double *cadd, int nq, double *out, int64_t out_len) {
   KDE_SERIALISE();
   if (int rc = ensure_init()) return rc;
-  return gibbs_exact_probe(trees, ndens, Niter, density, level, mu, cadd, nq, out, out_len);
+  return gibbs_exact_probe(trees, ndens, Niter, density, level, pass0, mu, cadd, nq, out, out_len);
 }
 
 int kdeb200_pruned_stats(double *kept_fraction, int64_t *redo_rows) {

@@ -78,7 +78,7 @@ constexpr size_t SCHED_KEEP[NROUTES] = {8, 4, 4};
 std::mutex g_sched_mu;
 std::list<SchedEntry> g_sched[NROUTES][KDEB200_MAX_GPUS];
 unsigned long long *g_counters[KDEB200_MAX_GPUS] = {nullptr};
-constexpr int NCOUNTERS = 5;
+constexpr int NCOUNTERS = 7;
 
 void sched_free(SchedEntry &e, cudaStream_t st) {
   if (e.d_base) cudaFreeAsync(e.d_base, st);
@@ -206,7 +206,8 @@ static int take_counters(int first, int n, unsigned long long *h) {
 // K1f draws redone in FP64 since the last call
 int gibbs32_slow_draws(unsigned long long *out) { return take_counters(0, 1, out); }
 
-// K1x lane-draws and warp-draws redone in FP64 since the last call: leaf levels, certified internal levels
+// K1x lane-draws and warp-draws redone in FP64 since the last call: leaf levels, sampleIndex draws of internal levels,
+// sampleIndices! draws of internal levels
 int gibbs_exact_redone(unsigned long long *lanes, unsigned long long *warps) {
   unsigned long long h[2] = {0, 0};
   if (int rc = take_counters(1, 2, h)) return rc;
@@ -217,6 +218,13 @@ int gibbs_exact_redone(unsigned long long *lanes, unsigned long long *warps) {
 int gibbs_exact_redone_internal(unsigned long long *lanes, unsigned long long *warps) {
   unsigned long long h[2] = {0, 0};
   if (int rc = take_counters(3, 2, h)) return rc;
+  if (lanes) *lanes = h[0];
+  if (warps) *warps = h[1];
+  return 0;
+}
+int gibbs_exact_redone_b(unsigned long long *lanes, unsigned long long *warps) {
+  unsigned long long h[2] = {0, 0};
+  if (int rc = take_counters(5, 2, h)) return rc;
   if (lanes) *lanes = h[0];
   if (warps) *warps = h[1];
   return 0;

@@ -27,7 +27,8 @@ int gibbs_set_precision(int p);
 int gibbs32_slow_draws(unsigned long long *out);
 int gibbs_exact_redone(unsigned long long *lanes, unsigned long long *warps);
 int gibbs_exact_redone_internal(unsigned long long *lanes, unsigned long long *warps);
-int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, int level, const double *mu,
+int gibbs_exact_redone_b(unsigned long long *lanes, unsigned long long *warps);
+int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, int level, int pass0, const double *mu,
                       const double *cadd, int nq, double *out, int64_t out_len);
 void gibbs_invalidate_schedules();  // a tree is destroyed: cached schedules point into tree records
 void gibbs_drop_schedules(int slot);  // a context goes away: frees its schedules and counters
@@ -84,7 +85,7 @@ int sched_get(Route r, const kdeb200_tree_t *trees, int L, const SchedEntry &key
 
 // The route-specific part of a schedule build, run once the plan is made and the entry's memory is allocated: K1f's
 // affine map and FP32 records (gibbs_f32.cu), K1x's record statistics, FP32 records and XDraws (gibbs_exact.cu).
-// gibbs_exact_plan runs before the allocation: it moves K1x's large internal sampleIndex draws onto FP32 records.
+// gibbs_exact_plan runs before the allocation: it moves K1x's internal draws onto FP32 records.
 int gibbs32_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e);
 void gibbs_exact_plan(const kdeb200_tree_t *trees, Plan &S);
 int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e);
@@ -92,8 +93,8 @@ int gibbs32_launch(GibbsParams &P, const SchedEntry &E, int d, cudaStream_t st);
 int gibbs_exact_launch(GibbsParams &P, const SchedEntry &E, int d, cudaStream_t st);
 
 // Counters of the calling context, zeroed at allocation: [0] K1f draws redone in FP64, [1] K1x leaf lane-draws and [2]
-// K1x leaf warp-draws redone in FP64, [3] and [4] the same for K1x's certified internal draws (atomics: launches in
-// flight on several streams may share them).
+// K1x leaf warp-draws redone in FP64, [3] and [4] the same for K1x's internal sampleIndex draws, [5] and [6] for its
+// internal sampleIndices! draws (atomics: launches in flight on several streams may share them).
 int gibbs_counters(unsigned long long **out);
 
 // f(std::integral_constant<int, d>()) for the instantiated dimensions: 1..8, or 3 alone in the tuning builds

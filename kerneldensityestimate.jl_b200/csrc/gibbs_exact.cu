@@ -1,6 +1,6 @@
-// gibbs_exact.cu -- host side of K1x (gibbs_exact_kernel.cuh): which draws are certified (leaf levels, large internal
-// sampleIndex levels), their FP32 records laid out for accuracy (per-tile centres, log-weights relative to the level's
-// largest), the XDraws over them, launch, and the bound probe.  Routing is gibbs_device's (gibbs.cu), the schedule
+// gibbs_exact.cu -- host side of K1x (gibbs_exact_kernel.cuh): every draw is certified; its FP32 records laid out for
+// accuracy (per-tile centres, log-weights relative to the level's largest), the XDraws over them, launch, and the bound
+// probe.  Routing is gibbs_device's (gibbs.cu), the schedule
 // gibbs.cu's (cache) and gibbs_plan.cuh's (draws, chunks, tiles), which gibbs_exact_plan adjusts.
 #include <cmath>
 #include <cstdlib>
@@ -28,28 +28,29 @@ constexpr double GX_RSQ_ERR = 0x1.0p-21;
 
 // ---- FP32 records -------------------------------------------------------------------------------------------------
 struct XPrep {
-  const double *src;  // A: [m.., ln w], C: [m.., b.., ln w] records, stride src_stride
+  const double *src;  // A: [m.., ln w], B: [m.., -0.5/b.., ln w - 0.5 sum ln b], C: [m.., b.., ln w] records
   float *dst;         // pair records, stride gf_stride(d, var)
-  double *stats;      // per tile (GX_STATS doubles): min m | max m | min b | max b (C) | max ln w
+  double *stats;      // per tile (GX_STATS doubles): min m | max m | min b | max b (B: of -0.5/b; C) | max of the last column
   int n, src_stride, tnodes, var;
   double lw2max;
 };
 constexpr int GX_STATS = 4 * KDEB200_MAX_DIM + 1;
 
-// pass a: one CTA per tile, per-dimension min / max of the means (and, variant C, of the variances) and the largest ln w
+// pass a: one CTA per tile, per-dimension min / max of the means (and, variants B and C, of the variance columns) and
+// the largest log-weight column
 __global__ void gibbs_exact_stats_kernel(const XPrep *preps, int D) {
   const XPrep pd = preps[blockIdx.y];
   const int t = blockIdx.x;
   const int z0 = t * pd.tnodes;
   if (z0 >= pd.n) return;
   const int z1 = min(z0 + pd.tnodes, pd.n);
-  const int nb = pd.var == VAR_C ? 2 * D : 0;  // min / max of b
+  const int nb = pd.var != VAR_A ? 2 * D : 0;  // min / max of the variance column
   const int nq = 2 * D + nb + 1;
   __shared__ double red[GX_STATS][4];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   for (int k = 0; k < nq; ++k) {
     const bool isw = k == nq - 1, ismax = isw || (k % (2 * D)) >= D;
-    const int col = isw ? (pd.var == VAR_C ? 2 * D : D) : (k < 2 * D ? k % D : D + k % D);
+    const int col = isw ? (pd.var != VAR_A ? 2 * D : D) : (k < 2 * D ? k % D : D + k % D);
     double v = ismax ? -INFINITY : INFINITY;
     for (int z = z0 + threadIdx.x; z < z1; z += blockDim.x) {
       const double x = pd.src[(size_t)z * pd.src_stride + col];
@@ -73,14 +74,16 @@ __global__ void gibbs_exact_stats_kernel(const XPrep *preps, int D) {
 }
 
 // pass b: pair records, m' = m - centre(tile), lw' = lw2max - log2 w >= 0:
-//   A: [m'_0(a), m'_0(b), .., lw'(a), lw'(b), pad];  C: [m'_0(a), m'_0(b), .., b_0(a), b_0(b), .., lw'(a), lw'(b), pad]
+//   A: [m'_0(a), m'_0(b), .., lw'(a), lw'(b), pad];  C: [m'_0(a), m'_0(b), .., b_0(a), b_0(b), .., lw'(a), lw'(b), pad];
+//   B: as C with 0.5 log2e / b_k in place of b_k and log2 w - 0.5 sum log2 b_k in place of log2 w, both from K1's own
+//   record values (-0.5/b_k and ln w - 0.5 sum ln b_k, times -log2e and log2e)
 __global__ void gibbs_exact_rec_kernel(const XPrep *preps, const double *ctrs_base, const size_t *ctr_off, int D) {
   const XPrep pd = preps[blockIdx.y];
   const double *ctr = ctrs_base + ctr_off[blockIdx.y];
   const int p = blockIdx.x * blockDim.x + threadIdx.x;
   if (2 * p >= pd.n) return;
   const int stride = gf_stride(D, pd.var);
-  const int nb = pd.var == VAR_C ? D : 0;
+  const int nb = pd.var != VAR_A ? D : 0;
   float *o = pd.dst + (size_t)p * stride;
   const double *c = ctr + (size_t)((2 * p) / pd.tnodes) * KDEB200_MAX_DIM;
   for (int hh = 0; hh < 2; ++hh) {
@@ -88,33 +91,33 @@ __global__ void gibbs_exact_rec_kernel(const XPrep *preps, const double *ctrs_ba
     const bool ok = z < pd.n;  // an odd level is padded with a node of probability zero (finite: no 0 * inf)
     const double *r = pd.src + (size_t)(ok ? z : 0) * pd.src_stride;
     for (int k = 0; k < D; ++k) o[2 * k + hh] = ok ? (float)(r[k] - c[k]) : 0.f;
-    for (int k = 0; k < nb; ++k) o[2 * (D + k) + hh] = ok ? (float)r[D + k] : 1.f;
+    for (int k = 0; k < nb; ++k)
+      o[2 * (D + k) + hh] = ok ? (float)(pd.var == VAR_B ? -r[D + k] * GF_LOG2E : r[D + k]) : (pd.var == VAR_B ? 0.f : 1.f);
     o[2 * (D + nb) + hh] = ok ? (float)fmax(pd.lw2max - r[D + nb] * GF_LOG2E, 0.0) : 1e30f;
   }
   for (int k = 2 * (D + nb + 1); k < stride; ++k) o[k] = 0.f;
 }
 
 // ---- schedule ---------------------------------------------------------------------------------------------------
-// plan_schedule(.., f32_leaf = true, f32_internal = false) gives every leaf draw FP32 records; this moves the sampleIndex
-// draws (variant C) of internal levels of at least GX_NMIN nodes onto FP32 records as well, with K1f's chunk and tile
-// rule, and rebuilds the tile stream.  Smaller internal levels and every sampleIndices! draw (variant B) keep K1's
-// FP64 tiles: those levels hold a few per cent of the nodes.
+// plan_schedule(.., b_records = true, f32_leaf = true, f32_internal = false) gives every leaf draw FP32 records; this
+// moves every internal draw (variants B and C) onto FP32 records as well, with K1f's chunk and tile rule, and rebuilds
+// the tile stream.  The draws keep K1's FP64 records in `rec`: the FP64 redo reads them.
 void gibbs_exact_plan(const kdeb200_tree_t *trees, Plan &S) {
   const int d = trees[0]->d;
-  const int stride = gf_stride(d, VAR_C);
+  const int stride = gf_stride(d, VAR_C);  // == gf_stride(d, VAR_B)
   std::vector<PlanTile> tiles;
   for (size_t i = 0; i < S.draws.size(); ++i) {
     Draw &dr = S.draws[i];
     const int t0 = dr.tile0;
     dr.tile0 = (int)tiles.size();
-    if (S.block[i] >= 0 || dr.variant != VAR_C || dr.n < GX_NMIN) {
+    if (S.block[i] >= 0) {
       tiles.insert(tiles.end(), S.tiles.begin() + t0, S.tiles.begin() + t0 + dr.ntiles);
       continue;
     }
     const kdeb200_tree_s *t = trees[dr.j];
     int G = 2;
     while ((int64_t)G * GB_MAXCK < dr.n) G *= 2;
-    const int want = 4 * gf_unr(d, VAR_C);
+    const int want = 4 * gf_unr(d, dr.variant);
     if (G < want && dr.n >= 2 * want) G = want;
     int tn = 2;
     while ((size_t)tn * stride * sizeof(float) <= GB_TILE_BYTES) tn *= 2;
@@ -122,7 +125,7 @@ void gibbs_exact_plan(const kdeb200_tree_t *trees, Plan &S) {
     dr.tnodes = tn;
     dr.nchunks = (dr.n + G - 1) / G;
     dr.ntiles = (dr.n + tn - 1) / tn;
-    const int blk = plan_block(S, dr.j, dr.level < t->depth ? dr.level : t->depth, VAR_C, dr.n, stride, tn);
+    const int blk = plan_block(S, dr.j, dr.level < t->depth ? dr.level : t->depth, dr.variant, dr.n, stride, tn);
     S.block[i] = blk;
     for (int a = 0; a < dr.n; a += tn) {
       const int cnt = (dr.n - a < tn) ? (dr.n - a) : tn;
@@ -133,7 +136,7 @@ void gibbs_exact_plan(const kdeb200_tree_t *trees, Plan &S) {
   S.tiles.swap(tiles);
 }
 
-// Every block of the plan holds FP32 records (a leaf level, or a certified internal level).  Pass a on the device, tile
+// Every block of the plan holds FP32 records (a leaf level, or an internal level's B or C records).  Pass a on the device, tile
 // centres / radii / variance ranges / largest weights on the host, pass b on the device; the persistent XDraws and
 // centres go to e.d_extra.
 int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
@@ -156,7 +159,7 @@ int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
   for (size_t i = 0; i < S.blocks.size(); ++i) {
     const kdeb200_tree_s *t = trees[S.blocks[i].j];
     const Level &lv = t->levels[S.blocks[i].level];
-    const bool isC = S.blocks[i].variant == VAR_C;
+    const int var = S.blocks[i].variant;
     XBlock &b = blk[i];
     b.ntiles = (int)((lv.n + S.blocks[i].tnodes - 1) / S.blocks[i].tnodes);
     b.ctr_off = coff[i] = nctr;
@@ -164,11 +167,11 @@ int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
     nctr += (size_t)b.ntiles * KDEB200_MAX_DIM;
     nstats += (size_t)b.ntiles * SW;
     XPrep &xp = preps[i];
-    xp.src = t->d_buf + (isC ? lv.offC : lv.offA);
+    xp.src = t->d_buf + (var == VAR_A ? lv.offA : var == VAR_B ? lv.offB : lv.offC);
     xp.dst = e.d_rec + S.blocks[i].off;
     xp.stats = nullptr;
     xp.n = (int)lv.n;
-    xp.src_stride = isC ? t->SC : t->SA;
+    xp.src_stride = var == VAR_A ? t->SA : t->SC;
     xp.tnodes = S.blocks[i].tnodes;
     xp.var = S.blocks[i].variant;
     xp.lw2max = 0.0;
@@ -202,7 +205,7 @@ int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
         for (size_t i = 0; i < blk.size(); ++i) {
           XBlock &b = blk[i];
           double lwmax = -INFINITY;
-          if (preps[i].var == VAR_C)
+          if (preps[i].var != VAR_A)
             for (int k = 0; k < d; ++k) b.bmin[k] = INFINITY;
           for (int tt = 0; tt < b.ntiles; ++tt) {
             const double *sv = &st[b.stats_off + (size_t)tt * SW];
@@ -214,10 +217,12 @@ int gibbs_exact_build(const kdeb200_tree_t *trees, Plan &S, SchedEntry &e) {
               const double r = std::fmax(hi - cc, cc - lo) * (1.0 + 1e-15) + std::fabs(cc) * 0x1.0p-51;
               if (!(r <= 1e20)) b.fp32 = false;  // outside FP32's comfortable range: FP64 redo for the whole level
               if (r > b.rad[k]) b.rad[k] = r;
-              if (preps[i].var == VAR_C) {
-                // c_k = b_k + Calmost_k in FP32 needs b_k in (0, 2^29]; the kernel checks Calmost per chain
-                const double bl = sv[2 * KDEB200_MAX_DIM + k], bh = sv[3 * KDEB200_MAX_DIM + k];
-                if (!(bl > 0.0) || !(bh <= 0x1.0p29)) b.fp32 = false;
+              if (preps[i].var != VAR_A) {
+                // c_k = b_k + Calmost_k in FP32 needs b_k in (0, 2^29]; the kernel checks Calmost per chain.  Variant B
+                // keeps b_k in the same range; its records hold -0.5/b_k, whose smallest value belongs to the smallest b_k
+                double bl = sv[2 * KDEB200_MAX_DIM + k], bh = sv[3 * KDEB200_MAX_DIM + k];
+                if (preps[i].var == VAR_B) bl = -0.5 / bl, bh = -0.5 / bh;
+                if (!(bl > 0.0) || !(bh > 0.0) || !(bh <= 0x1.0p29)) b.fp32 = false;
                 b.bmin[k] = std::fmin(b.bmin[k], bl);
               }
             }
@@ -286,6 +291,8 @@ int gibbs_exact_launch(GibbsParams &P, const SchedEntry &E, int d, cudaStream_t 
   X.warp_redone = d_count + 2;
   X.redone_int = d_count + 3;
   X.warp_redone_int = d_count + 4;
+  X.redone_b = d_count + 5;
+  X.warp_redone_b = d_count + 6;
   X.scr_stride = GX_SCR + E.redo_blocks;
   // The redo scratch belongs to this launch alone, stream-ordered on `st`: launches on other streams may be in flight
   // at the same time, and a warp that shared its (block, warp) slot with another launch would sum foreign terms.
@@ -298,8 +305,8 @@ int gibbs_exact_launch(GibbsParams &P, const SchedEntry &E, int d, cudaStream_t 
 }
 
 // ---- bound probe (tests) ------------------------------------------------------------------------------------------
-// For query conditionals (mu, Calmost) of one certified draw (the leaf draw, variant A, or the first sampleIndex draw of
-// an internal level, variant C): every node's FP32 term as K1x computes it, its bound, K1's FP64 term, K1's prefix sums,
+// For query conditionals (mu, Calmost) of one certified draw (the leaf draw, variant A; on an internal level the first
+// sampleIndex draw, variant C, or with pass0 the sampleIndices! draw, variant B, which ignores Calmost): every node's FP32 term as K1x computes it, its bound, K1's FP64 term, K1's prefix sums,
 // and the intervals K1x would claim for them -- per node as xa_decide forms them, and at checkpoints as xa_pass1 forms
 // them (trip sums in FP32, Q in FP32 per chunk).  One CTA per query.
 // out per query: [A, B, aabs, ok, lw2max, n, G, W] then per node [p32, acc32, p64, S64, lo, hi, lo_ck, hi_ck]
@@ -315,20 +322,19 @@ __global__ void gibbs_exact_probe_kernel(Draw dr, XDraw xd, const double *mu_all
   double *out = out_all + (size_t)qi * (GX_PROBE_HDR + (size_t)GX_PROBE_NODE * dr.n);
   double mu[D];
   Hoist<D, false> h;
-  float s32[D];
+  double cadd[D];
   for (int k = 0; k < D; ++k) {  // the expressions of gibbs_exact_kernel
     mu[k] = mu_all[qi * D + k];
     h.mu[k] = mu[k];
-    h.cadd[k] = cadd_all[qi * D + k];
+    cadd[k] = VAR == VAR_B ? 0.0 : cadd_all[qi * D + k];
+    h.cadd[k] = cadd[k];
     h.act[k] = true;
-    const double c = P.hvar[j][k] + h.cadd[k];
-    h.ich[k] = sqrt(0.5 / c);
-    s32[k] = (float)sqrt(GF_HL2E / c);
+    h.ich[k] = sqrt(0.5 / (P.hvar[j][k] + h.cadd[k]));
   }
   Hoist32<D> g;
   float ks[D], sv[D];
   double rsmax;
-  const bool rok = x_chain<D, VAR>(xd, h, s32, ks, sv, g, rsmax);
+  const bool rok = x_chain<D, VAR>(xd, cadd, P.hvar[j], ks, sv, g, rsmax);
   XBound bd = xa_bound<D, VAR>(xd, ks, rsmax, dr.n, GX_EX2_ERR, GX_RSQ_ERR, 1.0);
   bd.ok = bd.ok && rok;
   for (int z = threadIdx.x; z < dr.n; z += blockDim.x) {
@@ -384,7 +390,7 @@ __global__ void gibbs_exact_probe_kernel(Draw dr, XDraw xd, const double *mu_all
   }
 }
 
-int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, int level, const double *mu,
+int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, int level, int pass0, const double *mu,
                       const double *cadd, int nq, double *out, int64_t out_len) {
   if (!trees || ndens < 1 || ndens > KDEB200_MAX_DENS || j < 0 || j >= ndens || nq < 1 || !mu || !cadd || !out)
     KDE_FAIL(3, "gibbs_exact_probe: bad arguments");
@@ -404,7 +410,7 @@ int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, 
   KDE_CUDA(cudaMemcpy(xds.data(), E.d_xd, sizeof(XDraw) * E.ndraws, cudaMemcpyDeviceToHost));
   int di = -1;
   for (int i = 0; i < E.ndraws && di < 0; ++i)
-    if (draws[i].j == j && draws[i].level == level && (draws[i].variant == VAR_A || (draws[i].kind == 1 && xds[i].rec32)))
+    if (draws[i].j == j && draws[i].level == level && (draws[i].variant == VAR_A || draws[i].kind == (pass0 ? 0 : 1)))
       di = i;
   if (di < 0) KDE_FAIL(3, "gibbs_exact_probe: level %d of density %d has no certified draw", level, j + 1);
   const size_t per = GX_PROBE_HDR + (size_t)GX_PROBE_NODE * draws[di].n;
@@ -422,6 +428,8 @@ int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, 
   if (err == cudaSuccess) {
     if (draws[di].variant == VAR_A)
       gibbs_exact_probe_kernel<3, VAR_A><<<nq, 128, 0, c.stream>>>(draws[di], xds[di], d_mu, d_mu + nq * d, P, j, d_out);
+    else if (draws[di].variant == VAR_B)
+      gibbs_exact_probe_kernel<3, VAR_B><<<nq, 128, 0, c.stream>>>(draws[di], xds[di], d_mu, d_mu + nq * d, P, j, d_out);
     else
       gibbs_exact_probe_kernel<3, VAR_C><<<nq, 128, 0, c.stream>>>(draws[di], xds[di], d_mu, d_mu + nq * d, P, j, d_out);
     err = cudaGetLastError();

@@ -1,16 +1,15 @@
 // gibbs_exact_kernel.cuh -- K1x (device code and launch template; gibbs_exact.cu holds the host side,
-// gibbs_exact_d<N>.cu one explicit instantiation per d): the FP64 Gibbs sampler with the labels of the leaf levels and of
-// the large internal sampleIndex levels DECIDED from certified FP32 prefix sums.
+// gibbs_exact_d<N>.cu one explicit instantiation per d): the FP64 Gibbs sampler with every label DECIDED from certified
+// FP32 prefix sums.
 //
 // Same schedule, chain state, RNG addressing and outputs as gibbs_kernel (K1), bit for bit.  K1 picks on every level
-// the first z with target = fl(u * pT) <= S_z, S_z its sequential FP64 prefix sums (else n - 1).  On the leaf levels
-// (variant A) and on the sampleIndex draws of internal levels of at least GX_NMIN nodes (variant C) K1x instead
-// evaluates the nodes in packed FP32 (gibbs_f32_kernel.cuh's pair records and arithmetic) and carries next to every FP32
-// prefix sum S'_z a bound E_z on |S'_z - S_z / W| (W: the level's largest weight; DESIGN.md "K1x" derives it).  A lane's
-// label is taken only when the intervals prove it:  hi(S_{z-1}) < lo(target)  and  hi(target) <= lo(S_z).  A lane that
-// cannot prove its label is redone by its warp with K1's FP64 arithmetic (K1w's scheme: lanes evaluate, one lane sums
-// in node order, the result is K1's label by construction).  The other internal draws (variant B, small levels) run
-// K1's own pass1 / pass2 unchanged.
+// the first z with target = fl(u * pT) <= S_z, S_z its sequential FP64 prefix sums (else n - 1).  On every draw -- leaf
+// levels (variant A), the sampleIndices! draws (variant B) and the sampleIndex draws (variant C) of internal levels --
+// K1x instead evaluates the nodes in packed FP32 (gibbs_f32_kernel.cuh's pair records and arithmetic) and carries next
+// to every FP32 prefix sum S'_z a bound E_z on |S'_z - S_z / W| (W: the level's largest weight; DESIGN.md "K1x" derives
+// it).  A lane's label is taken only when the intervals prove it:  hi(S_{z-1}) < lo(target)  and  hi(target) <= lo(S_z).
+// A lane that cannot prove its label is redone by its warp with K1's FP64 arithmetic (K1w's scheme: lanes evaluate, one
+// lane sums in node order, the result is K1's label by construction), reading K1's exp table from global memory.
 #pragma once
 #include <type_traits>
 
@@ -20,14 +19,18 @@ namespace kdeb200 {
 
 constexpr int GX_SCR = 256;   // nodes per block of the cooperative FP64 redo (its per-warp global scratch: GX_SCR doubles
                               // of terms, then one running sum per block)
-constexpr int GX_NMIN = 256;  // internal sampleIndex levels of at least this many nodes are certified in FP32
+// resident CTAs per SM the register budget is cut for: 4 (128 registers), the fastest of 4 / 5 / 6 / 8 at d = 3 now that
+// no exp table limits the shared memory (DESIGN.md "K1x" has the sweep)
+#ifndef GX_MINBLOCKS
+#define GX_MINBLOCKS 4
+#endif
 
 // per-draw extras of K1x (certified draws only; zero elsewhere)
 struct alignas(16) XDraw {
   const float *rec32;                 // FP32 pair records, coordinates relative to the tile centre
   const double *ctr;                  // tile centres, KDEB200_MAX_DIM doubles per tile of this draw
   double rad[KDEB200_MAX_DIM];        // max over the level of |m - centre| per dimension (FP64, rounded up)
-  double bmin[KDEB200_MAX_DIM];       // variant C: the level's smallest node variance b_k per dimension
+  double bmin[KDEB200_MAX_DIM];       // variants B, C: the level's smallest node variance b_k per dimension
   double lw2max;                      // log2 of the level's largest weight (records hold lw2max - log2 w >= 0)
   int G, nchunks;                     // K1x's own checkpoint chunks (nodes, power of two)
   int fp32;                           // 0: the level is outside the FP32 range guard, every lane takes the FP64 redo
@@ -39,8 +42,10 @@ struct XParams {
   double *scratch;                    // scr_stride doubles per warp of the grid
   unsigned long long *redone;         // leaf lane-draws redone in FP64 (live chains only)
   unsigned long long *warp_redone;    // leaf warp-draws with at least one redone lane
-  unsigned long long *redone_int;     // the same two for the certified internal draws
+  unsigned long long *redone_int;     // the same two for the sampleIndex draws of internal levels (variant C)
   unsigned long long *warp_redone_int;
+  unsigned long long *redone_b;       // the same two for the sampleIndices! draws (variant B)
+  unsigned long long *warp_redone_b;
   double ex2_err;                     // relative error bound of ex2.approx.ftz.f32 on [-126, 0]
   double rsq_err;                     // relative error bound of rsqrt.approx.ftz.f32 on normal floats
   double inflate;                     // test hook: multiplies the bound (1 in production)
@@ -54,35 +59,43 @@ struct XBound {
   bool ok;
 };
 
-// The per-chain FP32 constants of a certified draw, from K1's FP64 conditionals h:
-//   ks: kernel-width scale per dimension (A: s_k = sqrt(0.5 log2e / c_k); C: the same for the level's narrowest
-//       c_k = b_min,k + Calmost_k), which measures the tile radii of the bound;
-//   sv: what the tile hoist clamps with (A: s_k; C: |mu - centre| <= 1e12 kernel widths);
-//   g.a, g.c: A: s_k; C: 1 and Calmost_k, so that gf_pre forms c_k = b_k + Calmost_k and d_k = m'_k - (mu_k - centre_k);
-//   rsmax: C: the largest normaliser prod_k c_k^-1/2 of the level (1 for A).
-// Returns false when a variant-C chain's c_k could leave [2^-30, 2^30] (FP32 products of three of them stay normal).
+// The per-chain FP32 constants of a certified draw, from K1's FP64 conditional (Calmost = cadd, leaf variances hvar):
+//   ks: kernel-width scale per dimension (A: s_k = sqrt(0.5 log2e / c_k), c_k = hvar_k + Calmost_k; B: the same for the
+//       level's narrowest b_min,k; C: for the level's narrowest c_k = b_min,k + Calmost_k), which measures the tile
+//       radii of the bound;
+//   sv: what the tile hoist clamps with (A: s_k; B, C: |mu - centre| <= 1e12 kernel widths);
+//   g.a, g.c: A: s_k; B: 1; C: 1 and Calmost_k, so that gf_pre forms c_k = b_k + Calmost_k and
+//       d_k = m'_k - (mu_k - centre_k);
+//   rsmax: C: the largest normaliser prod_k c_k^-1/2 of the level (1 for A and B).
+// Returns false when a variant-C chain's c_k could leave [2^-30, 2^30] (FP32 products of three of them stay normal), or
+// a variant-B level's b_min,k lies below 2^-30 (the scale ks would be clamped, and the radii of the bound with it).
 template <int D, int VAR>
-__device__ __forceinline__ bool x_chain(const XDraw &xd, const Hoist<D, false> &h, const float (&s32)[D], float (&ks)[D],
-                                        float (&sv)[D], Hoist32<D> &g, double &rsmax) {
+__device__ __forceinline__ bool x_chain(const XDraw &xd, const double (&cadd)[D], const double *__restrict__ hvar,
+                                        float (&ks)[D], float (&sv)[D], Hoist32<D> &g, double &rsmax) {
   bool ok = true;
   rsmax = 1.0;
 #pragma unroll
   for (int k = 0; k < D; ++k) {
     if (VAR == VAR_A) {
-      ks[k] = sv[k] = s32[k];
-      g.a[k] = gf_pack(s32[k], s32[k]);
+      const float s = (float)sqrt(GF_HL2E / (hvar[k] + cadd[k]));  // c_k as K1 forms it
+      ks[k] = sv[k] = s;
+      g.a[k] = gf_pack(s, s);
     } else {
-      const double cm = xd.bmin[k] + h.cadd[k];  // <= every node's c_k
-      ok = ok && cm >= 0x1.0p-30 && h.cadd[k] <= 0x1.0p29;  // the host keeps b_k <= 2^29
+      const double cm = (VAR == VAR_B) ? xd.bmin[k] : xd.bmin[k] + cadd[k];  // <= every node's b_k / c_k
+      // below 2^-30 the clamp in ks would shrink the radii of the bound: such a draw is not decided (both variants)
+      ok = ok && cm >= 0x1.0p-30;
+      if (VAR == VAR_C) ok = ok && cadd[k] <= 0x1.0p29;  // the host keeps b_k <= 2^29
       ks[k] = (float)sqrt(GF_HL2E / fmax(cm, 0x1.0p-30));
       sv[k] = (float)(1e12 / (double)ks[k]);
       rsmax *= cm;
-      const float cf = (float)h.cadd[k];
       g.a[k] = gf_pack(1.f, 1.f);
-      g.c[k] = gf_pack(cf, cf);
+      if (VAR == VAR_C) {
+        const float cf = (float)cadd[k];
+        g.c[k] = gf_pack(cf, cf);
+      }
     }
   }
-  if (VAR == VAR_C) rsmax = 1.0 / sqrt(fmax(rsmax, 1e-300));
+  rsmax = (VAR == VAR_C) ? 1.0 / sqrt(fmax(rsmax, 1e-300)) : 1.0;
   return ok;
 }
 
@@ -99,9 +112,10 @@ __device__ __forceinline__ XBound xa_bound(const XDraw &xd, const float (&ks)[D]
     R2 += R * R;
   }
   // variant C: d_k is one FFMA (4.02u on t^2 instead of A's 6.02u), c_k = b_k + Calmost_k 2.01u, the reciprocals from
-  // rs^2 and two products 2 eps_rsq + 5u, D + 3 roundings of the non-negative sum
+  // rs^2 and two products 2 eps_rsq + 5u, D + 3 roundings of the non-negative sum.  Variant B: d_k as C (4.02u), the
+  // record's 0.5 log2e / b_k 1.01u, the FMUL of d^2 u, D FFMA and lw' (D + 1)u: A's (D + 7.03)u
   constexpr int ng = (D + 3) / 4;  // rsqrt groups of gf_pre
-  const double a1 = (VAR == VAR_A ? (D + 7.2) * u : (D + 14.2) * u + 2.02 * rsq_err) + 2.05 * u * Rmax;
+  const double a1 = (VAR != VAR_C ? (D + 7.2) * u : (D + 14.2) * u + 2.02 * rsq_err) + 2.05 * u * Rmax;
   const double a0 = 2.05 * u * Rsum + 1e-13 * R2;
   XBound b;
   b.ok = xd.fp32 && (a1 * 130.0 + a0 <= 1e-3) && (R2 == R2);
@@ -114,12 +128,12 @@ __device__ __forceinline__ XBound xa_bound(const XDraw &xd, const float (&ks)[D]
   b.B = inflate * qsum * (1.003 * ln2 * 1.001 * a1 + 5e-15);
   // variant C: the normaliser rs32 = fl(rsqrt(fl(prod c32))) against prod c^-1/2, and the product ex2 * rs32; K1's
   // own FP64 rsqrt, products and reciprocals as a further relative 1e-14
-  const double norm = (VAR == VAR_A) ? 0.0 : 1.01 * (ng * rsq_err + (1.51 * D + 2.0 * ng) * u) + 1e-14;
+  const double norm = (VAR != VAR_C) ? 0.0 : 1.01 * (ng * rsq_err + (1.51 * D + 2.0 * ng) * u) + 1e-14;
   b.A = inflate * (1.003 * (ln2 * (a0 + 1.001 * a1 * a0) + 1.01 * ex2_err + norm) + 2.0 * gf_unr(D, VAR) * 1.01 * u +
                    (double)n * 0x1.0p-52 + 1e-15 * (6.0 + lwm));
   // ex2.approx.ftz flushes 2^-acc below 2^-126 to zero (variant C: times the normaliser, and the FP32 product may be
   // subnormal); K1 clamps exponents below -700 (kde_exp_flush)
-  b.aabs = (VAR == VAR_A) ? 0x1.0p-125 + exp(-699.0 - xd.lw2max * ln2)
+  b.aabs = (VAR != VAR_C) ? 0x1.0p-125 + exp(-699.0 - xd.lw2max * ln2)
                           : 1.01 * (0x1.0p-125 * (1.0 + rsmax) + exp(-699.0 - xd.lw2max * ln2) * rsmax);
   b.eta = (double)n * 1.2e-16 + 1e-15;
   return b;
@@ -338,20 +352,42 @@ __device__ __noinline__ int xa_redo(const Draw &dr, const Hoist<D, false> &h, do
   return f;
 }
 
+// K1's conditional of a draw, from the chain state and with K1's expressions (so its FP64 values are K1's): sampleIndices!
+// (kind 0) evaluates against the level's point X, sampleIndex (kind 1) against the product of the other densities'
+// selected kernels.  The certified draw calls it again where it needs Calmost after pass 1, instead of keeping it live.
 template <int D, int MD>
-__global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_exact_kernel(const __grid_constant__ GibbsParams P,
-                                                                               const __grid_constant__ XParams X) {
-  constexpr bool MASK = false;
+__device__ __forceinline__ void x_cond(int kind, int j, int M, const double (&lam)[MD * D], const double (&lmu)[MD * D],
+                                       const double (&X)[D], double (&mu)[D], double (&cadd)[D]) {
+#pragma unroll
+  for (int k = 0; k < D; ++k) {
+    if (kind == 0) {
+      mu[k] = X[k];
+      cadd[k] = 0.0;
+      continue;
+    }
+    double Lm = 0.0, Hm = 0.0;
+    for (int i = 0; i < M; ++i) {
+      if (i == j) continue;
+      Lm += lam[i * D + k];
+      Hm += lmu[i * D + k];
+    }
+    const double cov = 1.0 / Lm;  // M > 1 on this route
+    cadd[k] = cov;
+    mu[k] = cov * Hm;
+  }
+}
+
+template <int D, int MD>
+__global__ void __launch_bounds__(GB_THREADS, GX_MINBLOCKS) gibbs_exact_kernel(const __grid_constant__ GibbsParams P,
+                                                                                   const __grid_constant__ XParams X) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double *tiles = reinterpret_cast<double *>(smem_raw);
-  __shared__ __align__(16) double tab[KDE_EXP_TAB];
   __shared__ __align__(8) uint64_t bars[GB_STAGES];
   const int tid = threadIdx.x, lane = tid & 31;
   const int M = P.M;
   const unsigned FULL = 0xffffffffu;
   double *scr = X.scratch + ((size_t)blockIdx.x * (GB_THREADS / 32) + (tid >> 5)) * X.scr_stride;
 
-  for (int i = tid; i < KDE_EXP_TAB; i += GB_THREADS) tab[i] = P.exptab[i];
   if (tid == 0) {
     for (int s = 0; s < GB_STAGES; ++s) mbar_init(&bars[s], 1);
     mbar_fence_init();
@@ -384,7 +420,7 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_exact_kernel(c
   double ck[GB_MAXCK];
   float ckq[GB_MAXCK];
   int selpos[MD];
-  unsigned redone = 0, wredone = 0, redone_i = 0, wredone_i = 0;
+  unsigned redone[3] = {0, 0, 0}, wredone[3] = {0, 0, 0};  // per variant
 
   while (batch < P.nbatches) {
     int64_t s = P.s0 + (int64_t)batch * GB_THREADS + tid;
@@ -432,143 +468,76 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_exact_kernel(c
         }
       }
 
-      Hoist<D, MASK> h;
-      double scale = 1.0;
-      if (dr.kind == 0) {
-#pragma unroll
-        for (int k = 0; k < D; ++k) {
-          h.mu[k] = X_[k];
-          h.cadd[k] = 0.0;
-          h.act[k] = true;
-        }
-      } else {
-#pragma unroll
-        for (int k = 0; k < D; ++k) {
-          double Lm = 0.0, Hm = 0.0;
-          for (int i = 0; i < M; ++i) {
-            if (i == j) continue;
-            Lm += lam[i * D + k];
-            Hm += lmu[i * D + k];
-          }
-          const double cov = 1.0 / Lm;  // M > 1 on this route
-          h.cadd[k] = cov;
-          h.mu[k] = cov * Hm;
-          h.act[k] = true;
-        }
-      }
-      float s32[D];
-      if (dr.variant == VAR_A) {
-        double prod = 1.0;
-#pragma unroll
-        for (int k = 0; k < D; ++k) {
-          const double c = P.hvar[j][k] + h.cadd[k];
-          h.ich[k] = sqrt(0.5 / c);
-          prod *= c;
-          s32[k] = (float)sqrt(GF_HL2E / c);
-        }
-        scale = kde_rsqrt(prod);
-      }
-
       // a certified draw: FP32 pass 1, the bound, the FP32 decision, the FP64 redo of the lanes it leaves undecided
       auto certified = [&](auto var) -> int {
         constexpr int VAR = decltype(var)::value;
         const XDraw xd = X.xd[di];
         Hoist32<D> g;
         float ks[D], sv[D];
-        double rsmax;
-        const bool rok = x_chain<D, VAR>(xd, h, s32, ks, sv, g, rsmax);
+        double rsmax, mu[D];
+        bool rok;
+        {
+          double cadd[D];
+          x_cond<D, MD>(dr.kind, j, M, lam, lmu, X_, mu, cadd);
+          rok = x_chain<D, VAR>(xd, cadd, P.hvar[j], ks, sv, g, rsmax);
+        }
         double Qt;
-        const double pT = xa_pass1<D, VAR>(dr, xd, h.mu, sv, g, R, q, ck, ckq, Qt);
+        const double pT = xa_pass1<D, VAR>(dr, xd, mu, sv, g, R, q, ck, ckq, Qt);
         int z = 0;
-        bool und = false;
-        double u = 0.0;
-        if (dr.n > 1) {
-          const uint32_t c = (uint32_t)(M + di);
-          u = P.randU ? P.randU[s * P.perU + c - 1] : philox_uniform(P.seed, (uint64_t)s, c);
-          XBound bd = xa_bound<D, VAR>(xd, ks, rsmax, dr.n, X.ex2_err, X.rsq_err, X.inflate);
-          bd.ok = bd.ok && rok;
-          const double E = xa_err(bd, pT, Qt, dr.n);
-          const double pLo = (pT - E) * (1.0 - bd.eta), pHi = (pT + E) * (1.0 + bd.eta);
-          // K1's pT * scale < 1e-99 rule (scale = 1 on internal levels) must provably not fire; u in [0, 1) keeps the
-          // target interval ordered
-          und = !(bd.ok && u >= 0.0 && u < 1.0 && pLo > 0.0 && pLo * exp2(xd.lw2max) * scale >= 1.000001e-99);
-          if (!und) {
-            const double tLo = u * pLo * (1.0 - 0x1.0p-50), tHi = u * pHi * (1.0 + 0x1.0p-50);
-            z = xa_decide<D, VAR>(dr, xd, bd, h.mu, sv, g, ck, ckq, u * pT, tLo, tHi);
-            und = z < 0;
-          }
-        }
-        unsigned ub = __ballot_sync(FULL, und);
-        if (ub) {
-          if (live && und) ++(VAR == VAR_A ? redone : redone_i);
-          if (lane == 0) ++(VAR == VAR_A ? wredone : wredone_i);
-        }
-        while (ub) {
-          const int L = __ffs(ub) - 1;
-          ub &= ub - 1;
-          Hoist<D, MASK> hl;
-#pragma unroll
-          for (int k = 0; k < D; ++k) {
-            hl.mu[k] = __shfl_sync(FULL, h.mu[k], L);
-            hl.ich[k] = __shfl_sync(FULL, h.ich[k], L);
-            hl.cadd[k] = __shfl_sync(FULL, h.cadd[k], L);
-            hl.act[k] = true;
-          }
-          const int zl = xa_redo<D, VAR>(dr, hl, __shfl_sync(FULL, scale, L), __shfl_sync(FULL, u, L), tab, P.ec, scr);
-          if (lane == L) z = zl;
-        }
-        return z;
-      };
-      int zs = 0;
-      if (dr.variant == VAR_A) {
-        zs = certified(std::integral_constant<int, VAR_A>());
-      } else if (dr.variant == VAR_C && X.xd[di].rec32) {
-        zs = certified(std::integral_constant<int, VAR_C>());
-      } else {  // internal levels: K1's own arithmetic
-        double pT;
-        if (dr.variant == VAR_B)
-          pT = pass1<D, MASK, VAR_B>(dr, h, tab, P.ec, R, q, ck);
-        else
-          pT = pass1<D, MASK, VAR_C>(dr, h, tab, P.ec, R, q, ck);
         if (dr.n > 1) {
           const uint32_t c = (uint32_t)(M + di);
           const double u = P.randU ? P.randU[s * P.perU + c - 1] : philox_uniform(P.seed, (uint64_t)s, c);
-          if (pT * scale < 1e-99) {
-            const double w = dr.wts[dr.n - 1];
-            double tot = 0.0;
-            for (int z = 0; z < dr.n; ++z) tot += w;
-            const double qv = w / tot;
-            double cdf = 0.0;
-            zs = dr.n - 1;
-            bool found = false;
-            for (int z = 0; z < dr.n - 1; ++z) {
-              cdf += qv;
-              if (!found && u <= cdf) {
-                zs = z;
-                found = true;
+          XBound bd = xa_bound<D, VAR>(xd, ks, rsmax, dr.n, X.ex2_err, X.rsq_err, X.inflate);
+          bd.ok = bd.ok && rok;
+          double scale = 1.0;  // K1's normaliser of a leaf draw; internal draws have none (K1's scale = 1)
+          if (VAR == VAR_A) {
+            double mu2[D], cadd[D], prod = 1.0;
+            x_cond<D, MD>(dr.kind, j, M, lam, lmu, X_, mu2, cadd);
+#pragma unroll
+            for (int k = 0; k < D; ++k) prod *= P.hvar[j][k] + cadd[k];
+            scale = kde_rsqrt(prod);
+          }
+          const double E = xa_err(bd, pT, Qt, dr.n);
+          const double pLo = (pT - E) * (1.0 - bd.eta), pHi = (pT + E) * (1.0 + bd.eta);
+          // K1's pT * scale < 1e-99 rule must provably not fire; u in [0, 1) keeps the target interval ordered
+          bool und = !(bd.ok && u >= 0.0 && u < 1.0 && pLo > 0.0 && pLo * exp2(xd.lw2max) * scale >= 1.000001e-99);
+          if (!und) {
+            const double tLo = u * pLo * (1.0 - 0x1.0p-50), tHi = u * pHi * (1.0 + 0x1.0p-50);
+            z = xa_decide<D, VAR>(dr, xd, bd, mu, sv, g, ck, ckq, u * pT, tLo, tHi);
+            und = z < 0;
+          }
+          unsigned ub = __ballot_sync(FULL, und);
+          if (ub) {
+            if (live && und) ++redone[VAR];
+            if (lane == 0) ++wredone[VAR];
+            double cadd[D];
+            x_cond<D, MD>(dr.kind, j, M, lam, lmu, X_, mu, cadd);
+            while (ub) {
+              const int L = __ffs(ub) - 1;
+              ub &= ub - 1;
+              Hoist<D, false> hl;
+#pragma unroll
+              for (int k = 0; k < D; ++k) {
+                hl.mu[k] = __shfl_sync(FULL, mu[k], L);
+                hl.cadd[k] = __shfl_sync(FULL, cadd[k], L);
+                hl.ich[k] = (VAR == VAR_A) ? sqrt(0.5 / (P.hvar[j][k] + hl.cadd[k])) : 0.0;  // K1's expression
+                hl.act[k] = true;
               }
-            }
-          } else {
-            const double target = u * pT;
-            int lo = 0, hi = dr.nchunks;
-            while (lo < hi) {
-              const int mid = (lo + hi) >> 1;
-              if (target <= ck[mid]) hi = mid; else lo = mid + 1;
-            }
-            if (lo >= dr.nchunks) {
-              zs = dr.n - 1;
-            } else if (dr.G == 1) {
-              zs = lo;
-            } else {
-              const double S0 = lo > 0 ? ck[lo - 1] : 0.0;
-              if (dr.variant == VAR_B)
-                zs = pass2<D, MASK, VAR_B>(dr, h, tab, P.ec, lo, S0, target);
-              else
-                zs = pass2<D, MASK, VAR_C>(dr, h, tab, P.ec, lo, S0, target);
+              const int zl = xa_redo<D, VAR>(dr, hl, __shfl_sync(FULL, scale, L), __shfl_sync(FULL, u, L), P.exptab,
+                                             P.ec, scr);
+              if (lane == L) z = zl;
             }
           }
         }
-      }
+        return z;
+      };
+      int zs;
+      if (dr.variant == VAR_A)
+        zs = certified(std::integral_constant<int, VAR_A>());
+      else if (dr.variant == VAR_B)
+        zs = certified(std::integral_constant<int, VAR_B>());
+      else
+        zs = certified(std::integral_constant<int, VAR_C>());
       selpos[j] = zs;
       if (P.level_labels && dr.kind == 1 && live)
         P.level_labels[((s - P.s0) * M + j) * P.L + (dr.level - 1)] = dr.levperm[zs];
@@ -608,10 +577,13 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_exact_kernel(c
     }
     batch = batch_next;
   }
-  if (redone) atomicAdd(X.redone, (unsigned long long)redone);
-  if (wredone) atomicAdd(X.warp_redone, (unsigned long long)wredone);
-  if (redone_i) atomicAdd(X.redone_int, (unsigned long long)redone_i);
-  if (wredone_i) atomicAdd(X.warp_redone_int, (unsigned long long)wredone_i);
+  unsigned long long *const lanes_out[3] = {X.redone, X.redone_b, X.redone_int};
+  unsigned long long *const warps_out[3] = {X.warp_redone, X.warp_redone_b, X.warp_redone_int};
+#pragma unroll
+  for (int v = 0; v < 3; ++v) {
+    if (redone[v]) atomicAdd(lanes_out[v], (unsigned long long)redone[v]);
+    if (wredone[v]) atomicAdd(warps_out[v], (unsigned long long)wredone[v]);
+  }
 }
 
 template <int D>

@@ -31,7 +31,12 @@ extern "C" {
 #endif
 
 #define KDEB200_MAX_DIM 8
+/* KDEB200_MAX_DENS bounds the densities of one problem of the batched Gibbs calls (kdeb200_gibbs_batch,
+ * kdeb200_product_kde_batch) and of the probe kdeb200_gibbs_exact_bound_probe.  KDEB200_MAX_DENS_LARGE bounds the
+ * densities of one single Gibbs call (kdeb200_gibbs, kdeb200_gibbs_device, kdeb200_product_kde, kdeb200_gibbs_sizes):
+ * products of up to KDEB200_MAX_DENS densities run the tuned kernels, larger ones a kernel sized for up to 64. */
 #define KDEB200_MAX_DENS 16
+#define KDEB200_MAX_DENS_LARGE 64
 #define KDEB200_MAX_GPUS 16
 
 #define KDEB200_F64 0 /* FP64 arithmetic (parity mode: 1e-12 eval, exact labels) */
@@ -105,6 +110,11 @@ int kdeb200_tree_build_host(int d, int64_t N, const double *points, const double
  *   level_labels_out  optional (NULL = off): glbs.recordChoosen / labelsChoosen[sample][density][level]
  *             (:29-31,109-112) as int64 [(s1-s0)][ndens][Nlevels]: permutation of the node selected by
  *             the last sampleIndex call of each level (0 for internal nodes, -1 if Niter == 0).
+ *   ndens     1..KDEB200_MAX_DENS_LARGE (3 outside).  Products of more than KDEB200_MAX_DENS densities run one
+ *             thread-per-chain FP64 kernel at every Np and precision (kdeb200_set_gibbs_precision does not apply), with
+ *             the same labels and points as the reference; they refuse (code 5) densities with a zero, non-finite or
+ *             out-of-range (variance outside [1e-30, 1e30]) bandwidth, mean or weight, which smaller products run
+ *             through the reference's verbatim arithmetic.
  */
 int kdeb200_gibbs(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, int add_entropy,
                   const uint8_t *dimmask, const double *randU, int64_t nU, const double *randN, int64_t nN,
@@ -120,7 +130,7 @@ int kdeb200_gibbs_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int
  * followed by ONE kernel that sorts every coordinate, rebuilds the 1-D ball-tree statistics of ksize / neighborMinMax on
  * chip and runs all golden-section searches (bit-identical to kdeb200_gibbs + kdeb200_kde_lcv); larger Np fall back to that
  * two-step route inside the call.  The caller builds the product density as kde!(points_out, bw_std_out).
- * indices_out (ndens x Np) and nloo_calls_out (d) may be NULL. */
+ * indices_out (ndens x Np) and nloo_calls_out (d) may be NULL.  ndens: 1..KDEB200_MAX_DENS_LARGE, as kdeb200_gibbs. */
 int kdeb200_product_kde(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, int add_entropy,
                         const uint8_t *dimmask, uint64_t seed, double *points_out, int64_t *indices_out,
                         double *bw_std_out, int *nloo_calls_out);
@@ -190,7 +200,7 @@ int kdeb200_gibbs_exact_redone_b(unsigned long long *lanes_out, unsigned long lo
  * largest weight.  out_len: capacity of out in doubles. */
 int kdeb200_gibbs_exact_bound_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int density, int level, int pass0,
                                     const double *mu, const double *cadd, int nq, double *out, int64_t out_len);
-/* glbs.Nlevels (src/MSGibbs01.jl:555-568) and the per-sample stream consumption. */
+/* glbs.Nlevels (src/MSGibbs01.jl:555-568) and the per-sample stream consumption (ndens 1..KDEB200_MAX_DENS_LARGE). */
 int kdeb200_gibbs_sizes(const kdeb200_tree_t *trees, int ndens, int Niter, int *nlevels,
                         int64_t *uniforms_per_sample, int64_t *normals_per_sample,
                         int64_t *kernel_evals_per_sample);

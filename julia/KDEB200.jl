@@ -78,6 +78,9 @@ euclidean(addop, diffop) = all(f -> f === (+), addop) && all(f -> f === (-), dif
 # ---- S1: gibbs1 -------------------------------------------------------------------------
 # Same positional arguments as KDE.gibbs1; writes pts (d*Np) and ind (Ndens x Np) in place.
 # randU / randN === nothing selects the library's Philox streams (keyed by `seed`).
+# Ndens: 1..64 (KDEB200_MAX_DENS_LARGE), like the reference's any number of incoming messages; products of more than 16
+# densities run a kernel of their own with the same labels and points, and refuse degenerate (zero / non-finite /
+# out-of-range) bandwidths with an error instead of the reference's NaN rules.
 function gibbs1!(Ndens::Int, trees::Vector{BallTreeDensity}, Np::Int, Niter::Int,
                  pts::Vector{Float64}, ind::Matrix{Int},
                  randU::Union{Nothing,Vector{Float64}}, randN::Union{Nothing,Vector{Float64}};

@@ -874,7 +874,8 @@ def prodAppxMSGibbsS(npd0, trees, anFcns=None, anParams=None, Niter=3, addop=Non
     reference's keyword arguments; without them the kernel draws from Philox4x32-10(seed).
     s0, s1 restrict the call to samples [s0, s1) of the Np-sample run (multi-GPU sharding); the
     returned arrays then hold only that range.  recordLabels=True (the reference's
-    glbs.recordChoosen) adds a third result: labelsChoosen as an int64 array [n, Ndens, Nlevels]."""
+    glbs.recordChoosen) adds a third result: labelsChoosen as an int64 array [n, Ndens, Nlevels].  Ndens: 1..64
+    (more than 16 densities run in FP64 whatever set_gibbs_precision says, and refuse degenerate bandwidths)."""
     _require_euclidean(addop=addop, diffop=diffop, getMu=getMu, getLambda=getLambda)
     trees = list(trees)
     M = len(trees) if Ndens is None else int(Ndens)
@@ -921,7 +922,8 @@ def prodAppxMSGibbsS(npd0, trees, anFcns=None, anParams=None, Niter=3, addop=Non
 
 def prod(trees, glbs=None, addEntropy=True, seed=None, recordLabels=False):
     """*(trees::Vector{BallTreeDensity}) (src/MSGibbs01.jl:707-726).  recordLabels=True mirrors
-    `glbs.recordChoosen = true` (examples/ExtractingLabels.jl) and returns (density, labelsChoosen)."""
+    `glbs.recordChoosen = true` (examples/ExtractingLabels.jl) and returns (density, labelsChoosen).  Up to 64
+    densities, as prodAppxMSGibbsS."""
     trees = list(trees)
     if len(trees) == 1 and not addEntropy:
         return kde(getPoints(trees[0]).copy())

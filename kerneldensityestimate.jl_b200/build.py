@@ -7,9 +7,10 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libkdeb200.so")
-SOURCES = ["context.cu", "tree.cu", "eval.cu", "eval_pruned.cu", "eval_f32.cu", "extras.cu", "lcv.cu", "gibbs.cu", "gibbs_f32.cu", "gibbs_exact.cu", "gibbs_batch.cu", "eval_batch.cu", "sample_batch.cu", "peaks.cu", "capi.cu"] + [
+SOURCES = ["context.cu", "tree.cu", "eval.cu", "eval_pruned.cu", "eval_f32.cu", "extras.cu", "lcv.cu", "gibbs.cu", "gibbs_f32.cu", "gibbs_exact.cu", "gibbs_batch.cu", "gibbs_many.cu", "eval_batch.cu", "sample_batch.cu", "peaks.cu", "capi.cu"] + [
     "gibbs_d%d.cu" % d for d in range(1, 9)] + ["gibbs_f32_d%d.cu" % d for d in range(1, 9)] + [
-    "gibbs_exact_d%d.cu" % d for d in range(1, 9)] + ["gibbs_batch_d%d.cu" % d for d in range(1, 9)]
+    "gibbs_exact_d%d.cu" % d for d in range(1, 9)] + ["gibbs_batch_d%d.cu" % d for d in range(1, 9)] + [
+    "gibbs_many_d%d.cu" % d for d in range(1, 9)]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
          "-ccbin", "/usr/bin/g++", "-Xptxas", "-v"]

@@ -122,7 +122,7 @@ static int gibbs_host_block(const kdeb200_tree_t *trees, int ndens, int64_t Np, 
   const int d = trees[0]->d;
   const int64_t n = b - a;
   if (n <= 0) return 0;
-  kdeb200_tree_t loc[KDEB200_MAX_DENS];
+  kdeb200_tree_t loc[KDEB200_MAX_DENS_LARGE];
   for (int j = 0; j < ndens; ++j)
     if (int rc = tree_on(trees[j], c.slot, &loc[j])) return rc;
   DevBuf dU(c.stream), dN(c.stream), dP(c.stream), dI(c.stream), dR(c.stream);

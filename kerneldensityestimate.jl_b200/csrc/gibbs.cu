@@ -1,4 +1,4 @@
-// gibbs.cu -- host side of the Gibbs sampler: argument checks, routing (K1w, K1f, K1x, K1), the schedule cache of the
+// gibbs.cu -- host side of the Gibbs sampler: argument checks, routing (K1w, K1f, K1x, K1, K1m), the schedule cache of the
 // thread-per-chain kernels, the launches of K1 and K1w, Philox stream materialisation.  K1's kernels live in
 // gibbs_kernel.cuh and are instantiated once per dimension in gibbs_d<N>.cu; the schedule is planned in gibbs_plan.cuh.
 #include <atomic>
@@ -41,7 +41,8 @@ int gibbs_nlevels(const kdeb200_tree_t *trees, int ndens) {
 
 int gibbs_sizes(const kdeb200_tree_t *trees, int ndens, int Niter, int *nlevels, int64_t *perU, int64_t *perN,
                 int64_t *evals) {
-  if (ndens < 1 || ndens > KDEB200_MAX_DENS) KDE_FAIL(3, "gibbs: ndens=%d outside 1..%d", ndens, KDEB200_MAX_DENS);
+  if (ndens < 1 || ndens > KDEB200_MAX_DENS_LARGE)
+    KDE_FAIL(3, "gibbs: ndens=%d outside 1..%d", ndens, KDEB200_MAX_DENS_LARGE);
   if (Niter < 0) KDE_FAIL(3, "gibbs: Niter must be >= 0");
   for (int j = 0; j < ndens; ++j) {
     if (!trees[j]) KDE_FAIL(3, "gibbs: tree %d is NULL", j);
@@ -66,7 +67,7 @@ int gibbs_sizes(const kdeb200_tree_t *trees, int ndens, int Niter, int *nlevels,
 // The static schedule (draws + tile list, and K1f's / K1x's FP32 records) depends only on the tree set, Niter and the
 // route's key (SchedEntry).  It used to be rebuilt, allocated, uploaded and SYNCHRONISED on every call -- irrelevant at
 // 1M samples, but it was the difference between a 0.34 ms kernel and a 0.39 ms call at the small configurations, and it
-// made kdeb200_gibbs_device block.  Entries are invalidated wholesale whenever any tree is destroyed (a global epoch);
+// made kdeb200_gibbs_device block.  K1m (gibbs_many.cu, more than KDEB200_MAX_DENS densities) uses route K1's entries.  Entries are invalidated wholesale whenever any tree is destroyed (a global epoch);
 // each context keeps the most recent ones of each route (K1 8, K1f 4, K1x 4).  Batch counters come from a ring of 256
 // slots per entry, zeroed once at creation and reset by the LAST CTA of each launch.
 std::atomic<uint64_t> g_tree_epoch{1};
@@ -267,6 +268,9 @@ int gibbs_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, 
     if (trees[j]->degenerate) literal = true;
     if (trees[j]->slot != c.slot) KDE_FAIL(3, "gibbs: tree %d lives on another GPU of the set than the calling context", j);
   }
+  if (ndens > KDEB200_MAX_DENS)  // more densities than GibbsParams holds: K1m at every Np and precision (gibbs_many.cu)
+    return gibbs_many_device(trees, ndens, L, perU, perN, Niter, add_entropy, dimmask, d_randU, d_randN, seed, s0, s1,
+                             d_points, d_indices, d_level_labels, st, launches);
 
   GibbsParams P;
   std::memset(&P, 0, sizeof(P));

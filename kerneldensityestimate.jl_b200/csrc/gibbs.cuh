@@ -20,6 +20,11 @@ int gibbs_device(const kdeb200_tree_t *trees, int ndens, int64_t Np, int Niter, 
                  const uint8_t *dimmask, const double *d_randU, int64_t nU, const double *d_randN, int64_t nN,
                  uint64_t seed, int64_t s0, int64_t s1, double *d_points, int64_t *d_indices,
                  int64_t *d_level_labels, cudaStream_t st, int *launches);
+// K1m, the call of more than KDEB200_MAX_DENS densities (gibbs_many.cu); gibbs_device checks the arguments and routes
+int gibbs_many_device(const kdeb200_tree_t *trees, int ndens, int L, int64_t perU, int64_t perN, int Niter,
+                      int add_entropy, const uint8_t *dimmask, const double *d_randU, const double *d_randN,
+                      uint64_t seed, int64_t s0, int64_t s1, double *d_points, int64_t *d_indices,
+                      int64_t *d_level_labels, cudaStream_t st, int *launches);
 int philox_streams_device(uint64_t seed, int64_t Np, int64_t perU, int64_t perN, double *d_U, double *d_G,
                           cudaStream_t st);
 int gibbs_precision();
@@ -64,8 +69,8 @@ struct SchedEntry {
   uint64_t epoch = 0;
   int M = 0, T = 0;
   bool masked = false, literal = false;
-  unsigned char mask[KDEB200_MAX_DENS][KDEB200_MAX_DIM] = {};
-  kdeb200_tree_t trees[KDEB200_MAX_DENS] = {nullptr};
+  unsigned char mask[KDEB200_MAX_DENS][KDEB200_MAX_DIM] = {};  // K1f only, which serves M <= KDEB200_MAX_DENS
+  kdeb200_tree_t trees[KDEB200_MAX_DENS_LARGE] = {nullptr};    // K1 also caches K1m's schedules (gibbs_many.cu)
   char *d_base = nullptr;   // draws | tiles | counters | FP32 records, one allocation on the context's device
   char *d_extra = nullptr;  // K1x: XDraws | tile centres
   Draw *d_draws = nullptr;

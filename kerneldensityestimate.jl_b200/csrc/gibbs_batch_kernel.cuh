@@ -9,13 +9,18 @@
 // verbatim (state init, samplePoint!, hoist, the 1e-99 rule, the chunk search, the final point), and so are the Philox addressing
 // (problem seed, local sample index) and the injected-stream indexing.  Every problem's outputs are those of K1 run on
 // that problem alone, bit for bit.
+// The same kernel at MD = 32 / 64 is K1m (DESIGN.md "K1m", host side gibbs_many.cu, instantiations gibbs_many_d<N>.cu):
+// a single call of more than KDEB200_MAX_DENS densities, run as a one-problem launch over the call's sample slice.
 #pragma once
 #include "gibbs_kernel.cuh"
 
 namespace kdeb200 {
 
-// One problem of a batch, in device memory: what gibbs_device puts into GibbsParams for a single K1 call.
-struct alignas(16) BatchProb {
+// One problem of a batch, in device memory: what gibbs_device puts into GibbsParams for a single K1 call.  MDC is the
+// capacity of the per-density arrays: KDEB200_MAX_DENS for K1b, 32 or 64 for the single call of more than
+// KDEB200_MAX_DENS densities (gibbs_many.cu), which GibbsParams cannot describe.
+template <int MDC>
+struct alignas(16) BatchProbT {
   const Draw *draws;
   const TileDesc *tiles;
   const double *randU, *randN;  // the problem's injected streams or null (Philox)
@@ -24,30 +29,41 @@ struct alignas(16) BatchProb {
   int64_t Np, perU, perN;
   uint64_t seed;
   int ndraws, ntiles, M, L, add_entropy, pad_;
-  const double *root_rec[KDEB200_MAX_DENS];
-  const int64_t *labels[KDEB200_MAX_DENS];
-  double hvar[KDEB200_MAX_DENS][KDEB200_MAX_DIM];
-  unsigned char mask[KDEB200_MAX_DENS][KDEB200_MAX_DIM];
-  unsigned char other[KDEB200_MAX_DENS][KDEB200_MAX_DIM];
+  const double *root_rec[MDC];
+  const int64_t *labels[MDC];
+  double hvar[MDC][KDEB200_MAX_DIM];
+  unsigned char mask[MDC][KDEB200_MAX_DIM];
+  unsigned char other[MDC][KDEB200_MAX_DIM];
 };
+using BatchProb = BatchProbT<KDEB200_MAX_DENS>;
 static_assert(sizeof(BatchProb) % 16 == 0, "BatchProb is copied to shared memory in 16-byte words");
+static_assert(sizeof(BatchProbT<KDEB200_MAX_DENS_LARGE>) % 16 == 0, "BatchProbT is copied in 16-byte words");
 
-// One launch: the problems of one (d, masked) class.
+// One launch: the problems of one (d, masked) class (K1b), or the one problem of a many-density single call.
 struct BatchParams {
-  const BatchProb *probs;
+  const void *probs;  // BatchProbT<max(MD, KDEB200_MAX_DENS)>[nprob]
   const int *block0;  // nprob + 1 entries: first CTA of each problem, then the grid size
   int nprob;
   const double *exptab;
   ExpConsts ec;
+  // Read only by the capacities above KDEB200_MAX_DENS, which run one problem, the single call's slice of samples
+  // [s0, Np) (Np is then the slice's end, s1), with outputs at s - s0 and the optional labelsChoosen record
+  // [(s1 - s0)][M][L] of K1 (GibbsParams::level_labels).
+  int64_t s0;
+  int64_t *level_labels;
 };
 
+// MD = capacity of the per-chain state in densities, as in K1: 4, 8 or 16 for K1b; 32 or 64 for the single call of
+// more than KDEB200_MAX_DENS densities (ONE below), whose descriptor is a BatchProbT<MD>.
 template <int D, bool MASK, int MD>
 __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_batch_kernel(const __grid_constant__ BatchParams B) {
+  constexpr bool ONE = MD > KDEB200_MAX_DENS;
+  using Prob = BatchProbT<ONE ? MD : KDEB200_MAX_DENS>;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double *tiles = reinterpret_cast<double *>(smem_raw);
   __shared__ __align__(16) double tab[KDE_EXP_TAB];
   __shared__ __align__(8) uint64_t bars[GB_STAGES];
-  __shared__ BatchProb P;
+  __shared__ Prob P;
   const int tid = threadIdx.x;
 
   int lo = 0, hi = B.nprob - 1;  // the last problem whose first block is <= blockIdx.x (every problem has a block)
@@ -56,9 +72,9 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_batch_kernel(c
     if (B.block0[mid] <= (int)blockIdx.x) lo = mid; else hi = mid - 1;
   }
   {
-    const int4 *src = reinterpret_cast<const int4 *>(B.probs + lo);
+    const int4 *src = reinterpret_cast<const int4 *>(static_cast<const Prob *>(B.probs) + lo);
     int4 *dst = reinterpret_cast<int4 *>(&P);
-    for (int i = tid; i < (int)(sizeof(BatchProb) / 16); i += GB_THREADS) dst[i] = src[i];
+    for (int i = tid; i < (int)(sizeof(Prob) / 16); i += GB_THREADS) dst[i] = src[i];
   }
   for (int i = tid; i < KDE_EXP_TAB; i += GB_THREADS) tab[i] = B.exptab[i];
   if (tid == 0) {
@@ -87,6 +103,7 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_batch_kernel(c
   int selpos[MD];
 
   int64_t s = (int64_t)((int)blockIdx.x - B.block0[lo]) * GB_THREADS + tid;
+  if constexpr (ONE) s += B.s0;
   const bool live = s < P.Np;
   if (!live) s = P.Np - 1;  // idle lanes replay the last chain (keeps the CTA in lock-step)
 
@@ -225,6 +242,10 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_batch_kernel(c
       }
     }
     selpos[j] = zs;
+    if constexpr (ONE) {  // sampleIndex records permutation[ind[j]] per (sample, density, level), as in K1
+      if (B.level_labels && dr.kind == 1 && live)
+        B.level_labels[((s - B.s0) * M + j) * P.L + (dr.level - 1)] = dr.levperm[zs];
+    }
 
     // updateGlbParticlesVariance!(j)
     {
@@ -254,7 +275,8 @@ __global__ void __launch_bounds__(GB_THREADS, GB_MINBLOCKS) gibbs_batch_kernel(c
   double *points = P.points;
   int64_t *indices = P.indices;
   if (live) {
-    const int64_t o = s;
+    int64_t o = s;
+    if constexpr (ONE) o -= B.s0;
     for (int j = 0; j < M; ++j) indices[o * M + j] = P.labels[j][selpos[j]];
 #pragma unroll
     for (int k = 0; k < D; ++k) {
@@ -296,6 +318,23 @@ cudaError_t launch_gibbs_batch_d(const BatchParams &B, bool masked, int maxM, in
   if (maxM <= 4) return launch(gibbs_batch_kernel<D, false, 4>);
   if (maxM <= 8) return launch(gibbs_batch_kernel<D, false, 8>);
   return launch(gibbs_batch_kernel<D, false, KDEB200_MAX_DENS>);
+}
+
+// the single call of M > KDEB200_MAX_DENS densities (gibbs_many.cu): one problem, MD = 32 or 64 from M
+template <int D>
+cudaError_t launch_gibbs_many_d(const BatchParams &B, bool masked, int M, int grid, cudaStream_t st) {
+  const size_t smem = GB_STAGES * GB_TILE_BYTES;
+  auto launch = [&](auto kern) -> cudaError_t {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    if (e != cudaSuccess) return e;
+    kern<<<grid, GB_THREADS, smem, st>>>(B);
+    return cudaGetLastError();
+  };
+  static_assert(KDEB200_MAX_DENS_LARGE == 64, "the instantiated capacities are 32 and 64");
+  if (masked) return M <= 32 ? launch(gibbs_batch_kernel<D, true, 32>) : launch(gibbs_batch_kernel<D, true, 64>);
+  return M <= 32 ? launch(gibbs_batch_kernel<D, false, 32>) : launch(gibbs_batch_kernel<D, false, 64>);
 }
 
 }  // namespace kdeb200

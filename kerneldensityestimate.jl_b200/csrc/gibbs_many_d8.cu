@@ -1,0 +1,5 @@
+// gibbs_many_d8.cu -- explicit instantiation of the many-density Gibbs kernel (K1m, MD = 32 and 64) for d = 8.
+#include "gibbs_batch_kernel.cuh"
+namespace kdeb200 {
+template cudaError_t launch_gibbs_many_d<8>(const BatchParams &, bool, int, int, cudaStream_t);
+}

@@ -187,10 +187,13 @@ int kdeb200_gibbs_f32_slow_draws(unsigned long long *count_out);
  * (KDEB200_GIBBS_EXACT=0 forces the all-FP64 kernel).  Counts the redone leaf-level lane-draws and the warp-draws that
  * contained one (warps_out may be NULL) on the calling context's device since the last call;
  * kdeb200_gibbs_exact_redone_internal counts the same for the sampleIndex draws of every internal level, and
- * kdeb200_gibbs_exact_redone_b for the sampleIndices! draws (one per internal level and density). */
+ * kdeb200_gibbs_exact_redone_b for the sampleIndices! draws (one per internal level and density).  A redone draw is
+ * first decided from warp-parallel FP64 sums with a proven error bound; kdeb200_gibbs_exact_tier3 counts the lane-draws
+ * of every class that bound could not decide either, which were summed serially in node order, and their warp-draws. */
 int kdeb200_gibbs_exact_redone(unsigned long long *lanes_out, unsigned long long *warps_out);
 int kdeb200_gibbs_exact_redone_internal(unsigned long long *lanes_out, unsigned long long *warps_out);
 int kdeb200_gibbs_exact_redone_b(unsigned long long *lanes_out, unsigned long long *warps_out);
+int kdeb200_gibbs_exact_tier3(unsigned long long *lanes_out, unsigned long long *warps_out);
 /* Diagnostic for tests of the bound above (d = 3): for nq query conditionals (mu, Calmost: nq x d each, row-major) of the
  * certified draw of density `density` (0-based) on schedule level `level` (1-based) -- the leaf-level draw, or on an
  * internal level the first sampleIndex draw, or with pass0 != 0 the sampleIndices! draw (which evaluates against mu alone

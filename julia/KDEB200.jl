@@ -45,6 +45,13 @@ function gibbs_f32_slow_draws()
   check(ccall((:kdeb200_gibbs_f32_slow_draws, LIB), Cint, (Ref{Culonglong},), n))
   return Int(n[])
 end
+# FP64 (default) calls: (lane-draws, warp-draws) whose label neither the certified FP32 nor the certified warp-parallel
+# FP64 sums could decide, so that they were summed serially in node order, since the last call
+function gibbs_exact_tier3()
+  n, w = Ref{Culonglong}(0), Ref{Culonglong}(0)
+  check(ccall((:kdeb200_gibbs_exact_tier3, LIB), Cint, (Ref{Culonglong}, Ref{Culonglong}), n, w))
+  return Int(n[]), Int(w[])
+end
 
 # ---- S0: device-resident BallTreeDensity -------------------------------------------------
 mutable struct DeviceTree

@@ -70,6 +70,7 @@ SIGNATURES = {
     "kdeb200_gibbs_exact_redone": (C.c_int, [C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]),
     "kdeb200_gibbs_exact_redone_internal": (C.c_int, [C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]),
     "kdeb200_gibbs_exact_redone_b": (C.c_int, [C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]),
+    "kdeb200_gibbs_exact_tier3": (C.c_int, [C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]),
     "kdeb200_gibbs_exact_bound_probe": (C.c_int, [C.POINTER(tree_t), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, f64p,
                                                   f64p, C.c_int, f64p, C.c_int64]),
     "kdeb200_pruned_stats": (C.c_int, [f64p, i64p]),

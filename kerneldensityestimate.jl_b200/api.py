@@ -29,7 +29,7 @@ __all__ = [
     "KDEError", "BallTree", "BallTreeDensity", "kde", "kde_bang", "getPoints", "getBW", "getWeights", "marginal",
     "sample", "rand", "resample", "sample_batch", "rand_batch", "resample_batch", "evaluateDualTree", "evaluateDualTree_batch", "kde_batch", "lcv_bandwidths_batch", "evalAvgLogL", "entropy", "kld", "minkld", "nLOO_LL", "golden",
     "ksize", "neighborMinMax", "lcv_bandwidths", "updateBandwidth", "prodAppxMSGibbsS", "prodAppxMSGibbsS_batch", "prod_batch", "gibbs_batch_split", "Ndim", "Npts", "init", "init_multi", "multi_count", "gibbs_sizes",
-    "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "gibbs_exact_redone_internal", "gibbs_exact_redone_b", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
+    "philox_streams", "pipe_peak", "last_kernel_ms", "F64", "F32", "F64_BOUNDED", "F32_BOUNDED", "setForceEvalDirect", "set_pruning", "set_gibbs_precision", "gibbs_f32_slow_draws", "gibbs_exact_redone", "gibbs_exact_redone_internal", "gibbs_exact_redone_b", "gibbs_exact_tier3", "pruned_stats", "prod", "getKDERange", "getKDERangeLinspace",
     "getKDEMax", "getKDEMean", "getKDEfit", "intersIntgAppxIS", "eval_marginals", "to_string", "from_string",
 ]
 
@@ -106,6 +106,14 @@ def gibbs_exact_redone_b():
     bound could not decide and that were redone in FP64, since the last call"""
     n, w = C.c_ulonglong(0), C.c_ulonglong(0)
     check(lib().kdeb200_gibbs_exact_redone_b(C.byref(n), C.byref(w)))
+    return int(n.value), int(w.value)
+
+
+def gibbs_exact_tier3():
+    """(lane-draws, warp-draws) of the FP64 sampler, any class, that were redone in FP64 and that the warp-parallel FP64
+    sums could not decide either, so that they were summed serially in node order, since the last call"""
+    n, w = C.c_ulonglong(0), C.c_ulonglong(0)
+    check(lib().kdeb200_gibbs_exact_tier3(C.byref(n), C.byref(w)))
     return int(n.value), int(w.value)
 
 

@@ -694,6 +694,13 @@ int kdeb200_gibbs_exact_redone_b(unsigned long long *lanes_out, unsigned long lo
   return gibbs_exact_redone_b(lanes_out, warps_out);
 }
 
+int kdeb200_gibbs_exact_tier3(unsigned long long *lanes_out, unsigned long long *warps_out) {
+  KDE_SERIALISE();
+  if (!lanes_out) KDE_FAIL(2, "gibbs_exact_tier3: NULL argument");
+  if (int rc = ensure_init()) return rc;
+  return gibbs_exact_tier3(lanes_out, warps_out);
+}
+
 int kdeb200_gibbs_exact_bound_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int density, int level, int pass0,
                                     const double *mu, const double *cadd, int nq, double *out, int64_t out_len) {
   KDE_SERIALISE();

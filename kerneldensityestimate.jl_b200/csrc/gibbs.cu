@@ -79,7 +79,7 @@ constexpr size_t SCHED_KEEP[NROUTES] = {8, 4, 4};
 std::mutex g_sched_mu;
 std::list<SchedEntry> g_sched[NROUTES][KDEB200_MAX_GPUS];
 unsigned long long *g_counters[KDEB200_MAX_GPUS] = {nullptr};
-constexpr int NCOUNTERS = 7;
+constexpr int NCOUNTERS = 9;
 
 void sched_free(SchedEntry &e, cudaStream_t st) {
   if (e.d_base) cudaFreeAsync(e.d_base, st);
@@ -226,6 +226,14 @@ int gibbs_exact_redone_internal(unsigned long long *lanes, unsigned long long *w
 int gibbs_exact_redone_b(unsigned long long *lanes, unsigned long long *warps) {
   unsigned long long h[2] = {0, 0};
   if (int rc = take_counters(5, 2, h)) return rc;
+  if (lanes) *lanes = h[0];
+  if (warps) *warps = h[1];
+  return 0;
+}
+// of those, the ones the warp-parallel FP64 sum could not decide either (every class)
+int gibbs_exact_tier3(unsigned long long *lanes, unsigned long long *warps) {
+  unsigned long long h[2] = {0, 0};
+  if (int rc = take_counters(7, 2, h)) return rc;
   if (lanes) *lanes = h[0];
   if (warps) *warps = h[1];
   return 0;

@@ -33,6 +33,7 @@ int gibbs32_slow_draws(unsigned long long *out);
 int gibbs_exact_redone(unsigned long long *lanes, unsigned long long *warps);
 int gibbs_exact_redone_internal(unsigned long long *lanes, unsigned long long *warps);
 int gibbs_exact_redone_b(unsigned long long *lanes, unsigned long long *warps);
+int gibbs_exact_tier3(unsigned long long *lanes, unsigned long long *warps);
 int gibbs_exact_probe(const kdeb200_tree_t *trees, int ndens, int Niter, int j, int level, int pass0, const double *mu,
                       const double *cadd, int nq, double *out, int64_t out_len);
 void gibbs_invalidate_schedules();  // a tree is destroyed: cached schedules point into tree records

@@ -284,7 +284,7 @@ int gibbs_exact_launch(GibbsParams &P, const SchedEntry &E, int d, cudaStream_t 
   X.ex2_err = GX_EX2_ERR;
   X.rsq_err = GX_RSQ_ERR;
   X.inflate = 1.0;
-  if (const char *ev = getenv("KDEB200_GIBBS_EXACT_INFLATE")) X.inflate = atof(ev);  // tests: force the FP64 redo
+  if (const char *ev = getenv("KDEB200_GIBBS_EXACT_INFLATE")) X.inflate = atof(ev);  // tests: force the FP64 tiers
   unsigned long long *d_count = nullptr;
   if (int rc = gibbs_counters(&d_count)) return rc;
   X.redone = d_count + 1;
@@ -293,6 +293,8 @@ int gibbs_exact_launch(GibbsParams &P, const SchedEntry &E, int d, cudaStream_t 
   X.warp_redone_int = d_count + 4;
   X.redone_b = d_count + 5;
   X.warp_redone_b = d_count + 6;
+  X.tier3 = d_count + 7;
+  X.warp_tier3 = d_count + 8;
   X.scr_stride = GX_SCR + E.redo_blocks;
   // The redo scratch belongs to this launch alone, stream-ordered on `st`: launches on other streams may be in flight
   // at the same time, and a warp that shared its (block, warp) slot with another launch would sum foreign terms.

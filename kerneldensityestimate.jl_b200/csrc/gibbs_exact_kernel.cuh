@@ -8,8 +8,9 @@
 // K1x instead evaluates the nodes in packed FP32 (gibbs_f32_kernel.cuh's pair records and arithmetic) and carries next
 // to every FP32 prefix sum S'_z a bound E_z on |S'_z - S_z / W| (W: the level's largest weight; DESIGN.md "K1x" derives
 // it).  A lane's label is taken only when the intervals prove it:  hi(S_{z-1}) < lo(target)  and  hi(target) <= lo(S_z).
-// A lane that cannot prove its label is redone by its warp with K1's FP64 arithmetic (K1w's scheme: lanes evaluate, one
-// lane sums in node order, the result is K1's label by construction), reading K1's exp table from global memory.
+// A lane that cannot prove its label is redone by its warp with K1's FP64 node values, reading K1's exp table from
+// global memory: first summed in parallel and certified again with an FP64-sized bound (xa_tier2), and only what that
+// cannot prove summed by one lane in node order (xa_redo, K1w's scheme: K1's label by construction).
 #pragma once
 #include <type_traits>
 
@@ -33,7 +34,7 @@ struct alignas(16) XDraw {
   double bmin[KDEB200_MAX_DIM];       // variants B, C: the level's smallest node variance b_k per dimension
   double lw2max;                      // log2 of the level's largest weight (records hold lw2max - log2 w >= 0)
   int G, nchunks;                     // K1x's own checkpoint chunks (nodes, power of two)
-  int fp32;                           // 0: the level is outside the FP32 range guard, every lane takes the FP64 redo
+  int fp32;                           // 0: the level is outside the FP32 range guard, every lane goes to xa_tier2
   int pad;
 };
 
@@ -46,9 +47,11 @@ struct XParams {
   unsigned long long *warp_redone_int;
   unsigned long long *redone_b;       // the same two for the sampleIndices! draws (variant B)
   unsigned long long *warp_redone_b;
+  unsigned long long *tier3;          // lane-draws (live chains) and warp-draws of every class that the warp-parallel
+  unsigned long long *warp_tier3;     // FP64 sum (xa_tier2) could not decide and the serial sweep (xa_redo) did
   double ex2_err;                     // relative error bound of ex2.approx.ftz.f32 on [-126, 0]
   double rsq_err;                     // relative error bound of rsqrt.approx.ftz.f32 on normal floats
-  double inflate;                     // test hook: multiplies the bound (1 in production)
+  double inflate;                     // test hook: multiplies the FP32 bound and xa_tier2's delta (1 in production)
   int scr_stride;                     // GX_SCR + the largest number of redo blocks of a level
 };
 
@@ -281,9 +284,115 @@ __device__ __forceinline__ int xa_decide(const Draw &dr, const XDraw &xd, const 
   return -1;
 }
 
-// K1's label for one lane's certified draw, computed by the whole warp: lanes evaluate the nodes with K1's eval_node,
-// lane 0 adds them in node order (the same additions as K1's pass 1 and pass 2), pT < 1e-99 rule included.  The first
-// sweep records the running sum at the end of every block of GX_SCR nodes (scr[GX_SCR + b]); the second sweep
+// K1's label when its pT * scale < 1e-99 rule fires (:311-315: all p[z] = weight(last node)); rare, lane 0 computes it
+__device__ __forceinline__ int x_flat(const Draw &dr, double u) {
+  const int n = dr.n;
+  int zs = n - 1;
+  if ((threadIdx.x & 31) == 0) {
+    const double w = dr.wts[n - 1];
+    double tot = 0.0;
+    for (int z = 0; z < n; ++z) tot += w;
+    const double qv = w / tot;
+    double cdf = 0.0;
+    bool found = false;
+    for (int z = 0; z < n - 1; ++z) {
+      cdf += qv;
+      if (!found && u <= cdf) {
+        zs = z;
+        found = true;
+      }
+    }
+  }
+  return __shfl_sync(0xffffffffu, zs, 0);
+}
+
+// Tier 2 of an undecided draw: K1's FP64 node values, summed by the whole warp in parallel, with a certificate.  One
+// block of GX_SCR nodes: lane l evaluates nodes base + GX_RUN l .. + GX_RUN - 1 with K1's eval_node and adds them in
+// order (p[i]: its run's partial sums); a warp scan of the run totals gives each lane the sum of the runs before it
+// (excl) and the block total (tot).  Every term reaches p[i] through at most GX_RUN roundings, excl and tot through at
+// most GX_RUN + 5.
+constexpr int GX_RUN = GX_SCR / 32;
+template <int D, int VAR>
+__device__ __forceinline__ void x2_block(const Draw &dr, const Hoist<D, false> &h, const double *__restrict__ tab,
+                                         const ExpConsts &ec, int base, double (&p)[GX_RUN], double &excl, double &tot) {
+  const unsigned FULL = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  const int z0 = base + lane * GX_RUN;
+  double s = 0.0;
+#pragma unroll
+  for (int i = 0; i < GX_RUN; ++i) {
+    if (z0 + i < dr.n) s = __dadd_rn(s, eval_node<D, false, VAR, true>(dr.rec + (size_t)(z0 + i) * dr.stride, h, tab, ec));
+    p[i] = s;
+  }
+  double inc = s;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const double t = __shfl_up_sync(FULL, inc, o);
+    if (lane >= o) inc = __dadd_rn(inc, t);
+  }
+  excl = __shfl_up_sync(FULL, inc, 1);
+  if (lane == 0) excl = 0.0;
+  tot = __shfl_sync(FULL, inc, 31);
+}
+
+// K1's label for one lane's undecided draw from the warp-parallel FP64 sums of x2_block, or -1 when they cannot prove
+// it.  Block end-sums C_b = C_{b-1} + tot_b go to scr[GX_SCR + b]; node prefixes are C_{b-1} + (excl + p[i]).  Each
+// computed sum S'_z is a sum of K1's non-negative terms through at most nb + GX_RUN + 7 roundings, K1's own S_z one
+// through at most n, so S_z lies in S'_z [1 - delta, 1 + delta] with delta = 1.001 (n + nb + GX_RUN + 7) 2^-53
+// (DESIGN.md "K1x" derives it; `inflate` scales it like the FP32 bound).  The label is taken as xa_decide takes it:
+// the first node whose interval can reach the target, when its lower end provably reaches it (or it is node n - 1).
+template <int D, int VAR>
+__device__ __noinline__ int xa_tier2(const Draw &dr, const Hoist<D, false> &h, double scale, double u,
+                                     const double *__restrict__ tab, const ExpConsts &ec, double *__restrict__ scr,
+                                     double inflate) {
+  const unsigned FULL = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  const int n = dr.n;
+  const int nb = (n + GX_SCR - 1) / GX_SCR;
+  const double delta = inflate * 1.001 * (double)(n + nb + GX_RUN + 7) * 0x1.0p-53;
+  const double fLo = __dadd_rd(1.0, -delta), fHi = __dadd_ru(1.0, delta);
+  double p[GX_RUN], excl, tot, C = 0.0;
+  for (int b = 0; b < nb; ++b) {
+    x2_block<D, VAR>(dr, h, tab, ec, b * GX_SCR, p, excl, tot);
+    C = __dadd_rn(C, tot);
+    if (lane == 0) scr[GX_SCR + b] = C;
+  }
+  __syncwarp();
+  // non-finite sums, a uniform outside [0, 1) (the target interval would not be ordered) and a 1e-99 rule that could
+  // go either way are left to tier 3
+  if (!isfinite(C) || !(u >= 0.0 && u < 1.0)) return -1;
+  const double pLo = __dmul_rd(C, fLo), pHi = __dmul_ru(C, fHi);
+  if (__dmul_ru(pHi, scale) < 1e-99) return x_flat(dr, u);  // K1's rule fires for every pT in the interval
+  if (!(pLo > 0.0 && __dmul_rd(pLo, scale) >= 1e-99)) return -1;
+  // K1's target fl(u pT) lies in [tLo, tHi]: fl is monotone, and rounds no lower than RD nor higher than RU
+  const double tLo = __dmul_rd(u, pLo), tHi = __dmul_ru(u, pHi);
+  unsigned bf = (unsigned)nb;  // first block whose end-sum interval reaches tLo; K1's sums before it all lie below
+  for (int b = lane; b < nb; b += 32)
+    if (tLo <= __dmul_ru(scr[GX_SCR + b], fHi)) {
+      bf = (unsigned)b;
+      break;
+    }
+  bf = __reduce_min_sync(FULL, bf);
+  if (bf >= (unsigned)nb) return -1;
+  const int base = (int)bf * GX_SCR;
+  const double C0 = bf ? scr[GX_SCR + bf - 1] : 0.0;
+  __syncwarp();  // scr is tier 3's to overwrite after this
+  x2_block<D, VAR>(dr, h, tab, ec, base, p, excl, tot);
+  // per lane the first of its nodes whose interval reaches tLo, key 2 z + (not certified); the warp takes the least z
+  unsigned key = 0xffffffffu;
+#pragma unroll
+  for (int i = GX_RUN - 1; i >= 0; --i) {
+    const int z = base + lane * GX_RUN + i;
+    const double S = __dadd_rn(C0, __dadd_rn(excl, p[i]));
+    if (z < n && tLo <= __dmul_ru(S, fHi)) key = 2u * (unsigned)z + ((tHi <= __dmul_rd(S, fLo) || z == n - 1) ? 0u : 1u);
+  }
+  key = __reduce_min_sync(FULL, key);
+  return (key & 1u) ? -1 : (int)(key >> 1);
+}
+
+// Tier 3: K1's label for one lane's undecided draw, computed by the whole warp: lanes evaluate the nodes with K1's
+// eval_node, lane 0 adds them in node order (the same additions as K1's pass 1 and pass 2), pT < 1e-99 rule included.
+// The first sweep records the running sum at the end of every block of GX_SCR nodes (scr[GX_SCR + b]); the second sweep
 // re-evaluates only the block whose end-sum first reaches the target, continuing from the exact sum before it.
 template <int D, int VAR>
 __device__ __noinline__ int xa_redo(const Draw &dr, const Hoist<D, false> &h, double scale, double u,
@@ -306,24 +415,7 @@ __device__ __noinline__ int xa_redo(const Draw &dr, const Hoist<D, false> &h, do
   }
   const double pT = __shfl_sync(FULL, S, 0);
   int zs = n - 1;
-  if (pT * scale < 1e-99) {  // :311-315: all p[z] = weight(last node)
-    if (lane == 0) {
-      const double w = dr.wts[n - 1];
-      double tot = 0.0;
-      for (int z = 0; z < n; ++z) tot += w;
-      const double qv = w / tot;
-      double cdf = 0.0;
-      bool found = false;
-      for (int z = 0; z < n - 1; ++z) {
-        cdf += qv;
-        if (!found && u <= cdf) {
-          zs = z;
-          found = true;
-        }
-      }
-    }
-    return __shfl_sync(FULL, zs, 0);
-  }
+  if (pT * scale < 1e-99) return x_flat(dr, u);  // :311-315: all p[z] = weight(last node)
   const double target = u * pT;
   unsigned bf = (unsigned)nb;  // first block whose end-sum reaches the target
   for (int b = lane; b < nb; b += 32)
@@ -350,6 +442,42 @@ __device__ __noinline__ int xa_redo(const Draw &dr, const Hoist<D, false> &h, do
   f = __shfl_sync(FULL, f, 0);
   __syncwarp();
   return f;
+}
+
+// The FP64 tiers for the undecided lanes `ub` of a warp-draw, one lane at a time with the whole warp: tier 2
+// (xa_tier2), and tier 3 (xa_redo) for what tier 2 cannot prove.  Returns this lane's label (z if it was decided in
+// FP32).  Out of line with everything it needs, so that the hot loop's register allocation does not see it; tier 3 is
+// rare at inflate 1, so its counters are global atomics here.
+template <int D, int VAR>
+__device__ __noinline__ int xa_undecided(const Draw &dr, unsigned ub, const double (&mu)[D], const double (&cadd)[D],
+                                         const double *__restrict__ hvar, double scale, double u, bool live, int z,
+                                         const double *__restrict__ tab, const ExpConsts &ec, double *__restrict__ scr,
+                                         const XParams &X) {
+  const unsigned FULL = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  bool t3 = false;  // this warp-draw reached tier 3
+  while (ub) {
+    const int L = __ffs(ub) - 1;
+    ub &= ub - 1;
+    Hoist<D, false> hl;
+#pragma unroll
+    for (int k = 0; k < D; ++k) {
+      hl.mu[k] = __shfl_sync(FULL, mu[k], L);
+      hl.cadd[k] = __shfl_sync(FULL, cadd[k], L);
+      hl.ich[k] = (VAR == VAR_A) ? sqrt(0.5 / (hvar[k] + hl.cadd[k])) : 0.0;  // K1's expression
+      hl.act[k] = true;
+    }
+    const double sL = __shfl_sync(FULL, scale, L), uL = __shfl_sync(FULL, u, L);
+    int zl = xa_tier2<D, VAR>(dr, hl, sL, uL, tab, ec, scr, X.inflate);
+    if (zl < 0) {
+      zl = xa_redo<D, VAR>(dr, hl, sL, uL, tab, ec, scr);
+      if (__shfl_sync(FULL, (int)live, L) && lane == 0) atomicAdd(X.tier3, 1ull);
+      t3 = true;
+    }
+    if (lane == L) z = zl;
+  }
+  if (t3 && lane == 0) atomicAdd(X.warp_tier3, 1ull);
+  return z;
 }
 
 // K1's conditional of a draw, from the chain state and with K1's expressions (so its FP64 values are K1's): sampleIndices!
@@ -468,7 +596,7 @@ __global__ void __launch_bounds__(GB_THREADS, GX_MINBLOCKS) gibbs_exact_kernel(c
         }
       }
 
-      // a certified draw: FP32 pass 1, the bound, the FP32 decision, the FP64 redo of the lanes it leaves undecided
+      // a certified draw: FP32 pass 1, the bound, the FP32 decision, the FP64 tiers for the lanes it leaves undecided
       auto certified = [&](auto var) -> int {
         constexpr int VAR = decltype(var)::value;
         const XDraw xd = X.xd[di];
@@ -512,21 +640,7 @@ __global__ void __launch_bounds__(GB_THREADS, GX_MINBLOCKS) gibbs_exact_kernel(c
             if (lane == 0) ++wredone[VAR];
             double cadd[D];
             x_cond<D, MD>(dr.kind, j, M, lam, lmu, X_, mu, cadd);
-            while (ub) {
-              const int L = __ffs(ub) - 1;
-              ub &= ub - 1;
-              Hoist<D, false> hl;
-#pragma unroll
-              for (int k = 0; k < D; ++k) {
-                hl.mu[k] = __shfl_sync(FULL, mu[k], L);
-                hl.cadd[k] = __shfl_sync(FULL, cadd[k], L);
-                hl.ich[k] = (VAR == VAR_A) ? sqrt(0.5 / (P.hvar[j][k] + hl.cadd[k])) : 0.0;  // K1's expression
-                hl.act[k] = true;
-              }
-              const int zl = xa_redo<D, VAR>(dr, hl, __shfl_sync(FULL, scale, L), __shfl_sync(FULL, u, L), P.exptab,
-                                             P.ec, scr);
-              if (lane == L) z = zl;
-            }
+            z = xa_undecided<D, VAR>(dr, ub, mu, cadd, P.hvar[j], scale, u, live, z, P.exptab, P.ec, scr, X);
           }
         }
         return z;

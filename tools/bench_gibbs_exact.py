@@ -2,8 +2,9 @@
 python tools/bench_gibbs_exact.py [Np] [dims] [reps] -> one JSON object.  dims is a comma list (default 3 = the C4 shape:
 8 densities x 4096 components, Niter 5).  Kernel times are the library's own CUDA-event times.  `redone_*` are the
 lane-draws / warp-draws K1x redid in FP64 per leaf-level draw, `redone_b_*` the same per sampleIndices! draw of an
-internal level, `redone_int_*` per sampleIndex draw of an internal level; `identical` compares points and labels bit for
-bit.
+internal level, `redone_int_*` per sampleIndex draw of an internal level; `tier3_lanes` / `tier3_warps` count the
+redone lane-draws / warp-draws (all classes, per call) that the warp-parallel FP64 sums could not decide either, which
+were summed serially in node order; `identical` compares points and labels bit for bit.
 Also reports the card's name and power limit: the times belong to them."""
 import json, os, subprocess, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -41,7 +42,7 @@ for d in dims:
     r = {"k1_ms": [], "k1x_ms": []}
     run("1", trees)  # schedule, records and scratch are built on the first call
     counters = {"": K.gibbs_exact_redone, "_b": K.gibbs_exact_redone_b, "_int": K.gibbs_exact_redone_internal}
-    for f in counters.values():
+    for f in list(counters.values()) + [K.gibbs_exact_tier3]:
         f()
     for _ in range(reps):
         ref, ms = run("0", trees)
@@ -57,6 +58,7 @@ for d in dims:
         lanes, warps = f()
         r["redone%s_lane_frac" % cls] = lanes / max(draws[cls], 1)
         r["redone%s_warp_frac" % cls] = warps / max(draws[cls] / 32, 1)
+    r["tier3_lanes"], r["tier3_warps"] = [v / reps for v in K.gibbs_exact_tier3()]
     r["identical"] = bool(all(np.array_equal(a, b) for a, b in zip(ref, new)))
     r["k1_samples_per_s"] = Np / min(r["k1_ms"]) * 1e3
     r["k1x_samples_per_s"] = Np / min(r["k1x_ms"]) * 1e3
